@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the Reflexiv hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5] [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...            (one rank per GPU)
 
 Workloads (BASELINE.json `configs`, selected by --config; the default and the driver's run is 2):
@@ -290,6 +290,44 @@ def contig_digests(bases, offs):
     return sorted(out)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def result_arrays(ctx, mode: str) -> dict:
+    """What a caller of the timed path receives from `ctx`, as float arrays that hold every value exactly.  The library
+    leaves the order of table rows and of contigs unspecified, so rows are sorted by key and contigs by sequence: two
+    runs or two builds that compute the same result give the same arrays."""
+    import numpy as np
+    if mode == "counter":
+        keys, cnts = ctx.counts()
+        order = np.lexsort(keys.T)
+        # a 64-bit key word does not fit a float64 mantissa, its two 32-bit halves do
+        return {"count_keys": keys[order].view(np.uint32).astype(np.float64), "count_values": cnts[order].astype(np.float64)}
+    bases, offs, left, right = ctx.contigs_raw()
+    seqs = [bases[int(offs[i]):int(offs[i + 1])].tobytes() for i in range(len(left))]
+    order = sorted(range(len(seqs)), key=lambda i: (seqs[i], left[i], right[i]))
+    return {"contig_bases": np.frombuffer(b"".join(seqs[i] for i in order), dtype=np.uint8).astype(np.float32),
+            "contig_lengths": np.array([len(seqs[i]) for i in order], dtype=np.float64),
+            "contig_left": left[order].astype(np.float64), "contig_right": right[order].astype(np.float64)}
+
+
+def dump_outputs(arrays: dict, out_dir: str, limit: int = DUMP_BYTES, suffix: str = "") -> None:
+    """Writes every array as out_dir/<name><suffix>.npy, at most `limit` bytes in all.  Small arrays are kept whole; one
+    that does not fit its share of what is left is cut to a seeded sample of its rows, the same rows for the same shape."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    room = limit - 4096 * len(arrays)  # what the .npy headers leave
+    names = sorted(arrays, key=lambda n: arrays[n].nbytes)
+    for i, name in enumerate(names):
+        a = arrays[name]
+        share = room // (len(names) - i)
+        if a.nbytes > share:
+            rows = share // (a.nbytes // len(a))
+            a = a[np.unique(np.random.default_rng(0).integers(0, len(a), rows))]
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+        room -= a.nbytes
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -306,7 +344,14 @@ def main():
     ap.add_argument("--error-rate", type=float, default=None, help="variant: override the configuration's per-base substitution rate")
     ap.add_argument("--minimizer", type=int, default=0)
     ap.add_argument("--bin-target", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (contigs, or the count table for config 3) as DIR/<name>.npy, "
+                         "float32 / float64, at most 64 MB in all (a seeded sample of rows beyond that); N > 1: one file set per rank")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm returns no arrays")
     # stdout carries exactly one JSON line: everything else any library prints goes to stderr, and the line itself is
     # written to the saved descriptor at the end
     sys.stdout.flush()
@@ -441,6 +486,8 @@ def main():
     t_dev, stats, launches, _ = timed(args.steps, False)
     clocks = sampler.stop()
     shard_st = ctx.shard_stats() if world > 1 else None
+    if args.dump_outputs:
+        dump_outputs(result_arrays(ctx, mode), args.dump_outputs, DUMP_BYTES // world, f"_rank{rank}" if world > 1 else "")
     d_text = None  # the end-to-end steps upload from the pinned host copy: give the device copy back first
     torch.cuda.empty_cache()
     t_e2e, d2h_bytes = None, 0
