@@ -248,10 +248,12 @@ int rfx_load_counts_device(rfx_ctx* ctx, const void* d_keys, const uint32_t* d_c
  * rfx_count_sharded / rfx_assemble_sharded are collective: every rank must call them (from its own host thread or
  * process); they meet in cross-GPU barriers and fail with RFX_E_STATE if a peer never arrives.  Ranks that share a device
  * inside one process meet on the host instead and need CUDA_MODULE_LOADING=EAGER in the environment (no kernel may be
- * loaded lazily while a peer on the same device waits).  rfx_assemble_sharded needs the table rfx_count_sharded left (rows
- * sharded by minimiser bin); a table loaded with rfx_load_counts is assembled with rfx_assemble.
- * On return from rfx_count_sharded the context holds its shard of the global table (the rows whose minimiser bin it
- * owns; rfx_counts_* work on it); after rfx_assemble_sharded it holds the contigs whose first k-mer it owns
+ * loaded lazily while a peer on the same device waits).  rfx_assemble_sharded needs a table sharded by minimiser bin: the
+ * one rfx_count_sharded leaves, or a loaded one after rfx_shard_table:
+ *   every rank:  ... rfx_shard_connect -> { rfx_reset, rfx_load_counts* (any slice, may be empty), rfx_shard_table,
+ *                rfx_assemble_sharded, results }*
+ * On return from rfx_count_sharded / rfx_shard_table the context holds its shard of the global table (the rows whose
+ * minimiser bin it owns; rfx_counts_* work on it); after rfx_assemble_sharded it holds the contigs whose first k-mer it owns
  * (rfx_contigs_* work on them): the union over the ranks is the result of the single-GPU calls. */
 #define RFX_SHARD_HANDLE_BYTES 128
 #define RFX_SHARD_MAX_RANKS 8
@@ -266,6 +268,8 @@ typedef struct {
     float ms_comm;                /* barriers + value exchanges of the last sharded calls */
     int32_t fell_back;            /* last rfx_assemble_sharded met a closed path: rank 0 assembled the whole table */
 } rfx_shard_stats_t;
+/* Arena size: rfx_shard_table needs about twice its share of the table in the arena
+ * (send buffer + new table, 2 * (8 or 16 + 4) bytes a row), plus the loaded slice when the new table outgrows it. */
 int rfx_shard_init(rfx_ctx* ctx, int32_t rank, int32_t world, uint64_t arena_bytes /* 0: half of the free device memory */);
 int rfx_shard_export(rfx_ctx* ctx, void* handle /* RFX_SHARD_HANDLE_BYTES */);
 int rfx_shard_connect(rfx_ctx* ctx, const void* handles /* world * RFX_SHARD_HANDLE_BYTES, rank order */, int32_t world);
@@ -273,6 +277,14 @@ int rfx_shard_connect(rfx_ctx* ctx, const void* handles /* world * RFX_SHARD_HAN
  * front it lets rfx_push_fastq scan each uploaded chunk straight into the slabs; otherwise the ranks agree on it. */
 int rfx_shard_set_bins(rfx_ctx* ctx, uint32_t n_bins_total);
 int rfx_count_sharded(rfx_ctx* ctx);
+/* Collective re-shard of a loaded table: every rank holds a slice loaded with rfx_load_counts / rfx_load_counts_device
+ * (slices may be empty and uneven); on return every rank holds exactly the rows whose minimiser bin it owns, as after
+ * rfx_count_sharded.  Rows are neither merged nor de-duplicated, their order inside a shard is unspecified.  The bin
+ * count B is the one of rfx_shard_set_bins if the caller set one (the same on every rank), else
+ * rfx_choose_bins(ctx, 64 * global rows, world) -- what counting from reads picks at typical coverage, ~100 rows a bin.
+ * A rank without a table, a different k or a B that is no multiple of world makes EVERY rank fail with the same error
+ * (RFX_E_STATE / RFX_E_INVALID) after the first exchange.  rfx_stats: ms_partition is the call's time. */
+int rfx_shard_table(rfx_ctx* ctx);
 int rfx_assemble_sharded(rfx_ctx* ctx);
 int rfx_shard_stats(rfx_ctx* ctx, rfx_shard_stats_t* out);
 

@@ -73,6 +73,7 @@ public final class ReflexivCuda implements AutoCloseable {
     private static final MethodHandle SHARD_EXPORT = h("rfx_shard_export", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));
     private static final MethodHandle SHARD_CONNECT = h("rfx_shard_connect", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT));
     private static final MethodHandle COUNT_SHARDED = h("rfx_count_sharded", FunctionDescriptor.of(JAVA_INT, ADDRESS));
+    private static final MethodHandle SHARD_TABLE = h("rfx_shard_table", FunctionDescriptor.of(JAVA_INT, ADDRESS));
     private static final MethodHandle ASSEMBLE_SHARDED = h("rfx_assemble_sharded", FunctionDescriptor.of(JAVA_INT, ADDRESS));
     public static final int SHARD_HANDLE_BYTES = 128;
 
@@ -155,6 +156,10 @@ public final class ReflexivCuda implements AutoCloseable {
 
     /** collective: every rank calls it from its own thread */
     public void countSharded() { call(() -> (int) COUNT_SHARDED.invoke(ctx)); }
+
+    /** collective, after every rank loaded any slice of a Count_k table (loadCounts, may be empty): afterwards this rank holds
+     *  the rows whose minimiser bin it owns, as after countSharded(), and assembleSharded() follows */
+    public void shardTable() { call(() -> (int) SHARD_TABLE.invoke(ctx)); }
 
     /** collective: every rank calls it from its own thread */
     public void assembleSharded() { call(() -> (int) ASSEMBLE_SHARDED.invoke(ctx)); }

@@ -387,26 +387,76 @@ struct Rank {
     int rc = RFX_OK;
     const char* what = "";
 };
-static int run_sharded(int n_gpus, rfx_params p, bool counter, const std::string& pattern, const std::string& outdir, const std::string& target, bool gz) {
+// Contexts for n_gpus ranks (fewer devices than ranks: ranks share devices, how a one-GPU box runs this path), each with its
+// peer-visible arena, connected to each other.  On failure everything is destroyed and false returned.
+static void destroy_ranks(std::vector<Rank>& R) {
+    for (auto& k : R) if (k.c) rfx_destroy(k.c);
+    R.clear();
+}
+static bool open_ranks(int n_gpus, rfx_params p, std::vector<Rank>& R) {
     int32_t n_dev = 0;
-    if (rfx_device_count(&n_dev) != RFX_OK || n_dev < 1) { fprintf(stderr, "reflexiv: no CUDA device\n"); return 1; }
-    std::vector<Rank> R(n_gpus);
+    if (rfx_device_count(&n_dev) != RFX_OK || n_dev < 1) { fprintf(stderr, "reflexiv: no CUDA device\n"); return false; }
+    R.assign(n_gpus, Rank());
     const int dev0 = p.device;
     for (int r = 0; r < n_gpus; r++) {
-        p.device = (dev0 + r) % n_dev;  // fewer devices than ranks: ranks share devices (how a one-GPU box runs this path)
-        if (rfx_create(&R[r].c, &p) != RFX_OK) { fprintf(stderr, "reflexiv: rfx_create (rank %d): %s\n", r, rfx_last_error(nullptr)); return 1; }
+        p.device = (dev0 + r) % n_dev;
+        if (rfx_create(&R[r].c, &p) != RFX_OK) { fprintf(stderr, "reflexiv: rfx_create (rank %d): %s\n", r, rfx_last_error(nullptr)); destroy_ranks(R); return false; }
     }
-    auto destroy_all = [&] { for (auto& k : R) if (k.c) rfx_destroy(k.c); };
     uint64_t arena = getenv("REFLEXIV_ARENA_MB") ? (uint64_t)atoll(getenv("REFLEXIV_ARENA_MB")) << 20 : 0;
-    if (!arena && n_dev < n_gpus) { fprintf(stderr, "reflexiv: %d ranks on %d device(s): set REFLEXIV_ARENA_MB (device memory per rank)\n", n_gpus, n_dev); destroy_all(); return 1; }
+    if (!arena && n_dev < n_gpus) { fprintf(stderr, "reflexiv: %d ranks on %d device(s): set REFLEXIV_ARENA_MB (device memory per rank)\n", n_gpus, n_dev); destroy_ranks(R); return false; }
     std::vector<unsigned char> blobs((size_t)n_gpus * RFX_SHARD_HANDLE_BYTES);
     for (int r = 0; r < n_gpus; r++) {
         if (rfx_shard_init(R[r].c, r, n_gpus, arena) != RFX_OK || rfx_shard_export(R[r].c, blobs.data() + (size_t)r * RFX_SHARD_HANDLE_BYTES) != RFX_OK) {
-            fprintf(stderr, "reflexiv: rfx_shard_init (rank %d): %s\n", r, rfx_last_error(R[r].c)); destroy_all(); return 1;
+            fprintf(stderr, "reflexiv: rfx_shard_init (rank %d): %s\n", r, rfx_last_error(R[r].c)); destroy_ranks(R); return false;
         }
     }
     for (int r = 0; r < n_gpus; r++)
-        if (rfx_shard_connect(R[r].c, blobs.data(), n_gpus) != RFX_OK) { fprintf(stderr, "reflexiv: rfx_shard_connect (rank %d): %s\n", r, rfx_last_error(R[r].c)); destroy_all(); return 1; }
+        if (rfx_shard_connect(R[r].c, blobs.data(), n_gpus) != RFX_OK) { fprintf(stderr, "reflexiv: rfx_shard_connect (rank %d): %s\n", r, rfx_last_error(R[r].c)); destroy_ranks(R); return false; }
+    return true;
+}
+// the collective stages, one thread per rank; false (every failure reported) if a rank failed
+static bool run_ranks(std::vector<Rank>& R, const std::function<void(Rank&, int)>& body) {
+    std::vector<std::thread> th;
+    for (int r = 0; r < (int)R.size(); r++) th.emplace_back([&, r] { body(R[r], r); });
+    for (auto& t : th) t.join();
+    bool ok = true;
+    for (int r = 0; r < (int)R.size(); r++)
+        if (R[r].rc != RFX_OK) { fprintf(stderr, "reflexiv: %s (rank %d): %s\n", R[r].what, r, rfx_last_error(R[r].c)); ok = false; }
+    return ok;
+}
+// one part file per rank (contig ids continue across ranks) + _SUCCESS
+static int write_ranks(std::vector<Rank>& R, bool counter, const std::string& outdir, const std::string& target, bool gz) {
+    const int n_gpus = (int)R.size();
+    mkdir(outdir.c_str(), 0755);
+    mkdir(target.c_str(), 0755);
+    if (counter) clear_dir(target);
+    uint64_t id_base = 0;
+    rfx_stats_t tot;
+    memset(&tot, 0, sizeof(tot));
+    for (int r = 0; r < n_gpus; r++) {
+        uint64_t n = 0;
+        const bool ok = counter ? write_csv_part(R[r].c, false, target, r, gz) : write_contig_part(R[r].c, target, r, id_base, gz, &n);
+        if (!ok) { fprintf(stderr, "reflexiv: writing the output of rank %d failed: %s\n", r, rfx_last_error(R[r].c)); destroy_ranks(R); return 1; }
+        id_base += n;
+        rfx_stats_t s;
+        rfx_stats(R[r].c, &s);
+        tot.n_reads += s.n_reads; tot.n_instances += s.n_instances; tot.n_distinct += s.n_distinct; tot.n_rows += s.n_rows; tot.n_contigs += s.n_contigs;
+    }
+    FILE* okf = fopen((target + "/_SUCCESS").c_str(), "wb");
+    if (okf) fclose(okf);
+    rfx_shard_stats_t sh;
+    rfx_shard_stats(R[0].c, &sh);
+    char msg[512];
+    snprintf(msg, sizeof(msg), "done on %d ranks: %llu reads, %llu k-mers, %llu distinct, %llu rows, %llu contigs; rank 0: %llu neighbour probes answered by a peer, %.2f ms in barriers",
+             n_gpus, (unsigned long long)tot.n_reads, (unsigned long long)tot.n_instances, (unsigned long long)tot.n_distinct, (unsigned long long)tot.n_rows,
+             (unsigned long long)tot.n_contigs, (unsigned long long)sh.n_remote_probes, sh.ms_comm);
+    info(msg);
+    destroy_ranks(R);
+    return 0;
+}
+static int run_sharded(int n_gpus, rfx_params p, bool counter, const std::string& pattern, const std::string& outdir, const std::string& target, bool gz) {
+    std::vector<Rank> R;
+    if (!open_ranks(n_gpus, p, R)) return 1;
     // input: every file is cut into n_gpus runs of whole records (`run`) or whole lines (`counter`); rank r takes the r-th run of every file
     bool push_ok = true;
     const bool read_ok = stream_inputs(pattern, [&](const char* data, size_t n) {
@@ -435,48 +485,44 @@ static int run_sharded(int n_gpus, rfx_params p, bool counter, const std::string
     });
     if (!read_ok || !push_ok) {
         for (int r = 0; r < n_gpus; r++) if (R[r].rc != RFX_OK) fprintf(stderr, "reflexiv: %s (rank %d): %s\n", R[r].what, r, rfx_last_error(R[r].c));
-        destroy_all();
+        destroy_ranks(R);
         return 1;
     }
-    // collective stages, one thread per rank
-    std::vector<std::thread> th;
-    for (int r = 0; r < n_gpus; r++)
-        th.emplace_back([&, r] {
-            Rank& k = R[r];
-            k.what = "rfx_count_sharded";
-            if ((k.rc = rfx_count_sharded(k.c)) != RFX_OK) return;
-            if (!counter) { k.what = "rfx_assemble_sharded"; k.rc = rfx_assemble_sharded(k.c); }
-        });
-    for (auto& t : th) t.join();
-    for (int r = 0; r < n_gpus; r++)
-        if (R[r].rc != RFX_OK) { fprintf(stderr, "reflexiv: %s (rank %d): %s\n", R[r].what, r, rfx_last_error(R[r].c)); push_ok = false; }
-    if (!push_ok) { destroy_all(); return 1; }
-    mkdir(outdir.c_str(), 0755);
-    mkdir(target.c_str(), 0755);
-    if (counter) clear_dir(target);
-    uint64_t id_base = 0;
-    rfx_stats_t tot;
-    memset(&tot, 0, sizeof(tot));
-    for (int r = 0; r < n_gpus; r++) {
-        uint64_t n = 0;
-        const bool ok = counter ? write_csv_part(R[r].c, false, target, r, gz) : write_contig_part(R[r].c, target, r, id_base, false, &n);
-        if (!ok) { fprintf(stderr, "reflexiv: writing the output of rank %d failed: %s\n", r, rfx_last_error(R[r].c)); destroy_all(); return 1; }
-        id_base += n;
-        rfx_stats_t s;
-        rfx_stats(R[r].c, &s);
-        tot.n_reads += s.n_reads; tot.n_instances += s.n_instances; tot.n_distinct += s.n_distinct; tot.n_rows += s.n_rows; tot.n_contigs += s.n_contigs;
-    }
-    FILE* okf = fopen((target + "/_SUCCESS").c_str(), "wb");
-    if (okf) fclose(okf);
-    rfx_shard_stats_t sh;
-    rfx_shard_stats(R[0].c, &sh);
-    char msg[512];
-    snprintf(msg, sizeof(msg), "done on %d ranks: %llu reads, %llu k-mers, %llu distinct, %llu rows, %llu contigs; rank 0: %llu neighbour probes answered by a peer, %.2f ms in barriers",
-             n_gpus, (unsigned long long)tot.n_reads, (unsigned long long)tot.n_instances, (unsigned long long)tot.n_distinct, (unsigned long long)tot.n_rows,
-             (unsigned long long)tot.n_contigs, (unsigned long long)sh.n_remote_probes, sh.ms_comm);
-    info(msg);
-    destroy_all();
-    return 0;
+    const bool ok = run_ranks(R, [&](Rank& k, int) {
+        k.what = "rfx_count_sharded";
+        if ((k.rc = rfx_count_sharded(k.c)) != RFX_OK) return;
+        if (!counter) { k.what = "rfx_assemble_sharded"; k.rc = rfx_assemble_sharded(k.c); }
+    });
+    if (!ok) { destroy_ranks(R); return 1; }
+    return write_ranks(R, counter, outdir, target, counter && gz);  // -gzip applies to contigs from a count table only
+}
+// `run -kmerc <glob> --gpus N`: the table is parsed on the host (cover <= count <= maxcov), rank r loads the r-th contiguous
+// slice of its rows, rfx_shard_table sends every row to the owner of its minimiser bin, then the sharded assembly
+static int run_kmerc_sharded(int n_gpus, rfx_params p, const std::string& pattern, const std::string& outdir, const std::string& target, bool gz) {
+    std::vector<uint64_t> keys;
+    std::vector<uint32_t> counts;
+    bool well_formed = true;
+    const bool read_ok = stream_inputs(pattern, [&](const char* data, size_t n) {
+        well_formed = parse_counts(data, n, p.kmer_size, p.min_kmer_coverage, p.max_kmer_coverage, keys, counts);
+        return well_formed;
+    });
+    if (!well_formed) fprintf(stderr, "reflexiv: malformed k-mer count row\n");
+    if (!read_ok) return 1;
+    std::vector<Rank> R;
+    if (!open_ranks(n_gpus, p, R)) return 1;
+    const uint64_t rows = counts.size();
+    const size_t words = p.kmer_size <= 31 ? 1 : (size_t)(p.kmer_size / 32 + 1);
+    const bool ok = run_ranks(R, [&](Rank& k, int r) {
+        const uint64_t lo = rows * (uint64_t)r / (uint64_t)n_gpus, hi = rows * (uint64_t)(r + 1) / (uint64_t)n_gpus;
+        k.what = "rfx_load_counts";
+        if ((k.rc = rfx_load_counts(k.c, keys.data() + lo * words, counts.data() + lo, hi - lo)) != RFX_OK) return;
+        k.what = "rfx_shard_table";
+        if ((k.rc = rfx_shard_table(k.c)) != RFX_OK) return;
+        k.what = "rfx_assemble_sharded";
+        k.rc = rfx_assemble_sharded(k.c);
+    });
+    if (!ok) { destroy_ranks(R); return 1; }
+    return write_ranks(R, false, outdir, target, gz);
 }
 
 int main(int argc, char** argv) {
@@ -580,10 +626,11 @@ int main(int argc, char** argv) {
         return 1;
     }
 
-    if (n_gpus > 1 && (from_kmer || sorter)) { fprintf(stderr, "reflexiv: --gpus applies to runs from reads (-fastq); this one starts from a count table\n"); n_gpus = 1; }
+    if (n_gpus > 1 && (sorter || stitch)) { fprintf(stderr, "reflexiv: --gpus applies to runs from reads (-fastq) and to -kmerc runs without -stitch; this one runs on one GPU\n"); n_gpus = 1; }
     if (n_gpus > RFX_SHARD_MAX_RANKS) { fprintf(stderr, "reflexiv: --gpus %d: at most %d\n", n_gpus, RFX_SHARD_MAX_RANKS); return 1; }
     if (n_gpus > 1) {
         info("Initiating CUDA contexts ...");
+        if (from_kmer) return run_kmerc_sharded(n_gpus, p, v["kmerc"], outdir, target, gz);
         return run_sharded(n_gpus, p, counter, v["fastq"], outdir, target, gz);
     }
     info("Initiating CUDA context ...");

@@ -32,6 +32,15 @@ template <class KT> __device__ __forceinline__ void kmer_minima(KT X, int k, int
         }
     }
 }
+// minimiser bin of a row (a canonical k-mer): the smaller of its two minima, or its one m-mer when m == k (that m-mer lies
+// in neither the prefix nor the suffix part).  The shard that owns the bin owns the row: rfx_shard_table routes rows by it
+// and the sharded graph stages expect every row there.  The two minima are returned as well.
+template <class KT> __device__ __forceinline__ uint32_t row_bin(KT key, int k, int m, uint32_t n_bins, uint32_t& pre_min, uint32_t& suf_min) {
+    kmer_minima<KT>(key, k, m, pre_min, suf_min);
+    uint32_t h = pre_min < suf_min ? pre_min : suf_min;
+    if (m == k) h = mm_hash_m((uint32_t)key, m);
+    return bin_of_minimizer(h, n_bins);
+}
 // hash of the last m-mer of (S + b) / the first m-mer of (a + S), S a right-aligned (k-1)-mer
 template <class KT> __device__ __forceinline__ uint32_t last_mm_of(KT S, uint32_t b, int m) {
     const uint32_t low = (m >= 17) ? 0u : ((uint32_t)S & ((m >= 16) ? 0x3fffffffu : ((1u << (2 * (m - 1))) - 1u)));

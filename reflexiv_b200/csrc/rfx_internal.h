@@ -194,7 +194,8 @@ struct Ctx {
     uint32_t sh_bins = 0;                           // total bin count of sharded counting (0: agreed on per run)
     uint32_t sh_bins_run = 0;                       // ... the one in force for the slab scan (rfx_partition.cu: slab_begin)
     uint64_t sh_inst_global = 0;                    // k-mer instances extracted by all ranks
-    uint64_t sh_rows_global = 0;                    // rows of all shard tables (known to every rank after rfx_count_sharded)
+    uint64_t sh_rows_global = 0;                    // rows of all shard tables (known to every rank after rfx_count_sharded / rfx_shard_table)
+    DevBuf sh_send;                                 // rfx_shard_table: the loaded rows grouped by owner, pulled by the owners
     cudaEvent_t ev_comm[2] = {nullptr, nullptr};
     float ms_comm = 0;                              // cross-GPU barriers + value exchanges of the last sharded calls
     void* hbar = nullptr;                           // host-side barrier of ranks that share a device inside one process
@@ -278,7 +279,9 @@ int stage_stitch_begin(Ctx* c);
 int stitch_scan_reads(Ctx* c, const uint8_t* d_text, const uint64_t* rd_src, const uint32_t* rd_len, uint64_t n_reads);
 int stage_stitch_finish(Ctx* c);
 uint32_t choose_bin_count(const Ctx* c, uint64_t instances, int n_shards);
+void set_minimizer(Ctx* c, uint32_t n_bins_total);  // c->m from the TOTAL bin count (rfx_partition.cu)
 int stage_count_sharded(Ctx* c);
+int stage_shard_table(Ctx* c);
 int stage_assemble_sharded(Ctx* c);
 void shard_release(Ctx* c);
 

@@ -521,7 +521,7 @@ uint32_t choose_bin_count(const Ctx* c, uint64_t instances, int n_shards) {
 // Minimiser length.  Bins are whole minimiser values, so there must be many more values than bins or the bins come
 // out uneven: 4^11 / 2 = 2.1 M canonical 11-mers serve up to 2^16 bins, beyond that 15-mers (5.4 * 10^8 values).  The
 // rule depends on the TOTAL bin count only, so every rank of a sharded run derives the same m.
-static void set_minimizer(Ctx* c, uint32_t n_bins_total) {
+void set_minimizer(Ctx* c, uint32_t n_bins_total) {
     int m = c->prm.minimizer_len > 0 ? c->prm.minimizer_len : (n_bins_total > 65536u ? 15 : 11);
     if (m > 16) m = 16;
     if (m > c->k) m = c->k;

@@ -25,6 +25,7 @@
 #include <map>
 #include <mutex>
 
+#include "rfx_graph.cuh"
 #include "rfx_internal.h"
 #include "rfx_shard.h"
 
@@ -244,6 +245,200 @@ int stage_count_sharded(Ctx* c) {
     return RFX_OK;
 }
 
+// ---- re-sharding a loaded table (rfx_shard_table) ------------------------------------------------------------------
+// A Count_<k> table read from disk arrives in arbitrary slices.  Every rank routes its rows to the owner of their minimiser
+// bin (the very map the sharded graph stages expect), scatters them grouped by owner into a send buffer in its arena, and
+// every owner pulls its rows out of every rank's send buffer with one kernel: the table is then laid out as
+// rfx_count_sharded leaves it.  About 12 B per row (k <= 31) cross the links once.
+template <class KT>
+__global__ void table_route_kernel(const KT* __restrict__ keys, uint64_t n_rows, int k, int m, uint32_t B, uint32_t bps, uint8_t* __restrict__ owner,
+                                   unsigned long long* __restrict__ hist) {
+    __shared__ unsigned int s_hist[RFX_MAX_RANKS];
+    if (threadIdx.x < RFX_MAX_RANKS) s_hist[threadIdx.x] = 0;
+    __syncthreads();
+    for (uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n_rows; r += (uint64_t)gridDim.x * blockDim.x) {
+        uint32_t a, b;
+        const uint32_t o = row_bin<KT>(keys[r], k, m, B, a, b) / bps;
+        owner[r] = (uint8_t)o;
+        atomicAdd(&s_hist[o], 1u);
+    }
+    __syncthreads();
+    if (threadIdx.x < RFX_MAX_RANKS && s_hist[threadIdx.x]) atomicAdd(&hist[threadIdx.x], (unsigned long long)s_hist[threadIdx.x]);
+}
+
+// rows -> send buffer grouped by owner; the lanes of a warp that go to the same owner take their places with one atomic
+template <class KT>
+__global__ void table_scatter_kernel(const KT* __restrict__ keys, const uint32_t* __restrict__ counts, const uint8_t* __restrict__ owner, uint64_t n_rows,
+                                     unsigned long long* __restrict__ cursor, KT* __restrict__ out_keys, uint32_t* __restrict__ out_counts) {
+    const unsigned lane = threadIdx.x & 31u;
+    const uint64_t warps = (uint64_t)gridDim.x * (blockDim.x >> 5);
+    for (uint64_t base = ((uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * 32u; base < n_rows; base += warps * 32u) {
+        const uint64_t r = base + lane;
+        const bool valid = r < n_rows;
+        const int o = valid ? (int)owner[r] : -1;
+        const unsigned same = __match_any_sync(0xffffffffu, o);
+        const int leader = __ffs(same) - 1;
+        unsigned long long at = 0;
+        if (valid && (int)lane == leader) at = atomicAdd(&cursor[o], (unsigned long long)__popc(same));
+        at = __shfl_sync(0xffffffffu, at, leader);
+        if (valid) {
+            at += (unsigned long long)__popc(same & ((1u << lane) - 1u));
+            out_keys[at] = keys[r];
+            out_counts[at] = counts[r];
+        }
+    }
+}
+
+// what an owner pulls: sender q's rows for it start at keys[q] / counts[q] (addresses as seen from this device) and land at
+// [start[q], start[q + 1]) of the new table
+struct TablePull {
+    const void* keys[RFX_MAX_RANKS];
+    const uint32_t* counts[RFX_MAX_RANKS];
+    unsigned long long start[RFX_MAX_RANKS + 1];
+    int n;
+};
+template <class KT>
+__global__ void table_pull_kernel(const __grid_constant__ TablePull P, KT* __restrict__ keys, uint32_t* __restrict__ counts) {
+    const uint64_t total = P.start[P.n];
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (uint64_t)gridDim.x * blockDim.x) {
+        int q = 0;
+        while (i >= P.start[q + 1]) q++;
+        const uint64_t j = i - P.start[q];
+        keys[i] = reinterpret_cast<const KT*>(P.keys[q])[j];
+        counts[i] = P.counts[q][j];
+    }
+}
+
+static unsigned table_grid(uint64_t n) {
+    const uint64_t g = (n + 255) / 256, cap = (uint64_t)sm_count() * 8;
+    return (unsigned)(g < 1 ? 1 : g > cap ? cap : g);
+}
+
+// send buffer: [histogram per owner | cursor per owner] (256 B), keys (16-byte aligned), counts, owner of every row
+static size_t send_keys_off() { return 256; }
+static size_t send_counts_off(uint64_t n, size_t ksz) { return send_keys_off() + ((n * ksz + 255) & ~(size_t)255); }
+static size_t send_owner_off(uint64_t n, size_t ksz) { return send_counts_off(n, ksz) + ((n * sizeof(uint32_t) + 255) & ~(size_t)255); }
+
+template <class KT> static int table_route_scatter(Ctx* c, uint32_t B, uint32_t bps, unsigned long long* hist) {
+    cudaStream_t st = c->stream;
+    const uint64_t n = c->n_rows;
+    const size_t ksz = sizeof(KT);
+    RFX_TRY(devbuf_reserve(c, c->sh_send, send_owner_off(n, ksz) + n + 256));
+    uint8_t* s = c->sh_send.as<uint8_t>();
+    unsigned long long* d_hist = reinterpret_cast<unsigned long long*>(s);
+    uint8_t* owner = s + send_owner_off(n, ksz);
+    RFX_CUDA(c, cudaMemsetAsync(d_hist, 0, RFX_MAX_RANKS * sizeof(unsigned long long), st));
+    if (n) {
+        table_route_kernel<KT><<<table_grid(n), 256, 0, st>>>(c->keys.as<KT>(), n, c->k, c->m, B, bps, owner, d_hist);
+        c->launches++;
+        RFX_CUDA(c, cudaGetLastError());
+    }
+    RFX_CUDA(c, cudaMemcpyAsync(hist, d_hist, RFX_MAX_RANKS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    RFX_CUDA(c, cudaStreamSynchronize(st));
+    unsigned long long cur[RFX_MAX_RANKS], sum = 0;
+    for (int o = 0; o < RFX_MAX_RANKS; o++) { cur[o] = sum; sum += hist[o]; }
+    if (sum != n) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: routed %llu of %llu rows", sum, (unsigned long long)n);
+    if (n) {
+        RFX_CUDA(c, cudaMemcpyAsync(d_hist + RFX_MAX_RANKS, cur, sizeof(cur), cudaMemcpyHostToDevice, st));
+        table_scatter_kernel<KT><<<table_grid(n), 256, 0, st>>>(c->keys.as<KT>(), c->counts.as<uint32_t>(), owner, n, d_hist + RFX_MAX_RANKS,
+                                                                reinterpret_cast<KT*>(s + send_keys_off()), reinterpret_cast<uint32_t*>(s + send_counts_off(n, ksz)));
+        c->launches++;
+        RFX_CUDA(c, cudaGetLastError());
+    }
+    return RFX_OK;
+}
+
+template <class KT> static int table_pull(Ctx* c, const TablePull& P) {
+    const uint64_t recv = P.start[P.n];
+    RFX_TRY(devbuf_reserve(c, c->keys, (recv + 1) * sizeof(KT)));
+    RFX_TRY(devbuf_reserve(c, c->counts, (recv + 1) * sizeof(uint32_t)));
+    if (recv) {
+        table_pull_kernel<KT><<<table_grid(recv), 256, 0, c->stream>>>(P, c->keys.as<KT>(), c->counts.as<uint32_t>());
+        c->launches++;
+        RFX_CUDA(c, cudaGetLastError());
+    }
+    return RFX_OK;
+}
+
+int stage_shard_table(Ctx* c) {
+    if (c->sh_world < 1 || !c->peer_base[c->sh_rank]) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: call rfx_shard_init / rfx_shard_connect first");
+    const int world = c->sh_world, me = c->sh_rank;
+    unsigned long long mine[3 + RFX_MAX_RANKS], all[RFX_MAX_RANKS * RFX_PUB_SLOTS] = {};
+    auto got = [&](int r, int slot) { return all[(size_t)r * RFX_PUB_SLOTS + PUB_TABLE + slot]; };
+    c->st_active = false;
+    c->ms_comm = 0;
+    stage_begin(c);
+    // 1. what every rank holds.  Every rank checks every rank's values in the same order, so that all ranks return the same
+    //    error together instead of leaving their peers in a barrier
+    mine[0] = c->have_counts ? 1 : 0;
+    mine[1] = c->have_counts ? c->n_rows : 0;
+    mine[2] = (unsigned long long)c->k;
+    mine[3] = c->sh_bins;
+    RFX_TRY(shard_exchange(c, PUB_TABLE, 4, mine, all));
+    uint64_t rows_global = 0;
+    for (int r = 0; r < world; r++) {
+        if (!got(r, 0)) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: rank %d holds no count table (every rank loads a slice first, an empty one will do)", r);
+        if (got(r, 2) != got(0, 2)) return ctx_fail(c, RFX_E_INVALID, "rfx_shard_table: rank %d has k = %llu, rank 0 k = %llu", r, got(r, 2), got(0, 2));
+        if (got(r, 3) != got(0, 3)) return ctx_fail(c, RFX_E_INVALID, "rfx_shard_table: rank %d set %llu bins, rank 0 %llu", r, got(r, 3), got(0, 3));
+        rows_global += got(r, 1);
+    }
+    // the bin count: the caller's, or the one counting from reads picks for this many rows at typical coverage (~100 rows a bin)
+    uint32_t B = (uint32_t)got(0, 3);
+    if (!B) B = choose_bin_count(c, 64 * rows_global, world);
+    if (B % (uint32_t)world) return ctx_fail(c, RFX_E_INVALID, "rfx_shard_table: %u bins are not a multiple of %d ranks", B, world);
+    const uint32_t bps = B / (uint32_t)world;
+    set_minimizer(c, B);
+    // 2. own rows -> send buffer grouped by owner.  A rank that fails here still takes part in the next exchange
+    unsigned long long hist[RFX_MAX_RANKS] = {0};
+    const int rc_send = c->wide ? table_route_scatter<u128>(c, B, bps, hist) : table_route_scatter<uint64_t>(c, B, bps, hist);
+    const size_t ksz = c->wide ? sizeof(u128) : sizeof(uint64_t);
+    const unsigned long long send_at = c->sh_send.p ? (unsigned long long)(c->sh_send.as<uint8_t>() - c->arena) : 0ull;
+    mine[0] = rc_send == RFX_OK ? 0 : 1;
+    mine[1] = send_at + send_keys_off();
+    mine[2] = send_at + send_counts_off(c->n_rows, ksz);
+    for (int o = 0; o < world; o++) mine[3 + o] = hist[o];
+    RFX_TRY(shard_exchange(c, PUB_TABLE, 3 + world, mine, all));
+    if (rc_send != RFX_OK) return rc_send;
+    uint64_t sent = 0;
+    for (int r = 0; r < world; r++) {
+        if (got(r, 0)) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: rank %d could not route its rows", r);
+        for (int o = 0; o < world; o++) sent += got(r, 3 + o);
+    }
+    if (sent != rows_global) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: %llu rows routed, %llu loaded", (unsigned long long)sent, (unsigned long long)rows_global);
+    // 3. pull the own rows out of every rank's send buffer
+    TablePull P;
+    memset(&P, 0, sizeof(P));
+    P.n = world;
+    for (int q = 0; q < world; q++) {
+        uint64_t before = 0;  // rows of sender q that go to lower ranks
+        for (int o = 0; o < me; o++) before += got(q, 3 + o);
+        P.keys[q] = c->peer_base[q] + got(q, 1) + before * ksz;
+        P.counts[q] = reinterpret_cast<const uint32_t*>(c->peer_base[q] + got(q, 2)) + before;
+        P.start[q + 1] = P.start[q] + got(q, 3 + me);
+    }
+    const uint64_t recv = P.start[world];
+    const int rc_recv = c->wide ? table_pull<u128>(c, P) : table_pull<uint64_t>(c, P);
+    // 4. nobody may reuse its send buffer before every owner has pulled: one more exchange, which also checks the total
+    mine[0] = rc_recv == RFX_OK ? 0 : 1;
+    mine[1] = recv;
+    RFX_TRY(shard_exchange(c, PUB_TABLE, 2, mine, all));
+    if (rc_recv != RFX_OK) return rc_recv;
+    uint64_t received = 0;
+    for (int r = 0; r < world; r++) {
+        if (got(r, 0)) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: rank %d could not receive its rows", r);
+        received += got(r, 1);
+    }
+    if (received != rows_global) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: %llu rows received, %llu sent", (unsigned long long)received, (unsigned long long)rows_global);
+    c->ms[1] = stage_end(c);
+    c->sh_rows_global = rows_global;
+    c->n_rows = recv;
+    c->table_cap = recv + 1;
+    c->n_bins = B;
+    c->have_counts = true;
+    c->have_contigs = false; c->have_sorted = false;
+    return RFX_OK;
+}
+
 }  // namespace rfx
 
 using namespace rfx;
@@ -359,6 +554,12 @@ int rfx_count_sharded(rfx_ctx* c) {
     if (!c) return RFX_E_INVALID;
     cudaSetDevice(c->prm.device);
     return stage_count_sharded(c);
+}
+
+int rfx_shard_table(rfx_ctx* c) {
+    if (!c) return RFX_E_INVALID;
+    cudaSetDevice(c->prm.device);
+    return stage_shard_table(c);
 }
 
 int rfx_assemble_sharded(rfx_ctx* c) {

@@ -33,6 +33,7 @@ struct PeerBases {
 enum {
     PUB_INSTANCES = 0,
     PUB_SLAB_REC = 1,   // 8 slots: slab records, slab counts, slab cap, overflow records, overflow offsets, n overflow, bins, instances
+    PUB_TABLE = 1,      // rfx_shard_table, 3 + RFX_MAX_RANKS slots (never in use together with PUB_SLAB_REC)
     PUB_GRAPH = 12,     // rfx_shard_graph.cu: GPub
     PUB_END = RFX_PUB_SLOTS
 };

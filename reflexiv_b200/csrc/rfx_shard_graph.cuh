@@ -293,11 +293,8 @@ __global__ void sg_row_minima_kernel(const KT* __restrict__ keys, uint64_t n_row
     for (uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n_rows; r += (uint64_t)gridDim.x * blockDim.x) {
         const KT key = keys[r];
         uint32_t a, b;
-        kmer_minima<KT>(key, k, m, a, b);
+        const uint32_t bin = row_bin<KT>(key, k, m, B, a, b);
         rmin[r] = make_uint4(a, b, bin_of_minimizer(a, B), bin_of_minimizer(b, B));
-        uint32_t h = a < b ? a : b;
-        if (m == k) h = mm_hash_m((uint32_t)key, m);  // one m-mer, in neither the prefix nor the suffix part
-        const uint32_t bin = bin_of_minimizer(h, B);
         if (bin < bin_lo || bin >= bin_hi) atomicExch(&dstat[DS_GRAPH_ERR], 3ull);
         const uint64_t bit = (uint64_t)bin * rb + (((uint64_t)(uint32_t)key_hash(key) * rb) >> 32);
         atomicOr(&filter[bit >> 5], 1u << (bit & 31u));

@@ -295,6 +295,12 @@ class ReflexivContext:
         self._check(self.L.rfx_count_sharded(self._ctx), self._ctx)
         return self.stats()
 
+    def shard_table(self):
+        """Collective: every rank calls it after loading any slice of a count table (load_counts*, may be empty).  On return
+        this context holds the rows whose minimiser bin it owns, as after count_sharded()."""
+        self._check(self.L.rfx_shard_table(self._ctx), self._ctx)
+        return self.stats()
+
     def assemble_sharded(self):
         """Collective.  On return this context holds the contigs whose first k-mer it owns."""
         self._check(self.L.rfx_assemble_sharded(self._ctx), self._ctx)
