@@ -161,7 +161,8 @@ int rfx_oriented_copy(rfx_ctx* ctx, uint64_t* keys_hi, uint64_t* keys_lo, int32_
  *   min_repeat_fold     param.minRepeatFold    (util/DefaultParam.java:107: 1.5)
  *   max_kmer_size       param.kmerListInt[last] (util/DefaultParam.java:87: 95 for the default list)
  * RFX_E_UNSUPPORTED where the reference itself cannot run: min_error_coverage == 0, (k-1) % 31 == 0.
- * Invalidates the results of rfx_assemble (the graph index and flag arrays are shared). */
+ * Invalidates the results of rfx_assemble (the graph index and flag arrays are shared).
+ * rfx_sort_kmers_sharded (multi-GPU block below) is the same stage on a table sharded across ranks. */
 int rfx_sort_kmers(rfx_ctx* ctx, int32_t min_error_coverage, double min_repeat_fold, int32_t max_kmer_size);
 int rfx_sorted_size(rfx_ctx* ctx, uint64_t* n_rows);
 /* oriented k-mers (right-aligned, hi/lo halves) with their flags; caller buffers of n_rows elements each */
@@ -251,10 +252,11 @@ int rfx_load_counts_device(rfx_ctx* ctx, const void* d_keys, const uint32_t* d_c
  * loaded lazily while a peer on the same device waits).  rfx_assemble_sharded needs a table sharded by minimiser bin: the
  * one rfx_count_sharded leaves, or a loaded one after rfx_shard_table:
  *   every rank:  ... rfx_shard_connect -> { rfx_reset, rfx_load_counts* (any slice, may be empty), rfx_shard_table,
- *                rfx_assemble_sharded, results }*
+ *                rfx_assemble_sharded | rfx_sort_kmers_sharded, results }*
  * On return from rfx_count_sharded / rfx_shard_table the context holds its shard of the global table (the rows whose
  * minimiser bin it owns; rfx_counts_* work on it); after rfx_assemble_sharded it holds the contigs whose first k-mer it owns
- * (rfx_contigs_* work on them): the union over the ranks is the result of the single-GPU calls. */
+ * (rfx_contigs_* work on them), after rfx_sort_kmers_sharded the Count_<k>_sorted rows of its shard (rfx_sorted_* work on
+ * them): the union over the ranks is the result of the single-GPU calls. */
 #define RFX_SHARD_HANDLE_BYTES 128
 #define RFX_SHARD_MAX_RANKS 8
 typedef struct {
@@ -262,14 +264,20 @@ typedef struct {
     uint64_t arena_bytes, arena_used;
     uint64_t n_instances_global;  /* k-mer instances extracted by all ranks */
     uint64_t n_shard_instances;   /* ... that fell into this rank's bins */
-    uint64_t n_rows_global, n_oriented_global, n_contigs_global, n_contig_bases_global;
-    uint64_t n_remote_probes;     /* neighbour requests of peers this rank answered from its index (last rfx_assemble_sharded) */
+    uint64_t n_rows_global, n_oriented_global, n_contigs_global, n_contig_bases_global;  /* after rfx_sort_kmers_sharded:
+                                     n_oriented_global = Count_<k>_sorted rows of all ranks, no contigs */
+    uint64_t n_remote_probes;     /* neighbour requests of peers this rank answered from its index (last rfx_assemble_sharded
+                                     or rfx_sort_kmers_sharded) */
     uint64_t n_l1_splitters, n_l2_splitters;
     float ms_comm;                /* barriers + value exchanges of the last sharded calls */
     int32_t fell_back;            /* last rfx_assemble_sharded met a closed path: rank 0 assembled the whole table */
 } rfx_shard_stats_t;
 /* Arena size: rfx_shard_table needs about twice its share of the table in the arena
- * (send buffer + new table, 2 * (8 or 16 + 4) bytes a row), plus the loaded slice when the new table outgrows it. */
+ * (send buffer + new table, 2 * (8 or 16 + 4) bytes a row), plus the loaded slice when the new table outgrows it.
+ * rfx_sort_kmers_sharded needs, besides the shard table, about 106 bytes per own row (two oriented k-mers of 37 bytes:
+ * flags, alive byte, output flags, work list; 32 bytes of minima and index) plus the request / answer channels, world *
+ * (global rows / world + 65536) * (32 or 48) bytes, plus the replicated presence bits, 2 bytes per global row (8 at least
+ * per bin). */
 int rfx_shard_init(rfx_ctx* ctx, int32_t rank, int32_t world, uint64_t arena_bytes /* 0: half of the free device memory */);
 int rfx_shard_export(rfx_ctx* ctx, void* handle /* RFX_SHARD_HANDLE_BYTES */);
 int rfx_shard_connect(rfx_ctx* ctx, const void* handles /* world * RFX_SHARD_HANDLE_BYTES, rank order */, int32_t world);
@@ -286,6 +294,16 @@ int rfx_count_sharded(rfx_ctx* ctx);
  * (RFX_E_STATE / RFX_E_INVALID) after the first exchange.  rfx_stats: ms_partition is the call's time. */
 int rfx_shard_table(rfx_ctx* ctx);
 int rfx_assemble_sharded(rfx_ctx* ctx);
+/* Collective Count_<k>_sorted on a table sharded by minimiser bin (after rfx_count_sharded or rfx_shard_table): the same
+ * arguments, domain and results as rfx_sort_kmers.  On return every rank holds the sorted rows of its own shard
+ * (rfx_sorted_size / rfx_sorted_copy / rfx_sorted_csv); their union over the ranks equals, bit for bit, what rfx_sort_kmers
+ * gives on one context holding the whole table.  Like rfx_sort_kmers it takes the index and the flag arrays over: the
+ * contigs of an earlier rfx_assemble_sharded are gone (RFX_E_STATE), a later rfx_assemble_sharded rebuilds them.  The ranks
+ * agree on their arguments before any barrier, so a misuse makes EVERY rank fail with the same error at once: arguments
+ * that differ between ranks RFX_E_INVALID, a rank without a sharded table RFX_E_STATE, min_error_coverage == 0 or
+ * (k-1) % 31 == 0 RFX_E_UNSUPPORTED, more than 2^28 rows on a rank RFX_E_CAPACITY.  rfx_stats: ms_graph is the call's time;
+ * rfx_shard_stats: ms_comm and n_remote_probes cover the call. */
+int rfx_sort_kmers_sharded(rfx_ctx* ctx, int32_t min_error_coverage, double min_repeat_fold, int32_t max_kmer_size);
 int rfx_shard_stats(rfx_ctx* ctx, rfx_shard_stats_t* out);
 
 /* number of CUDA devices the library can use (a launcher maps ranks to devices with it) */

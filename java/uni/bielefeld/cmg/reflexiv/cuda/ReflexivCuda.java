@@ -75,6 +75,7 @@ public final class ReflexivCuda implements AutoCloseable {
     private static final MethodHandle COUNT_SHARDED = h("rfx_count_sharded", FunctionDescriptor.of(JAVA_INT, ADDRESS));
     private static final MethodHandle SHARD_TABLE = h("rfx_shard_table", FunctionDescriptor.of(JAVA_INT, ADDRESS));
     private static final MethodHandle ASSEMBLE_SHARDED = h("rfx_assemble_sharded", FunctionDescriptor.of(JAVA_INT, ADDRESS));
+    private static final MethodHandle SORT_KMERS_SHARDED = h("rfx_sort_kmers_sharded", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_DOUBLE, JAVA_INT));
     public static final int SHARD_HANDLE_BYTES = 128;
 
     /** One contig as the reference's DSKmerToContig sees it: bases plus the two end flags of the header. */
@@ -227,6 +228,13 @@ public final class ReflexivCuda implements AutoCloseable {
     /** Count_<k>_sorted (ReflexivDSKmerLeftAndRightSorting.java:105-243): rows `KMER,1|left|right\n`. */
     public byte[] sortedCsv(int minErrorCoverage, double minRepeatFold, int maxKmerSize) {
         call(() -> (int) SORT_KMERS.invoke(ctx, minErrorCoverage, minRepeatFold, maxKmerSize));
+        return csv(SORTED_CSV);
+    }
+
+    /** collective Count_<k>_sorted on a sharded table (after countSharded() or shardTable()): every rank calls it from its own
+     *  thread and gets the rows of its own shard; their union is what sortedCsv() gives on one context holding the whole table */
+    public byte[] sortKmersSharded(int minErrorCoverage, double minRepeatFold, int maxKmerSize) {
+        call(() -> (int) SORT_KMERS_SHARDED.invoke(ctx, minErrorCoverage, minRepeatFold, maxKmerSize));
         return csv(SORTED_CSV);
     }
 

@@ -424,20 +424,24 @@ static bool run_ranks(std::vector<Rank>& R, const std::function<void(Rank&, int)
         if (R[r].rc != RFX_OK) { fprintf(stderr, "reflexiv: %s (rank %d): %s\n", R[r].what, r, rfx_last_error(R[r].c)); ok = false; }
     return ok;
 }
+// what a rank writes: its contigs (Assemble_<k> or the run's output directory), its Count_<k> rows or its Count_<k>_sorted rows
+enum class Output { contigs, counts, sorted };
 // one part file per rank (contig ids continue across ranks) + _SUCCESS
-static int write_ranks(std::vector<Rank>& R, bool counter, const std::string& outdir, const std::string& target, bool gz) {
+static int write_ranks(std::vector<Rank>& R, Output what, const std::string& outdir, const std::string& target, bool gz) {
     const int n_gpus = (int)R.size();
     mkdir(outdir.c_str(), 0755);
     mkdir(target.c_str(), 0755);
-    if (counter) clear_dir(target);
-    uint64_t id_base = 0;
+    if (what != Output::contigs) clear_dir(target);
+    uint64_t id_base = 0, n_sorted = 0;
     rfx_stats_t tot;
     memset(&tot, 0, sizeof(tot));
     for (int r = 0; r < n_gpus; r++) {
         uint64_t n = 0;
-        const bool ok = counter ? write_csv_part(R[r].c, false, target, r, gz) : write_contig_part(R[r].c, target, r, id_base, gz, &n);
+        const bool ok = what == Output::contigs ? write_contig_part(R[r].c, target, r, id_base, gz, &n)
+                                                : write_csv_part(R[r].c, what == Output::sorted, target, r, gz) && (what != Output::sorted || rfx_sorted_size(R[r].c, &n) == RFX_OK);
         if (!ok) { fprintf(stderr, "reflexiv: writing the output of rank %d failed: %s\n", r, rfx_last_error(R[r].c)); destroy_ranks(R); return 1; }
-        id_base += n;
+        if (what == Output::contigs) id_base += n;
+        else n_sorted += n;
         rfx_stats_t s;
         rfx_stats(R[r].c, &s);
         tot.n_reads += s.n_reads; tot.n_instances += s.n_instances; tot.n_distinct += s.n_distinct; tot.n_rows += s.n_rows; tot.n_contigs += s.n_contigs;
@@ -447,9 +451,9 @@ static int write_ranks(std::vector<Rank>& R, bool counter, const std::string& ou
     rfx_shard_stats_t sh;
     rfx_shard_stats(R[0].c, &sh);
     char msg[512];
-    snprintf(msg, sizeof(msg), "done on %d ranks: %llu reads, %llu k-mers, %llu distinct, %llu rows, %llu contigs; rank 0: %llu neighbour probes answered by a peer, %.2f ms in barriers",
+    snprintf(msg, sizeof(msg), "done on %d ranks: %llu reads, %llu k-mers, %llu distinct, %llu rows, %llu %s; rank 0: %llu neighbour probes answered by a peer, %.2f ms in barriers",
              n_gpus, (unsigned long long)tot.n_reads, (unsigned long long)tot.n_instances, (unsigned long long)tot.n_distinct, (unsigned long long)tot.n_rows,
-             (unsigned long long)tot.n_contigs, (unsigned long long)sh.n_remote_probes, sh.ms_comm);
+             (unsigned long long)(what == Output::sorted ? n_sorted : tot.n_contigs), what == Output::sorted ? "sorted rows" : "contigs", (unsigned long long)sh.n_remote_probes, sh.ms_comm);
     info(msg);
     destroy_ranks(R);
     return 0;
@@ -494,20 +498,34 @@ static int run_sharded(int n_gpus, rfx_params p, bool counter, const std::string
         if (!counter) { k.what = "rfx_assemble_sharded"; k.rc = rfx_assemble_sharded(k.c); }
     });
     if (!ok) { destroy_ranks(R); return 1; }
-    return write_ranks(R, counter, outdir, target, counter && gz);  // -gzip applies to contigs from a count table only
+    return write_ranks(R, counter ? Output::counts : Output::contigs, outdir, target, counter && gz);  // -gzip applies to contigs from a count table only
 }
-// `run -kmerc <glob> --gpus N`: the table is parsed on the host (cover <= count <= maxcov), rank r loads the r-th contiguous
-// slice of its rows, rfx_shard_table sends every row to the owner of its minimiser bin, then the sharded assembly
-static int run_kmerc_sharded(int n_gpus, rfx_params p, const std::string& pattern, const std::string& outdir, const std::string& target, bool gz) {
-    std::vector<uint64_t> keys;
-    std::vector<uint32_t> counts;
+// The arguments of the Count_<k>_sorted stage (`sort`): E is rfx_params.min_error_coverage
+struct SortStage {
+    double min_repeat_fold;
+    int32_t max_kmer_size;
+    bool k_listed;  // k is in -klist: otherwise no row takes part (ReflexivDSKmerLeftAndRightSorting.java:1695)
+};
+// Reads a Count_<k> table the way the one-GPU `run -kmerc` / `sort` does: run keeps cover <= count <= maxcov
+// (ReflexivDSMain.java:405-412), sort count <= maxcov only (ReflexivDSKmerLeftAndRightSorting.java:186-193) and only k-mers whose
+// length is in the list.  False (reported) on a file that cannot be read.
+static bool read_count_table(const std::string& pattern, const rfx_params& p, const SortStage* sort, std::vector<uint64_t>& keys, std::vector<uint32_t>& counts) {
     bool well_formed = true;
     const bool read_ok = stream_inputs(pattern, [&](const char* data, size_t n) {
-        well_formed = parse_counts(data, n, p.kmer_size, p.min_kmer_coverage, p.max_kmer_coverage, keys, counts);
+        well_formed = parse_counts(data, n, p.kmer_size, sort ? INT32_MIN : p.min_kmer_coverage, p.max_kmer_coverage, keys, counts);
         return well_formed;
     });
+    if (sort && !sort->k_listed) { keys.clear(); counts.clear(); }
     if (!well_formed) fprintf(stderr, "reflexiv: malformed k-mer count row\n");
-    if (!read_ok) return 1;
+    return read_ok;
+}
+// `run -kmerc <glob> --gpus N` / `sort -kmerc <glob> --gpus N`: the table is parsed on the host (read_count_table), rank r loads
+// the r-th contiguous slice of its rows, rfx_shard_table sends every row to the owner of its minimiser bin, then the sharded
+// assembly or (sort != nullptr) the sharded Count_<k>_sorted stage
+static int run_kmerc_sharded(int n_gpus, rfx_params p, const SortStage* sort, const std::string& pattern, const std::string& outdir, const std::string& target, bool gz) {
+    std::vector<uint64_t> keys;
+    std::vector<uint32_t> counts;
+    if (!read_count_table(pattern, p, sort, keys, counts)) return 1;
     std::vector<Rank> R;
     if (!open_ranks(n_gpus, p, R)) return 1;
     const uint64_t rows = counts.size();
@@ -518,11 +536,16 @@ static int run_kmerc_sharded(int n_gpus, rfx_params p, const std::string& patter
         if ((k.rc = rfx_load_counts(k.c, keys.data() + lo * words, counts.data() + lo, hi - lo)) != RFX_OK) return;
         k.what = "rfx_shard_table";
         if ((k.rc = rfx_shard_table(k.c)) != RFX_OK) return;
-        k.what = "rfx_assemble_sharded";
-        k.rc = rfx_assemble_sharded(k.c);
+        if (sort) {
+            k.what = "rfx_sort_kmers_sharded";
+            k.rc = rfx_sort_kmers_sharded(k.c, p.min_error_coverage, sort->min_repeat_fold, sort->max_kmer_size);
+        } else {
+            k.what = "rfx_assemble_sharded";
+            k.rc = rfx_assemble_sharded(k.c);
+        }
     });
     if (!ok) { destroy_ranks(R); return 1; }
-    return write_ranks(R, false, outdir, target, gz);
+    return write_ranks(R, sort ? Output::sorted : Output::contigs, outdir, target, gz);
 }
 
 int main(int argc, char** argv) {
@@ -611,6 +634,7 @@ int main(int argc, char** argv) {
         }
     }
     const double min_repeat_fold = v.count("accurate") ? 2.0 : 1.5;  // DefaultParam.java:107
+    const SortStage sort_stage{min_repeat_fold, klist.back() /* param.kmerListInt[last], :445 */, std::find(klist.begin(), klist.end(), p.kmer_size) != klist.end()};
     if (!v.count("outfile")) { info("Output file not set of -outfile options"); return 0; }
     const std::string outdir = v["outfile"];
     p.counter_mode = counter ? 1 : 0;
@@ -626,11 +650,11 @@ int main(int argc, char** argv) {
         return 1;
     }
 
-    if (n_gpus > 1 && (sorter || stitch)) { fprintf(stderr, "reflexiv: --gpus applies to runs from reads (-fastq) and to -kmerc runs without -stitch; this one runs on one GPU\n"); n_gpus = 1; }
+    if (n_gpus > 1 && stitch) { fprintf(stderr, "reflexiv: --gpus applies to runs from reads (-fastq), to -kmerc runs without -stitch and to sort; this one runs on one GPU\n"); n_gpus = 1; }
     if (n_gpus > RFX_SHARD_MAX_RANKS) { fprintf(stderr, "reflexiv: --gpus %d: at most %d\n", n_gpus, RFX_SHARD_MAX_RANKS); return 1; }
     if (n_gpus > 1) {
         info("Initiating CUDA contexts ...");
-        if (from_kmer) return run_kmerc_sharded(n_gpus, p, v["kmerc"], outdir, target, gz);
+        if (from_kmer) return run_kmerc_sharded(n_gpus, p, sorter ? &sort_stage : nullptr, v["kmerc"], outdir, target, gz);
         return run_sharded(n_gpus, p, counter, v["fastq"], outdir, target, gz);
     }
     info("Initiating CUDA context ...");
@@ -639,16 +663,7 @@ int main(int argc, char** argv) {
     if (from_kmer) {
         std::vector<uint64_t> keys;
         std::vector<uint32_t> counts;
-        bool well_formed = true;
-        const bool read_ok = stream_inputs(v["kmerc"], [&](const char* data, size_t n) {
-            // run: cover <= count <= maxcov (ReflexivDSMain.java:405-412); sort: count <= maxcov only
-            // (ReflexivDSKmerLeftAndRightSorting.java:186-193) and only k-mers whose length is in the list (:1695)
-            well_formed = parse_counts(data, n, p.kmer_size, sorter ? INT32_MIN : p.min_kmer_coverage, p.max_kmer_coverage, keys, counts);
-            return well_formed;
-        });
-        if (sorter && std::find(klist.begin(), klist.end(), p.kmer_size) == klist.end()) { keys.clear(); counts.clear(); }
-        if (!well_formed) fprintf(stderr, "reflexiv: malformed k-mer count row\n");
-        if (!read_ok) { rfx_destroy(c); return 1; }
+        if (!read_count_table(v["kmerc"], p, sorter ? &sort_stage : nullptr, keys, counts)) { rfx_destroy(c); return 1; }
         if (rfx_load_counts(c, keys.data(), counts.data(), counts.size()) != RFX_OK) return fail(c, "rfx_load_counts");
     } else {
         bool push_ok = true, pushed = false;
@@ -664,7 +679,7 @@ int main(int argc, char** argv) {
     }
     mkdir(outdir.c_str(), 0755);
     if (counter || sorter) {
-        if (sorter && rfx_sort_kmers(c, p.min_error_coverage, min_repeat_fold, klist.back() /* param.kmerListInt[last], :445 */) != RFX_OK)
+        if (sorter && rfx_sort_kmers(c, p.min_error_coverage, sort_stage.min_repeat_fold, sort_stage.max_kmer_size) != RFX_OK)
             return fail(c, "rfx_sort_kmers");
         mkdir(target.c_str(), 0755);
         clear_dir(target);

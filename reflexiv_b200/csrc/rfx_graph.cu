@@ -895,8 +895,8 @@ template <class KT> static int sorted_impl(Ctx* c, int E, double fold, int X) {
     return RFX_OK;
 }
 
-int stage_sorted(Ctx* c, int E, double fold, int max_kmer_size) {
-    if (!c->have_counts) return ctx_fail(c, RFX_E_STATE, "rfx_sort_kmers: no count table (call rfx_count or rfx_load_counts first)");
+// the working domain of the reference's sorting stage (rfx_sort_kmers, rfx_sort_kmers_sharded)
+static int sorted_domain(Ctx* c, const char* who, int E, double fold, int max_kmer_size) {
     if (E == 0)
         return ctx_fail(c, RFX_E_UNSUPPORTED,
                         "min_error_coverage 0 selects DSFilterForkSubKmer, which reads five columns from a three-column row "
@@ -904,7 +904,13 @@ int stage_sorted(Ctx* c, int E, double fold, int max_kmer_size) {
     if (c->k < 2 || (c->k - 1) % 31 == 0)
         return ctx_fail(c, RFX_E_UNSUPPORTED, "k = %d: DSForwardSubKmerExtraction takes the last base from the wrong block when (k-1) %% 31 == 0 "
                         "(ReflexivDSKmerLeftAndRightSorting.java:930-936)", c->k);
-    if (!(fold > 0) || max_kmer_size < 1 || max_kmer_size + 3 >= 30000) return ctx_fail(c, RFX_E_INVALID, "rfx_sort_kmers: bad fold / max_kmer_size");
+    if (!(fold > 0) || max_kmer_size < 1 || max_kmer_size + 3 >= 30000) return ctx_fail(c, RFX_E_INVALID, "%s: bad fold / max_kmer_size", who);
+    return RFX_OK;
+}
+
+int stage_sorted(Ctx* c, int E, double fold, int max_kmer_size) {
+    if (!c->have_counts) return ctx_fail(c, RFX_E_STATE, "rfx_sort_kmers: no count table (call rfx_count or rfx_load_counts first)");
+    RFX_TRY(sorted_domain(c, "rfx_sort_kmers", E, fold, max_kmer_size));
     return c->wide ? sorted_impl<u128>(c, E, fold, max_kmer_size + 3) : sorted_impl<uint64_t>(c, E, fold, max_kmer_size + 3);
 }
 

@@ -283,6 +283,7 @@ void set_minimizer(Ctx* c, uint32_t n_bins_total);  // c->m from the TOTAL bin c
 int stage_count_sharded(Ctx* c);
 int stage_shard_table(Ctx* c);
 int stage_assemble_sharded(Ctx* c);
+int stage_sorted_sharded(Ctx* c, int min_error_coverage, double min_repeat_fold, int max_kmer_size);
 void shard_release(Ctx* c);
 
 inline void stage_begin(Ctx* c) { cudaEventRecord(c->ev0, c->stream); }

@@ -568,6 +568,13 @@ int rfx_assemble_sharded(rfx_ctx* c) {
     return stage_assemble_sharded(c);
 }
 
+int rfx_sort_kmers_sharded(rfx_ctx* c, int32_t min_error_coverage, double min_repeat_fold, int32_t max_kmer_size) {
+    if (!c) return RFX_E_INVALID;
+    cudaSetDevice(c->prm.device);
+    c->st_active = false;  // an open stitch stage is abandoned, as in rfx_sort_kmers
+    return stage_sorted_sharded(c, min_error_coverage, min_repeat_fold, max_kmer_size);
+}
+
 int rfx_device_count(int32_t* n_devices) {
     if (!n_devices) return RFX_E_INVALID;
     int n = 0;

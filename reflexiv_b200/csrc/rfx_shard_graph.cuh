@@ -107,6 +107,7 @@ struct SGProbe {
     uint32_t gid;    // oriented node (NONE32: no such k-mer)
     uint32_t count;
     uint32_t alive;  // its alive byte (when asked for)
+    uint32_t w;      // word w of an owner's answer: the candidate's right flag in the sorted filters' serve mode (0 otherwise)
 };
 // a request to the owner of a k-mer / its answer
 template <class KT> struct alignas(16) SGReq {
@@ -136,15 +137,16 @@ template <class KT> __device__ __forceinline__ uint32_t sg_lookup_own(const SGPe
 //           (ref = SG_REF_ASK | owner); sg_finish_pass1 turns the marks of a block into requests in the owners' inboxes and
 //           ref = owner << 29 | position, which says where the answer will be.  The node has to wait.
 //   PASS 2  (nodes that waited) a candidate with a ref takes the owner's answer, the others are looked up again.
-template <class KT, int PASS, bool WANT_ALIVE>
+// SORTED: a local candidate is read as sg_serve_kernel<SORTED> answers for a remote one: count = its lflag, w = its rflag.
+template <class KT, int PASS, bool WANT_ALIVE, bool SORTED = false>
 __device__ __forceinline__ SGProbe sg_probe(const SGView& V, KT Z, uint32_t h_new, uint32_t h_side, uint32_t bin_side, uint32_t oid, int stage, uint32_t& ref,
                                             unsigned long long* dstat) {
-    SGProbe out{NONE32, 0u, 0u};
+    SGProbe out{NONE32, 0u, 0u, 0u};
     if (PASS == 2 && ref != NONE32) {
         const uint4 a = V.p[V.me].respbox[(uint64_t)(ref >> 29) * V.chan_cap + (ref & SG_REF_MASK)];
 
         out.gid = a.y == NONE32 ? NONE32 : gid_make((int)(ref >> 29), a.y);
-        out.count = a.x; out.alive = a.z;
+        out.count = a.x; out.alive = a.z; out.w = a.w;
         return out;
     }
     const KT zc = revcomp(Z, V.k);
@@ -164,13 +166,16 @@ __device__ __forceinline__ SGProbe sg_probe(const SGView& V, KT Z, uint32_t h_ne
     if (v == NONE32) return out;
     const uint32_t y = 2u * v + (fwd ? 0u : 1u);
     out.gid = gid_make(V.me, y);
-    out.count = Me.counts[v];
+    out.count = SORTED ? (uint32_t)Me.lflag[y] : Me.counts[v];
     if (WANT_ALIVE) out.alive = Me.alive[y];
+    if (SORTED) out.w = (uint32_t)Me.rflag[y];
     return out;
 }
 // The owner's side: every request of every peer is looked up in the own index, the answer goes into the asker's answer box.
 // LINK: a surviving node that is asked for by its predecessor notes that predecessor (the asker links to it in its second pass).
-template <class KT, bool LINK>
+// SORTED (left filter of rfx_sort_kmers_sharded): the answer is {coverage, node, alive byte, right flag} as the right filter left
+// them on the node (lflag / rflag) instead of {count, node, alive byte, 0}.
+template <class KT, bool LINK, bool SORTED = false>
 __global__ void __launch_bounds__(256) sg_serve_kernel(const __grid_constant__ SGView V, int stage, unsigned long long* dstat) {
     const SGPeer& Me = V.p[V.me];
     unsigned long long served = 0;
@@ -186,7 +191,8 @@ __global__ void __launch_bounds__(256) sg_serve_kernel(const __grid_constant__ S
             uint4 a = make_uint4(0u, NONE32, 0u, 0u);
             if (v != NONE32) {
                 const uint32_t y = 2u * v + ((rq.oid & 0x80000000u) ? 0u : 1u);
-                a.x = Me.counts[v]; a.y = y; a.z = Me.alive[y];
+                a.x = SORTED ? (uint32_t)Me.lflag[y] : Me.counts[v]; a.y = y; a.z = Me.alive[y];
+                if (SORTED) a.w = (uint32_t)Me.rflag[y];
                 if (LINK && (a.z & 2)) Me.pred[y] = gid_make(r, rq.oid & SG_REF_MASK);  // the left filter left at most one predecessor
             }
             out[i] = a;  // posted store into the asker's memory
@@ -435,6 +441,100 @@ __global__ void __launch_bounds__(256, 8) sg_link_kernel(const __grid_constant__
             }
         }
         if (PASS == 1) sg_finish_pass1<KT>(V, W, 2, oid, ref, [&](uint32_t b) { return (KT)((suffix << 2) | (KT)b); }, dstat);
+    }
+}
+
+// ---- Count_<k>_sorted across ranks (rfx_sort_kmers_sharded; the single-GPU sorted_right_kernel / sorted_left_kernel) -------
+// The probes, requests and answers of A7 / A8 (request stages 0 and 1), the rules sorted_right_fork / sorted_left_fork.  The
+// right filter leaves the coverage it carries on in lflag and the right flag in rflag; the left filter needs both of every
+// candidate: a local one's from the own arrays, a remote one's from its owner (sg_serve_kernel<SORTED>: {lflag, node, alive, rflag}).
+template <class KT, int PASS>
+__global__ void __launch_bounds__(256, 8) sg_sorted_right_kernel(const __grid_constant__ SGView V, int E, double fold, int Xf, uint64_t n, const uint4* __restrict__ rmin,
+                                                                 SGWork W, unsigned long long* dstat) {
+    const SGPeer& Me = V.p[V.me];
+    const KT* keys = reinterpret_cast<const KT*>(Me.keys);
+    const uint64_t count = sg_work_count<PASS>(n, W);
+    for (uint64_t i0 = (uint64_t)blockIdx.x * blockDim.x; i0 < count; i0 += (uint64_t)gridDim.x * blockDim.x) {  // block-uniform trip count
+        const uint64_t i = i0 + threadIdx.x;
+        uint32_t ref[4] = {NONE32, NONE32, NONE32, NONE32};
+        uint32_t oid = 0;
+        KT prefix = 0;
+        if (i < count) {
+            if (PASS == 1) oid = (uint32_t)i; else sg_work_pop(W, i, oid, ref);
+            const uint32_t row = oid >> 1;
+            const KT key = keys[row];
+            const KT rc = revcomp(key, V.k);
+            if ((oid & 1u) && rc == key) Me.alive[oid] = 0;  // palindrome: one node, not two
+            else {
+                const KT Xk = (oid & 1u) ? rc : key;
+                prefix = Xk >> 2;
+                const uint32_t myb = (uint32_t)Xk & 3u;
+                const uint4 mm = rmin[row];
+                const uint32_t pre_min = (oid & 1u) ? mm.y : mm.x, pre_bin = (oid & 1u) ? mm.w : mm.z;
+                uint32_t cnt[4];
+                bool dup[4];
+#pragma unroll
+                for (uint32_t b = 0; b < 4; b++) {
+                    if (b == myb) { cnt[b] = Me.counts[row]; dup[b] = (rc == key); }
+                    else {
+                        const KT Z = (prefix << 2) | (KT)b;
+                        const SGProbe pr = sg_probe<KT, PASS, false>(V, Z, last_mm_of<KT>(prefix, b, V.m), pre_min, pre_bin, oid, 0, ref[b], dstat);
+                        cnt[b] = pr.gid == NONE32 ? 0u : pr.count;
+                        dup[b] = (Z == revcomp(Z, V.k));
+                    }
+                }
+                if (PASS == 2 || (ref[0] & ref[1] & ref[2] & ref[3]) == NONE32) {
+                    const SortedFork res = sorted_right_fork(cnt, dup, E, fold, Xf);
+                    const bool won = res.winner == (int)myb;
+                    Me.alive[oid] = won ? 1 : 0;
+                    if (won) { Me.lflag[oid] = res.left; Me.rflag[oid] = res.right; }
+                }
+            }
+        }
+        if (PASS == 1) sg_finish_pass1<KT>(V, W, 0, oid, ref, [&](uint32_t b) { return (KT)((prefix << 2) | (KT)b); }, dstat);
+    }
+}
+
+// A remote candidate's coverage and right flag are read only by its owner's stage-1 serve, which runs behind the barrier that
+// follows every rank's right pass 2: they are final there without a barrier of their own.  Local ones are final once this
+// rank's right pass 2 is (stream order).  The winner writes srt_left / srt_right, never lflag / rflag, which peers may still ask for.
+template <class KT, int PASS>
+__global__ void __launch_bounds__(256, 8) sg_sorted_left_kernel(const __grid_constant__ SGView V, int E, double fold, int Xf, uint64_t n, const uint4* __restrict__ rmin,
+                                                                SGWork W, int32_t* __restrict__ out_left, int32_t* __restrict__ out_right, unsigned long long* dstat) {
+    const SGPeer& Me = V.p[V.me];
+    const int top = 2 * (V.k - 1);
+    const KT sufmask = mask_bases<KT>(V.k - 1);
+    const uint64_t count = sg_work_count<PASS>(n, W);
+    for (uint64_t i0 = (uint64_t)blockIdx.x * blockDim.x; i0 < count; i0 += (uint64_t)gridDim.x * blockDim.x) {
+        const uint64_t i = i0 + threadIdx.x;
+        uint32_t ref[4] = {NONE32, NONE32, NONE32, NONE32};
+        uint32_t oid = 0;
+        KT suffix = 0;
+        if (i < count) {
+            if (PASS == 1) oid = (uint32_t)i; else sg_work_pop(W, i, oid, ref);
+            if (Me.alive[oid] & 1) {
+                const KT Xk = sg_oriented<KT>(V, gid_make(V.me, oid));
+                suffix = Xk & sufmask;
+                const uint32_t mya = (uint32_t)(Xk >> top) & 3u;
+                const uint4 mm = rmin[oid >> 1];
+                const uint32_t suf_min = (oid & 1u) ? mm.x : mm.y, suf_bin = (oid & 1u) ? mm.z : mm.w;
+                int32_t cv[4], rf[4];
+#pragma unroll
+                for (uint32_t a = 0; a < 4; a++) {
+                    cv[a] = 0; rf[a] = 0;
+                    if (a == mya) { cv[a] = Me.lflag[oid]; rf[a] = Me.rflag[oid]; }
+                    else {
+                        const SGProbe pr = sg_probe<KT, PASS, true, true>(V, ((KT)a << top) | suffix, first_mm_of<KT>(suffix, a, V.k, V.m), suf_min, suf_bin, oid, 1, ref[a], dstat);
+                        if (pr.gid != NONE32 && (pr.alive & 1)) { cv[a] = (int32_t)pr.count; rf[a] = (int32_t)pr.w; }
+                    }
+                }
+                if (PASS == 2 || (ref[0] & ref[1] & ref[2] & ref[3]) == NONE32) {
+                    const SortedFork res = sorted_left_fork(cv, rf, E, fold, Xf);
+                    if (res.winner == (int)mya) { Me.alive[oid] = 3; out_left[oid] = res.left; out_right[oid] = res.right; }  // bit 0 stays: others still read it
+                }
+            }
+        }
+        if (PASS == 1) sg_finish_pass1<KT>(V, W, 1, oid, ref, [&](uint32_t a) { return (KT)(((KT)a << top) | suffix); }, dstat);
     }
 }
 
@@ -767,8 +867,10 @@ __global__ void sg_gather_kernel(const __grid_constant__ SGView V, uint64_t m1, 
 }
 
 // ---- host side ------------------------------------------------------------------------------------------------------------
-// RFX_SHARD_PROF=1: event marks between the phases of rfx_assemble_sharded, printed by rank 0 when the call returns
+// RFX_SHARD_PROF=1: event marks between the phases of rfx_assemble_sharded / rfx_sort_kmers_sharded, printed by rank 0 when
+// the call returns
 struct SGProf {
+    const char* what = "rfx_assemble_sharded";
     bool on = false;
     cudaStream_t st = nullptr;
     std::vector<std::pair<const char*, cudaEvent_t>> marks;
@@ -782,7 +884,7 @@ struct SGProf {
     void report(int rank) {
         if (!on) return;
         cudaStreamSynchronize(st);
-        std::string line = "rfx_assemble_sharded rank " + std::to_string(rank) + " [ms]:";
+        std::string line = std::string(what) + " rank " + std::to_string(rank) + " [ms]:";
         for (size_t i = 1; i < marks.size(); i++) {
             float ms = 0;
             cudaEventElapsedTime(&ms, marks[i - 1].second, marks[i].second);
@@ -878,54 +980,43 @@ template <class KT> static int sg_fallback_whole_table(Ctx* c, const SGView& V, 
     return rc;
 }
 
-template <class KT> static int sharded_graph_impl(Ctx* c) {
+// The K5 prologue of rfx_assemble_sharded and rfx_sort_kmers_sharded: the per-node arrays of the fork filters, the index over
+// the own rows, the presence bits of all ranks and the request / answer channels, published to the peers.  `chains`: also the
+// buffers of the chain ranking and the contigs (K6, K7) and their presets.  Every rank must call it (a barrier when world > 1).
+template <class KT> static int sg_k5_prologue(Ctx* c, bool chains, SGView& V, unsigned long long* all, SGProf& prof) {
     cudaStream_t st = c->stream;
-    if (!c->gshard) c->gshard = new GShard();
     GShard* gs = c->gshard;
     const int world = c->sh_world;
     const uint64_t n_rows = c->n_rows, n = 2 * n_rows, nn = n ? n : 1;
     unsigned long long* dstat = c->dstat.as<unsigned long long>();
-    unsigned long long all[RFX_MAX_RANKS * RFX_PUB_SLOTS];
-    if (n >= GID_MASK) return ctx_fail(c, RFX_E_CAPACITY, "sharded assembly: more than 2^28 rows on one rank");
-    if (!c->n_bins || c->n_bins % (uint32_t)world) return ctx_fail(c, RFX_E_STATE, "sharded assembly needs the table of rfx_count_sharded (rows sharded by minimiser bin)");
-    RFX_CUDA(c, cudaMemsetAsync(c->dstat.p, 0, DS_NSLOTS * sizeof(uint64_t), st));
-    c->n_oriented = c->n_budget = c->n_budget_adm = c->n_cycles = c->n_contigs = c->n_contig_bases = 0;
-    c->have_sorted = false; c->have_contigs = false;
-    c->ms_comm = 0;
-    gs->fell_back = 0;
-
-    SGProf prof;
-    prof.on = getenv("RFX_SHARD_PROF") != nullptr && c->sh_rank == 0;
-    prof.st = st;
-    prof.mark("start");
-    // ---- K5 ----
-    stage_begin(c);
     RFX_TRY(devbuf_reserve(c, c->rflag, nn * sizeof(int32_t)));
     RFX_TRY(devbuf_reserve(c, c->lflag, nn * sizeof(int32_t)));
-    RFX_TRY(devbuf_reserve(c, c->eff_l, nn * sizeof(int32_t)));
-    RFX_TRY(devbuf_reserve(c, c->eff_r, nn * sizeof(int32_t)));
     RFX_TRY(devbuf_reserve(c, c->alive, nn + 8));
-    RFX_TRY(devbuf_reserve(c, c->succ, nn * sizeof(uint32_t)));
-    RFX_TRY(devbuf_reserve(c, c->pred, nn * sizeof(uint32_t)));
-    RFX_TRY(devbuf_reserve(c, c->spl_id, nn * sizeof(uint32_t)));
-    RFX_TRY(devbuf_reserve(c, c->spl_node, nn * sizeof(uint32_t)));
-    RFX_TRY(devbuf_reserve(c, c->loc, nn * sizeof(uint64_t)));
-    RFX_TRY(devbuf_reserve(c, c->ad[0], nn * sizeof(uint64_t)));
-    RFX_TRY(devbuf_reserve(c, c->chain_len, nn * sizeof(uint32_t)));
-    RFX_TRY(devbuf_reserve(c, c->ctg_idx, nn * sizeof(uint32_t)));
-    RFX_TRY(devbuf_reserve(c, gs->tail_rf, nn * sizeof(int32_t)));
     RFX_TRY(devbuf_reserve(c, gs->rmin, (n_rows + 1) * sizeof(uint4)));
-    RFX_TRY(devbuf_reserve(c, gs->l1_ent, nn * sizeof(ulonglong2)));
-    RFX_TRY(devbuf_reserve(c, gs->nxt_l1, nn * sizeof(uint32_t)));
-    RFX_TRY(devbuf_reserve(c, gs->l1_loc, nn * sizeof(uint64_t)));
-    RFX_TRY(devbuf_reserve(c, gs->l1_fin, nn * sizeof(uint64_t)));
-    RFX_TRY(devbuf_reserve(c, gs->l1_dst, nn * sizeof(uint64_t)));
-    RFX_TRY(devbuf_reserve(c, gs->l2_l1, nn * sizeof(uint32_t)));
-    RFX_TRY(devbuf_reserve(c, gs->l2_node, nn * sizeof(uint32_t)));
-    for (int i = 0; i < 2; i++) RFX_TRY(devbuf_reserve(c, gs->l2_up[i], nn * sizeof(uint64_t)));
-    RFX_TRY(devbuf_reserve(c, gs->l2_fin, nn * sizeof(uint64_t)));
-    RFX_TRY(devbuf_reserve(c, c->ctg_off, sizeof(uint64_t)));
-    RFX_TRY(devbuf_reserve(c, c->ctg_bases, 16));
+    if (chains) {
+        RFX_TRY(devbuf_reserve(c, c->eff_l, nn * sizeof(int32_t)));
+        RFX_TRY(devbuf_reserve(c, c->eff_r, nn * sizeof(int32_t)));
+        RFX_TRY(devbuf_reserve(c, c->succ, nn * sizeof(uint32_t)));
+        RFX_TRY(devbuf_reserve(c, c->pred, nn * sizeof(uint32_t)));
+        RFX_TRY(devbuf_reserve(c, c->spl_id, nn * sizeof(uint32_t)));
+        RFX_TRY(devbuf_reserve(c, c->spl_node, nn * sizeof(uint32_t)));
+        RFX_TRY(devbuf_reserve(c, c->loc, nn * sizeof(uint64_t)));
+        RFX_TRY(devbuf_reserve(c, c->ad[0], nn * sizeof(uint64_t)));
+        RFX_TRY(devbuf_reserve(c, c->chain_len, nn * sizeof(uint32_t)));
+        RFX_TRY(devbuf_reserve(c, c->ctg_idx, nn * sizeof(uint32_t)));
+        RFX_TRY(devbuf_reserve(c, gs->tail_rf, nn * sizeof(int32_t)));
+        RFX_TRY(devbuf_reserve(c, gs->l1_ent, nn * sizeof(ulonglong2)));
+        RFX_TRY(devbuf_reserve(c, gs->nxt_l1, nn * sizeof(uint32_t)));
+        RFX_TRY(devbuf_reserve(c, gs->l1_loc, nn * sizeof(uint64_t)));
+        RFX_TRY(devbuf_reserve(c, gs->l1_fin, nn * sizeof(uint64_t)));
+        RFX_TRY(devbuf_reserve(c, gs->l1_dst, nn * sizeof(uint64_t)));
+        RFX_TRY(devbuf_reserve(c, gs->l2_l1, nn * sizeof(uint32_t)));
+        RFX_TRY(devbuf_reserve(c, gs->l2_node, nn * sizeof(uint32_t)));
+        for (int i = 0; i < 2; i++) RFX_TRY(devbuf_reserve(c, gs->l2_up[i], nn * sizeof(uint64_t)));
+        RFX_TRY(devbuf_reserve(c, gs->l2_fin, nn * sizeof(uint64_t)));
+        RFX_TRY(devbuf_reserve(c, c->ctg_off, sizeof(uint64_t)));
+        RFX_TRY(devbuf_reserve(c, c->ctg_bases, 16));
+    }
     // the own index: one region, load factor <= 1/4.  Presence bits: a region per minimiser bin of ALL ranks (SGView), the
     // region size from the global row count rfx_count_sharded left behind, so that every rank computes the same
     const uint32_t B = c->n_bins, bps = B / (uint32_t)world;
@@ -950,7 +1041,6 @@ template <class KT> static int sharded_graph_impl(Ctx* c) {
     c->ht_cap = slots; c->g_bins = 1; c->g_m = c->m; c->g_bloom_mask = 0;
 
     // everything is allocated: tell the others where (nothing behind these addresses is valid yet)
-    SGView V;
     RFX_TRY(sg_publish(c, V, nullptr, 0, nullptr, all));
     gs->n_rows_global = sg_sum(all, world, GP_NROWS);
     prof.mark("reserve+publish1");
@@ -981,16 +1071,45 @@ template <class KT> static int sharded_graph_impl(Ctx* c) {
         ht_build_kernel<KT><<<grid_n(n_rows), 256, 0, st>>>(G, nullptr);
         c->launches++;
     }
-    cudaMemsetAsync(c->succ.p, 0xff, nn * sizeof(uint32_t), st);
-    cudaMemsetAsync(c->pred.p, 0xff, nn * sizeof(uint32_t), st);
-    cudaMemsetAsync(c->chain_len.p, 0, nn * sizeof(uint32_t), st);
-    cudaMemsetAsync(gs->tail_rf.p, 0, nn * sizeof(int32_t), st);
-    cudaMemsetAsync(c->loc.p, 0xff, nn * sizeof(uint64_t), st);
-    cudaMemsetAsync(gs->l1_loc.p, 0xff, nn * sizeof(uint64_t), st);
+    if (chains) {
+        cudaMemsetAsync(c->succ.p, 0xff, nn * sizeof(uint32_t), st);
+        cudaMemsetAsync(c->pred.p, 0xff, nn * sizeof(uint32_t), st);
+        cudaMemsetAsync(c->chain_len.p, 0, nn * sizeof(uint32_t), st);
+        cudaMemsetAsync(gs->tail_rf.p, 0, nn * sizeof(int32_t), st);
+        cudaMemsetAsync(c->loc.p, 0xff, nn * sizeof(uint64_t), st);
+        cudaMemsetAsync(gs->l1_loc.p, 0xff, nn * sizeof(uint64_t), st);
+    }
     cudaMemsetAsync(c->alive.p, 0, nn + 8, st);
     prof.mark("memsets+index");
     if (world > 1) RFX_CUDA(c, cudaStreamWaitEvent(st, c->copy_done[1], 0));  // the peers' presence bits have arrived
     prof.mark("filter_wait");
+    return RFX_OK;
+}
+
+template <class KT> static int sharded_graph_impl(Ctx* c) {
+    cudaStream_t st = c->stream;
+    if (!c->gshard) c->gshard = new GShard();
+    GShard* gs = c->gshard;
+    const int world = c->sh_world;
+    const uint64_t n_rows = c->n_rows, n = 2 * n_rows, nn = n ? n : 1;
+    unsigned long long* dstat = c->dstat.as<unsigned long long>();
+    unsigned long long all[RFX_MAX_RANKS * RFX_PUB_SLOTS];
+    if (n >= GID_MASK) return ctx_fail(c, RFX_E_CAPACITY, "sharded assembly: more than 2^28 rows on one rank");
+    if (!c->n_bins || c->n_bins % (uint32_t)world) return ctx_fail(c, RFX_E_STATE, "sharded assembly needs the table of rfx_count_sharded (rows sharded by minimiser bin)");
+    RFX_CUDA(c, cudaMemsetAsync(c->dstat.p, 0, DS_NSLOTS * sizeof(uint64_t), st));
+    c->n_oriented = c->n_budget = c->n_budget_adm = c->n_cycles = c->n_contigs = c->n_contig_bases = 0;
+    c->have_sorted = false; c->have_contigs = false;
+    c->ms_comm = 0;
+    gs->fell_back = 0;
+
+    SGProf prof;
+    prof.on = getenv("RFX_SHARD_PROF") != nullptr && c->sh_rank == 0;
+    prof.st = st;
+    prof.mark("start");
+    // ---- K5 ----
+    stage_begin(c);
+    SGView V;
+    RFX_TRY(sg_k5_prologue<KT>(c, true, V, all, prof));
     // (the peers' indexes are first touched by the answering kernels, behind the barrier that follows the first pass)
     const int E = c->prm.min_error_coverage;
     const uint4* rmin = gs->rmin.as<uint4>();
@@ -1201,6 +1320,127 @@ int stage_assemble_sharded(Ctx* c) {
     if (!c->prm.bubble) return ctx_fail(c, RFX_E_UNSUPPORTED, "-bubble: undefined in the reference (see rfx_assemble)");
     if (c->k < 2) return ctx_fail(c, RFX_E_INVALID, "assembly needs k >= 2");
     return c->wide ? sharded_graph_impl<u128>(c) : sharded_graph_impl<uint64_t>(c);
+}
+
+// ---- Count_<k>_sorted across ranks (rfx_sort_kmers_sharded) -------------------------------------------------------------
+// The K5 prologue of the assembly (no chain or contig buffers), the two sorted filters as request / answer passes, the
+// survivors counted as on one GPU.  A closing exchange makes a channel overflow or a misplaced row on any rank fail every rank.
+template <class KT> static int sharded_sorted_impl(Ctx* c, int E, double fold, int Xf) {
+    cudaStream_t st = c->stream;
+    if (!c->gshard) c->gshard = new GShard();
+    GShard* gs = c->gshard;
+    const int world = c->sh_world;
+    const uint64_t n = 2 * c->n_rows, nn = n ? n : 1;
+    unsigned long long* dstat = c->dstat.as<unsigned long long>();
+    unsigned long long all[RFX_MAX_RANKS * RFX_PUB_SLOTS];
+    RFX_CUDA(c, cudaMemsetAsync(c->dstat.p, 0, DS_NSLOTS * sizeof(uint64_t), st));
+    c->n_sorted = 0;
+    c->have_sorted = false; c->have_contigs = false;  // the index, the alive bytes and the flag arrays are taken over
+    gs->fell_back = 0; gs->n_l1 = gs->n_l2 = 0; gs->n_contigs_global = gs->n_bases_global = 0;
+
+    SGProf prof;
+    prof.what = "rfx_sort_kmers_sharded";
+    prof.on = getenv("RFX_SHARD_PROF") != nullptr && c->sh_rank == 0;
+    prof.st = st;
+    prof.mark("start");
+    RFX_TRY(devbuf_reserve(c, c->srt_left, nn * sizeof(int32_t)));
+    RFX_TRY(devbuf_reserve(c, c->srt_right, nn * sizeof(int32_t)));
+    SGView V;
+    RFX_TRY(sg_k5_prologue<KT>(c, false, V, all, prof));
+    const uint4* rmin = gs->rmin.as<uint4>();
+    // pass 1 over the own nodes (requests out), [barrier], the owners answer, [barrier], pass 2 over the nodes that waited
+    const unsigned g2 = sm_count() * 8u;
+    const SGWork W0{gs->work.as<uint32_t>(), gs->pend_ref.as<uint4>(), dstat + DS_WORK + 0};
+    const SGWork W1{gs->work.as<uint32_t>(), gs->pend_ref.as<uint4>(), dstat + DS_WORK + 1};
+    int32_t* out_l = c->srt_left.as<int32_t>();
+    int32_t* out_r = c->srt_right.as<int32_t>();
+    if (n) sg_sorted_right_kernel<KT, 1><<<grid_n(n), 256, 0, st>>>(V, E, fold, Xf, n, rmin, W0, dstat);
+    prof.mark("right");
+    if (world > 1) {
+        RFX_TRY(shard_barrier(c));
+        sg_serve_kernel<KT, false><<<g2, 256, 0, st>>>(V, 0, dstat);
+        RFX_TRY(shard_barrier(c));
+        prof.mark("right_serve");
+        if (n) sg_sorted_right_kernel<KT, 2><<<g2, 256, 0, st>>>(V, E, fold, Xf, n, rmin, W0, dstat);
+        prof.mark("right2");
+    }
+    if (n) sg_sorted_left_kernel<KT, 1><<<grid_n(n), 256, 0, st>>>(V, E, fold, Xf, n, rmin, W1, out_l, out_r, dstat);
+    prof.mark("left");
+    if (world > 1) {
+        // the first barrier follows every rank's right pass 2: the coverages and right flags this serve answers with are final
+        RFX_TRY(shard_barrier(c));
+        sg_serve_kernel<KT, false, true><<<g2, 256, 0, st>>>(V, 1, dstat);
+        RFX_TRY(shard_barrier(c));
+        prof.mark("left_serve");
+        if (n) sg_sorted_left_kernel<KT, 2><<<g2, 256, 0, st>>>(V, E, fold, Xf, n, rmin, W1, out_l, out_r, dstat);
+        prof.mark("left2");
+    }
+    c->launches += world > 1 ? 6 : 2;
+    // survivors (alive & 2), as rfx_sort_kmers counts them
+    uint64_t total = 0;
+    if (n) {
+        ScanPlan<uint64_t> plan;
+        RFX_TRY(devbuf_reserve(c, c->scan_ws, ScanPlan<uint64_t>::workspace_elems(n) * sizeof(uint64_t)));
+        plan.bind(n, c->scan_ws.as<uint64_t>());
+        scan_prepare(plan, AliveBoth{c->alive.as<uint8_t>()}, OpAddU64{}, (uint64_t)0, st);
+        c->launches += 2 * plan.levels;
+        RFX_CUDA(c, cudaMemcpyAsync(&total, plan.total, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+    }
+    cudaError_t e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return ctx_fail(c, RFX_E_CUDA, "sharded sorted-stage kernels failed: %s", cudaGetErrorString(e));
+    prof.mark("survivors");
+    // [barrier] every rank is done with its channels; survivors and error words of all ranks
+    {
+        const unsigned long long mine[3] = {total, 0, 0};  // slots 1, 2: filled from the device counters
+        const int slots_dev[2] = {DS_GRAPH_ERR, DS_REMOTE};
+        RFX_TRY(shard_exchange(c, PUB_TABLE, 3, mine, all, 2, slots_dev, PUB_TABLE + 1));
+    }
+    prof.mark("exchange");
+    unsigned long long survivors = 0, gerr = 0;
+    for (int r = 0; r < world; r++) {
+        survivors += all[(size_t)r * RFX_PUB_SLOTS + PUB_TABLE];
+        gerr += all[(size_t)r * RFX_PUB_SLOTS + PUB_TABLE + 1];
+    }
+    gs->n_remote = all[(size_t)c->sh_rank * RFX_PUB_SLOTS + PUB_TABLE + 2];
+    gs->n_oriented_global = survivors;
+    c->ms[3] = stage_end(c);
+    prof.report(c->sh_rank);
+    if (gerr) return ctx_fail(c, RFX_E_GRAPH, "sharded sorted filters: a row on a rank that does not own its minimiser bin (code 3) or a request channel that overflowed (4); codes add up to %llu", gerr);
+    c->n_sorted = total;
+    c->have_sorted = true;
+    return RFX_OK;
+}
+
+int stage_sorted_sharded(Ctx* c, int E, double fold, int max_kmer_size) {
+    if (c->sh_world < 1 || !c->peer_base[c->sh_rank]) return ctx_fail(c, RFX_E_STATE, "rfx_sort_kmers_sharded: call rfx_shard_init / rfx_shard_connect first");
+    const int world = c->sh_world;
+    unsigned long long mine[7], all[RFX_MAX_RANKS * RFX_PUB_SLOTS] = {};
+    auto got = [&](int r, int slot) { return all[(size_t)r * RFX_PUB_SLOTS + PUB_TABLE + slot]; };
+    c->ms_comm = 0;
+    stage_begin(c);
+    // What every rank holds and was asked for, before any barrier or buffer.  Every rank checks every rank's values in the same
+    // order, so that all ranks return the same error together instead of leaving their peers in a barrier.
+    unsigned long long fold_bits = 0;
+    memcpy(&fold_bits, &fold, sizeof(fold_bits));
+    mine[0] = c->have_counts && c->n_bins && c->n_bins % (uint32_t)world == 0 ? 1 : 0;
+    mine[1] = (unsigned long long)c->k;
+    mine[2] = c->n_bins;
+    mine[3] = (uint32_t)E;
+    mine[4] = fold_bits;
+    mine[5] = (uint32_t)max_kmer_size;
+    mine[6] = c->have_counts ? c->n_rows : 0;
+    RFX_TRY(shard_exchange(c, PUB_TABLE, 7, mine, all));
+    for (int r = 0; r < world; r++)
+        if (!got(r, 0))
+            return ctx_fail(c, RFX_E_STATE, "rfx_sort_kmers_sharded: rank %d holds no table sharded by minimiser bin (rfx_count_sharded, or rfx_load_counts* and rfx_shard_table first)", r);
+    static const char* what[6] = {"", "k", "bin count", "min_error_coverage", "min_repeat_fold", "max_kmer_size"};
+    for (int r = 1; r < world; r++)
+        for (int s = 1; s < 6; s++)
+            if (got(r, s) != got(0, s)) return ctx_fail(c, RFX_E_INVALID, "rfx_sort_kmers_sharded: rank %d has another %s than rank 0", r, what[s]);
+    RFX_TRY(sorted_domain(c, "rfx_sort_kmers_sharded", E, fold, max_kmer_size));
+    for (int r = 0; r < world; r++)
+        if (2 * got(r, 6) >= GID_MASK) return ctx_fail(c, RFX_E_CAPACITY, "rfx_sort_kmers_sharded: rank %d holds more than 2^28 rows", r);
+    return c->wide ? sharded_sorted_impl<u128>(c, E, fold, max_kmer_size + 3) : sharded_sorted_impl<uint64_t>(c, E, fold, max_kmer_size + 3);
 }
 
 void shard_graph_reset(Ctx* c) {

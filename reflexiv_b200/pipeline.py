@@ -306,6 +306,14 @@ class ReflexivContext:
         self._check(self.L.rfx_assemble_sharded(self._ctx), self._ctx)
         return self.stats()
 
+    def sort_kmers_sharded(self, min_error_coverage: int = 8, min_repeat_fold: float = 1.5, max_kmer_size: int = 95) -> int:
+        """Collective sort_kmers() on a table sharded by minimiser bin (after count_sharded() or shard_table()).  On return this
+        context holds the Count_<k>_sorted rows of its shard (sorted_rows(), sorted_csv()); returns their number."""
+        self._check(self.L.rfx_sort_kmers_sharded(self._ctx, min_error_coverage, min_repeat_fold, max_kmer_size), self._ctx)
+        n = C.c_uint64()
+        self._check(self.L.rfx_sorted_size(self._ctx, C.byref(n)), self._ctx)
+        return n.value
+
     def shard_stats(self) -> dict:
         s = _lib.RfxShardStats()
         self._check(self.L.rfx_shard_stats(self._ctx, C.byref(s)), self._ctx)
