@@ -284,6 +284,10 @@ int rfx_shard_connect(rfx_ctx* ctx, const void* handles /* world * RFX_SHARD_HAN
 /* optional: the total number of minimiser bins (a multiple of world, same on every rank; rfx_choose_bins).  Known up
  * front it lets rfx_push_fastq scan each uploaded chunk straight into the slabs; otherwise the ranks agree on it. */
 int rfx_shard_set_bins(rfx_ctx* ctx, uint32_t n_bins_total);
+/* Collective counting from the pushed reads.  A rank whose reads put most records into a few bins (poly-A / poly-G,
+ * microsatellites) scans them a second time with an overflow list of the size the first scan counted.  If its arena cannot
+ * hold that list, EVERY rank returns RFX_E_CAPACITY at once (raise arena_bytes in rfx_shard_init); any other failure of one
+ * rank's partition or count is likewise returned by every rank, with that rank's code.  The contexts stay usable. */
 int rfx_count_sharded(rfx_ctx* ctx);
 /* Collective re-shard of a loaded table: every rank holds a slice loaded with rfx_load_counts / rfx_load_counts_device
  * (slices may be empty and uneven); on return every rank holds exactly the rows whose minimiser bin it owns, as after

@@ -672,7 +672,9 @@ __global__ void __launch_bounds__(NT) sort_bins_kernel(CountArgs A) {
                 bool fits = true;
                 for (uint32_t q = 0; q < P; q++) fits = fits && s_hist[q] <= (uint32_t)CAPS;
                 if (fits) break;
-                if (P >= (uint32_t)MAXP) { if (tid == 0) atomicExch(&A.dstat[DS_OVERFLOW], 2ull); break; }  // (one k-mer more than CAPS times in a class of 1/64: not with real data)
+                // one k-mer more than CAPS times in a bin (poly-A / poly-G reads, microsatellites): no split helps, the host
+                // counts the run again with the hash kernel, which collapses identical records before it touches a k-mer
+                if (P >= (uint32_t)MAXP) { if (tid == 0) atomicExch(&A.dstat[DS_OVERFLOW], 2ull); break; }
                 P <<= 1;
             }
             if (tid == 0) atomicAdd(&A.dstat[DS_SPLITS], 1ull);
@@ -887,6 +889,7 @@ int stage_count_segments(Ctx* c, const ExtSrcs& S, int n_seg, uint32_t n_bins, b
     A.out_cap = cap;
     A.n_tickets = n_bins; A.bin_stride = 1; A.dry = 0;
     const bool any = check_instances ? c->n_records != 0 : n_bins != 0;
+    bool sorted_run = false;
     if (any) {
         cudaEventRecord(c->evk[4], st);
         cudaError_t le;
@@ -925,7 +928,8 @@ int stage_count_segments(Ctx* c, const ExtSrcs& S, int n_seg, uint32_t n_bins, b
             c->count_geometry = vs == "small" ? 1 : vs == "large" ? 2 : vs == "hash" ? 3 : 4;
             c->count_geometry_bins = n_bins;
         }
-        if (vs == "sort") le = c->wide ? launch_sort_count<true, 4096, 256>(A, st) : launch_sort_count<false, 8192, 256>(A, st);
+        sorted_run = vs == "sort";
+        if (sorted_run) le = c->wide ? launch_sort_count<true, 4096, 256>(A, st) : launch_sort_count<false, 8192, 256>(A, st);
         else if (c->wide) le = launch_count<true, 2048, 256, 192, 3>(A, st);
         else if (vs == "small") le = launch_count<false, 2048, 1024, 384, 3>(A, st);
         else if (vs == "large") le = launch_count<false, 4096, 1024, 384, 2>(A, st);
@@ -938,6 +942,20 @@ int stage_count_segments(Ctx* c, const ExtSrcs& S, int n_seg, uint32_t n_bins, b
     RFX_CUDA(c, cudaMemcpyAsync(h, c->dstat.p, sizeof(h), cudaMemcpyDeviceToHost, st));
     cudaError_t e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return ctx_fail(c, RFX_E_CUDA, "count kernel failed: %s", cudaGetErrorString(e));
+    if (sorted_run && h[DS_OVERFLOW] == 2) {
+        // The sort kernel met a k-mer that fills a hash class beyond its array on its own (one poly-A k-mer of a run of a few
+        // thousand reads does).  Count the whole run again with the hash kernel, from zeroed counters and output cursor, and
+        // remember that kernel, not the sort kernel, for this context's next runs.
+        RFX_CUDA(c, cudaMemsetAsync(c->dstat.p, 0, DS_NSLOTS * sizeof(uint64_t), st));
+        const cudaError_t le = c->wide ? launch_count<true, 2048, 256, 192, 3>(A, st) : launch_count<false, 4096, 1024, 384, 2>(A, st);
+        if (le != cudaSuccess) return ctx_fail(c, RFX_E_CUDA, "count kernel launch failed: %s", cudaGetErrorString(le));
+        cudaEventRecord(c->evk[5], st);
+        c->launches++;
+        if (c->count_geometry == 4) c->count_geometry = c->wide ? 3 : 2;
+        RFX_CUDA(c, cudaMemcpyAsync(h, c->dstat.p, sizeof(h), cudaMemcpyDeviceToHost, st));
+        e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) return ctx_fail(c, RFX_E_CUDA, "count kernel failed: %s", cudaGetErrorString(e));
+    }
     c->ms[2] += stage_end(c);
     c->ms_kernel[2] = 0;
     if (any) cudaEventElapsedTime(&c->ms_kernel[2], c->evk[4], c->evk[5]);

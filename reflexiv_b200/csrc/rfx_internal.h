@@ -266,7 +266,7 @@ inline unsigned sm_count() {
 int stage_parse_fastq(Ctx* c, const uint8_t* d_text, size_t len, bool first_chunk = true, bool more_follows = false);
 int stage_push_reads(Ctx* c, const uint8_t* h_bases, const uint64_t* h_offsets, uint64_t n_reads);
 int stage_partition(Ctx* c, int n_shards);
-int stage_partition_slab(Ctx* c);
+int stage_partition_slab(Ctx* c, uint64_t ovf_need = 0);
 int stage_stream_partition_begin(Ctx* c, uint64_t est_instances, uint64_t est_reads);
 int stage_stream_partition_scan(Ctx* c);
 int stage_rebin(Ctx* c);

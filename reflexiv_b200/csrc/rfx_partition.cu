@@ -600,8 +600,9 @@ __global__ void ovf_scatter_kernel(const uint64_t* __restrict__ ovf_rec, const u
 //   slab_begin   bin geometry and slabs from an (estimated) instance / read count
 //   slab_scan    the minimiser scan over reads [off, off + n), records stored as they are cut
 //   slab_finish  totals, overflow segment; leaves c->have_records false when the overflow list did not suffice
-//                (caller falls back to the two-pass path)
-static int slab_begin(Ctx* c, uint64_t est_instances, uint64_t est_reads) {
+//                (caller falls back to the two-pass path, or re-scans with a list of c->n_ovf records)
+// keep_cap / ovf_need (both 0 unless re-scanning): slab capacity of the scan before, and the overflow records it counted
+static int slab_begin(Ctx* c, uint64_t est_instances, uint64_t est_reads, uint32_t keep_cap = 0, uint64_t ovf_need = 0) {
     cudaStream_t st = c->stream;
     c->n_shards = 1;
     // sharded runs over peer memory: every rank scans into slabs over ALL bins of the run (rfx_shard.cu)
@@ -613,7 +614,9 @@ static int slab_begin(Ctx* c, uint64_t est_instances, uint64_t est_reads) {
     const uint64_t est = est_instances * 2 / (uint64_t)(w + 1) + est_reads + 1;
     uint64_t cap = ((c->wide ? 3 : 2) * est / nb + 8 + 3) & ~(uint64_t)3;  // k > 31: few minimiser loci per bin, uneven bins
     if (cap > 0x7fffffffull) cap = 0x7fffffffull;
-    const uint64_t ovf_cap = est / ((c->wide || c->sh_world > 0) ? 3 : 8) + 4096;
+    if (keep_cap) cap = keep_cap;
+    uint64_t ovf_cap = est / ((c->wide || c->sh_world > 0) ? 3 : 8) + 4096;
+    if (ovf_cap < ovf_need) ovf_cap = ovf_need;
     RFX_TRY(devbuf_reserve(c, c->bin_cursor, nb * 4 * sizeof(uint32_t)));
     RFX_TRY(devbuf_reserve(c, c->records, (nb * cap * c->recw + 2) * sizeof(uint64_t)));
     RFX_TRY(devbuf_reserve(c, c->ovf_rec, (ovf_cap * c->recw + 2) * sizeof(uint64_t)));
@@ -670,8 +673,8 @@ static int slab_finish(Ctx* c) {
         RFX_CUDA(c, cudaMemcpyAsync(&n_records, plan.total, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
         RFX_CUDA(c, cudaMemcpyAsync(&n_ovf, c->dstat.as<uint64_t>() + DS_OVF_RECORDS, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
         RFX_CUDA(c, cudaStreamSynchronize(st));
+        c->n_ovf = n_ovf;  // every record that missed its slab, also those the list had no room for
         if (n_ovf > c->sp_ovf_cap) return RFX_OK;  // a few very heavy bins (or a bad size estimate): this input needs the exact layout
-        c->n_ovf = n_ovf;
         if (n_ovf) {
             // exact partition of the overflow list -> segment 1 of the counting kernel
             RFX_TRY(devbuf_reserve(c, c->bin_off, (nb + 1) * sizeof(uint64_t)));
@@ -711,12 +714,15 @@ int stage_stream_partition_scan(Ctx* c) {
 }
 
 // One GPU, records stay local.  Uses what the streamed scans already did when they cover every read.
-int stage_partition_slab(Ctx* c) {
+// ovf_need > 0 (sharded runs, whose bins are fixed): the scan before left c->have_records false; scan every read again with the same bins and slab capacity and
+// an overflow list of ovf_need records.  How many records a bin overflows by, max(0, records of the bin - capacity), does
+// not depend on the order the records arrive in, so a list of the count the scan before made (c->n_ovf) always suffices.
+int stage_partition_slab(Ctx* c, uint64_t ovf_need) {
     stage_begin(c);
     int rc = RFX_OK;
     const bool bins_fit = !(c->sh_world > 0 && c->sh_bins_run) || c->n_bins == c->sh_bins_run;
-    if (!(c->sp_active && c->sp_done == c->n_reads && c->n_reads && bins_fit)) {
-        rc = slab_begin(c, c->n_instances, c->n_reads);
+    if (ovf_need || !(c->sp_active && c->sp_done == c->n_reads && c->n_reads && bins_fit)) {
+        rc = slab_begin(c, c->n_instances, c->n_reads, ovf_need ? c->sp_cap : 0u, ovf_need);
         if (rc == RFX_OK) rc = slab_scan(c, 0, c->n_reads);
     }
     c->sp_active = false;

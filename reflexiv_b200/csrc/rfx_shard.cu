@@ -181,8 +181,10 @@ void shard_release(Ctx* c) {
 int stage_count_sharded(Ctx* c) {
     if (c->sh_world < 1 || !c->peer_base[c->sh_rank]) return ctx_fail(c, RFX_E_STATE, "rfx_count_sharded: call rfx_shard_init / rfx_shard_connect first");
     const int world = c->sh_world, me = c->sh_rank;
-    unsigned long long mine[8], all[RFX_MAX_RANKS * RFX_PUB_SLOTS];
+    unsigned long long mine[9], all[RFX_MAX_RANKS * RFX_PUB_SLOTS];
     c->ms_comm = 0;
+    // Between two exchanges no rank returns without publishing why: a rank that fails alone would leave its peers waiting in
+    // the next barrier until it times out.  Every rank checks every rank's status word and returns the same code.
     // 1. the bin count every rank uses: given by the caller, or agreed on from the global number of k-mer instances
     uint32_t B = c->sh_bins;
     if (!B) {
@@ -197,12 +199,22 @@ int stage_count_sharded(Ctx* c) {
     // 2. own reads -> slabs over all B bins (the streamed scan of rfx_push_fastq already did it when it ran with B bins)
     c->sh_bins_run = B;
     c->shard_id = -1; c->n_seg = 0;
-    const int prc = stage_partition_slab(c);
+    int prc = stage_partition_slab(c);
+    if (prc == RFX_OK && !c->have_records) {
+        // A few minimiser bins hold most of this rank's records (low-complexity reads: poly-A / poly-G, microsatellites) and the
+        // overflow list was too small.  Unlike one GPU there is no compact layout to fall back to, but the scan counted every
+        // record that missed its slab: one more scan with a list of exactly that many records always fits.
+        const unsigned long long need = c->n_ovf;
+        prc = stage_partition_slab(c, need);
+        if (prc == RFX_E_NOMEM) {
+            const std::string why = c->err;
+            prc = ctx_fail(c, RFX_E_CAPACITY, "sharded counting: the overflow list of this rank's heavy minimiser bins (%llu records) does not fit: %s", need, why.c_str());
+        } else if (prc == RFX_OK && !c->have_records) {
+            prc = ctx_fail(c, RFX_E_STATE, "internal: the re-scan overflowed its list of %llu records (%llu)", need, (unsigned long long)c->n_ovf);
+        }
+    }
     c->sh_bins_run = c->sh_bins;
-    RFX_TRY(prc);
-    if (!c->have_records)
-        return ctx_fail(c, RFX_E_CAPACITY, "sharded counting: the slab overflow list was too small for this input (a few minimiser bins hold most records)");
-    // 3. tell the others where the slabs are
+    // 3. tell the others where the slabs are, or that this rank has none
     auto off_of = [&](const void* p) -> unsigned long long { return p ? (unsigned long long)((const uint8_t*)p - c->arena) : 0ull; };
     mine[0] = off_of(c->records.p);
     mine[1] = off_of(c->bin_cursor.p);
@@ -212,7 +224,13 @@ int stage_count_sharded(Ctx* c) {
     mine[5] = c->n_ovf;
     mine[6] = B;
     mine[7] = c->n_instances;
-    RFX_TRY(shard_exchange(c, PUB_SLAB_REC, 8, mine, all));
+    mine[8] = (unsigned long long)-prc;  // status word: 0, or the rfx_status (negated) this rank returns
+    RFX_TRY(shard_exchange(c, PUB_SLAB_REC, 9, mine, all));
+    if (prc != RFX_OK) return prc;
+    for (int r = 0; r < world; r++) {
+        const unsigned long long st = all[(size_t)r * RFX_PUB_SLOTS + PUB_SLAB_REC + 8];
+        if (st) return ctx_fail(c, -(int)st, "sharded counting: rank %d could not partition its reads (error %d there)", r, -(int)st);
+    }
     // 4. count the own bins out of everybody's slabs (and overflow lists)
     ExtSrcs S;
     memset(&S, 0, sizeof(S));
@@ -235,12 +253,18 @@ int stage_count_sharded(Ctx* c) {
         }
     }
     c->sh_inst_global = inst_global;
-    RFX_TRY(stage_count_segments(c, S, n_seg, bps, false));
+    const int crc = stage_count_segments(c, S, n_seg, bps, false);
     // 5. nobody may touch its slabs again before every rank has counted; the same exchange tells everybody the global row count
-    mine[0] = c->n_rows;
-    RFX_TRY(shard_exchange(c, PUB_INSTANCES, 1, mine, all));
+    mine[0] = crc == RFX_OK ? c->n_rows : 0;
+    mine[1] = (unsigned long long)-crc;
+    RFX_TRY(shard_exchange(c, PUB_INSTANCES, 2, mine, all));
+    if (crc != RFX_OK) return crc;
     c->sh_rows_global = 0;
-    for (int r = 0; r < world; r++) c->sh_rows_global += all[(size_t)r * RFX_PUB_SLOTS + PUB_INSTANCES];
+    for (int r = 0; r < world; r++) {
+        const unsigned long long st = all[(size_t)r * RFX_PUB_SLOTS + PUB_INSTANCES + 1];
+        if (st) return ctx_fail(c, -(int)st, "sharded counting: rank %d could not count its bins (error %d there)", r, -(int)st);
+        c->sh_rows_global += all[(size_t)r * RFX_PUB_SLOTS + PUB_INSTANCES];
+    }
     c->n_bins = B;
     return RFX_OK;
 }

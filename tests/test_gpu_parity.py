@@ -343,7 +343,9 @@ def test_repeated_runs_are_bit_identical(R, orc, monkeypatch):
 
 @pytest.mark.parametrize("k", [31, 61])
 def test_long_and_ragged_reads(R, orc, k):
-    """Reads far longer than the descriptor slots of the binning pass (spill path), mixed with short and empty ones."""
+    """Reads of up to 11 000 bases (warps of very uneven reads in the register-resident scan), mixed with short and empty
+    ones, on the default single-pass partition.  The same reads on the two-pass partition, whose spill pass they reach:
+    test_skewed_inputs.test_spill_pass_of_the_two_pass_partition."""
     rng = np.random.default_rng(9)
     g = "".join("ACGT"[i] for i in rng.integers(0, 4, 20_000))
     seqs = [g[a:a + n] for a, n in ((0, 5000), (3000, 4000), (100, k), (200, k + 1), (300, k + 2), (400, 150), (9000, 11000), (0, 0), (5, 3))]
