@@ -246,8 +246,11 @@ int rfx_load_counts_device(rfx_ctx* ctx, const void* d_keys, const uint32_t* d_c
  * then read and write peer HBM directly: no collective library on the data path.
  *   every rank:  rfx_shard_init -> rfx_shard_export -> [caller gathers the world * RFX_SHARD_HANDLE_BYTES bytes] ->
  *                rfx_shard_connect -> { rfx_reset, rfx_push_fastq*, rfx_count_sharded, rfx_assemble_sharded, results }*
- * rfx_count_sharded / rfx_assemble_sharded are collective: every rank must call them (from its own host thread or
- * process); they meet in cross-GPU barriers and fail with RFX_E_STATE if a peer never arrives.  Ranks that share a device
+ * rfx_count_sharded, rfx_shard_table, rfx_assemble_sharded and rfx_sort_kmers_sharded are collective: every rank must call
+ * them (from its own host thread or process); they meet in cross-GPU barriers and fail with RFX_E_STATE if a peer never
+ * arrives.  A collective call either succeeds on every rank or fails on every rank at once, with the code of the
+ * lowest-numbered rank that failed (that rank keeps its own message, the others name it), and the contexts stay usable for
+ * the next collective call.  Ranks that share a device
  * inside one process meet on the host instead and need CUDA_MODULE_LOADING=EAGER in the environment (no kernel may be
  * loaded lazily while a peer on the same device waits).  rfx_assemble_sharded needs a table sharded by minimiser bin: the
  * one rfx_count_sharded leaves, or a loaded one after rfx_shard_table:
@@ -285,27 +288,32 @@ int rfx_shard_connect(rfx_ctx* ctx, const void* handles /* world * RFX_SHARD_HAN
  * front it lets rfx_push_fastq scan each uploaded chunk straight into the slabs; otherwise the ranks agree on it. */
 int rfx_shard_set_bins(rfx_ctx* ctx, uint32_t n_bins_total);
 /* Collective counting from the pushed reads.  A rank whose reads put most records into a few bins (poly-A / poly-G,
- * microsatellites) scans them a second time with an overflow list of the size the first scan counted.  If its arena cannot
- * hold that list, EVERY rank returns RFX_E_CAPACITY at once (raise arena_bytes in rfx_shard_init); any other failure of one
- * rank's partition or count is likewise returned by every rank, with that rank's code.  The contexts stay usable. */
+ * microsatellites) scans them a second time with an overflow list of the size the first scan counted: RFX_E_CAPACITY if its
+ * arena cannot hold that list (raise arena_bytes in rfx_shard_init). */
 int rfx_count_sharded(rfx_ctx* ctx);
 /* Collective re-shard of a loaded table: every rank holds a slice loaded with rfx_load_counts / rfx_load_counts_device
  * (slices may be empty and uneven); on return every rank holds exactly the rows whose minimiser bin it owns, as after
  * rfx_count_sharded.  Rows are neither merged nor de-duplicated, their order inside a shard is unspecified.  The bin
  * count B is the one of rfx_shard_set_bins if the caller set one (the same on every rank), else
  * rfx_choose_bins(ctx, 64 * global rows, world) -- what counting from reads picks at typical coverage, ~100 rows a bin.
- * A rank without a table, a different k or a B that is no multiple of world makes EVERY rank fail with the same error
- * (RFX_E_STATE / RFX_E_INVALID) after the first exchange.  rfx_stats: ms_partition is the call's time. */
+ * A rank without a table: RFX_E_STATE; k or the caller's B differing between ranks, or a B that is no multiple of world:
+ * RFX_E_INVALID.  rfx_stats: ms_partition is the call's time. */
 int rfx_shard_table(rfx_ctx* ctx);
+/* Collective assembly (fork filters, chains, contigs: rfx_assemble across ranks) of a table sharded by minimiser bin, after
+ * rfx_count_sharded or rfx_shard_table.  A rank without a table, or with one not sharded by minimiser bin: RFX_E_STATE;
+ * -bubble: RFX_E_UNSUPPORTED; k < 2: RFX_E_INVALID; more than 2^28 rows on a rank: RFX_E_CAPACITY; an arena too small for
+ * the call's buffers: RFX_E_NOMEM (raise arena_bytes in rfx_shard_init); a (k-1)-mer of degree > 1 after the fork filters, a
+ * row on a rank that does not own its minimiser bin or a request channel that overflowed: RFX_E_GRAPH.  A closed path makes
+ * rank 0 assemble the whole table (fell_back in rfx_shard_stats), which may fail with the codes of rfx_assemble. */
 int rfx_assemble_sharded(rfx_ctx* ctx);
 /* Collective Count_<k>_sorted on a table sharded by minimiser bin (after rfx_count_sharded or rfx_shard_table): the same
  * arguments, domain and results as rfx_sort_kmers.  On return every rank holds the sorted rows of its own shard
  * (rfx_sorted_size / rfx_sorted_copy / rfx_sorted_csv); their union over the ranks equals, bit for bit, what rfx_sort_kmers
  * gives on one context holding the whole table.  Like rfx_sort_kmers it takes the index and the flag arrays over: the
  * contigs of an earlier rfx_assemble_sharded are gone (RFX_E_STATE), a later rfx_assemble_sharded rebuilds them.  The ranks
- * agree on their arguments before any barrier, so a misuse makes EVERY rank fail with the same error at once: arguments
- * that differ between ranks RFX_E_INVALID, a rank without a sharded table RFX_E_STATE, min_error_coverage == 0 or
- * (k-1) % 31 == 0 RFX_E_UNSUPPORTED, more than 2^28 rows on a rank RFX_E_CAPACITY.  rfx_stats: ms_graph is the call's time;
+ * agree on their arguments before any barrier: arguments that differ between ranks RFX_E_INVALID, a rank without a sharded
+ * table RFX_E_STATE, min_error_coverage == 0 or (k-1) % 31 == 0 RFX_E_UNSUPPORTED, more than 2^28 rows on a rank
+ * RFX_E_CAPACITY.  rfx_stats: ms_graph is the call's time;
  * rfx_shard_stats: ms_comm and n_remote_probes cover the call. */
 int rfx_sort_kmers_sharded(rfx_ctx* ctx, int32_t min_error_coverage, double min_repeat_fold, int32_t max_kmer_size);
 int rfx_shard_stats(rfx_ctx* ctx, rfx_shard_stats_t* out);

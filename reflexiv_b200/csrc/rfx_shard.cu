@@ -100,11 +100,11 @@ static bool host_barrier_wait(HostBarrier* hb) {
     return true;
 }
 
-// everybody's published slots [first, first + n) -> one local block, so that the host needs ONE device-to-host copy
-__global__ void gather_pub_kernel(PeerBases P, int par, int first, int n, unsigned long long* __restrict__ out) {
+// everybody's published slots [0, n) -> one local block, so that the host needs ONE device-to-host copy
+__global__ void gather_pub_kernel(PeerBases P, int par, int n, unsigned long long* __restrict__ out) {
     for (int i = threadIdx.x; i < P.n * n; i += blockDim.x) {
         const int r = i / n, s = i % n;
-        out[(size_t)r * RFX_PUB_SLOTS + first + s] = *reinterpret_cast<const volatile unsigned long long*>(&reinterpret_cast<const ShardCtl*>(P.base[r])->pub[par][first + s]);
+        out[(size_t)r * RFX_PUB_SLOTS + s] = *reinterpret_cast<const volatile unsigned long long*>(&reinterpret_cast<const ShardCtl*>(P.base[r])->pub[par][s]);
     }
 }
 
@@ -139,19 +139,21 @@ int shard_check(Ctx* c, const char* what) {
     return RFX_OK;
 }
 
-// Publish `n` values (slots [first, first + n) of the own control block), barrier, read everybody's slots back:
-// vals[r * RFX_PUB_SLOTS + slot].  One host synchronisation.
-int shard_exchange(Ctx* c, int first, int n, const unsigned long long* mine, unsigned long long* all, int n_dev, const int* dev_slots, int dev_first) {
+// Slot 0 of the published block: the status (-rc), then the n host values, then the n_dev device counters.  Every exchange
+// starts at slot 0 of the half its parity picks, and a caller reads back only what that exchange wrote.  One host
+// synchronisation.
+int shard_exchange(Ctx* c, int rc, int n, const unsigned long long* mine, PubVals& all, int n_dev, const int* dev_slots) {
     cudaEventRecord(c->ev_comm[0], c->stream);
     unsigned long long* h = c->h_pub;  // [0, SLOTS): staging of the own values, [SLOTS, ...): everybody's
-    for (int i = 0; i < n; i++) h[first + i] = mine[i];
+    h[0] = (unsigned long long)-rc;
+    for (int i = 0; i < n; i++) h[1 + i] = mine[i];
     ShardCtl* own = reinterpret_cast<ShardCtl*>(c->arena);
     const int par = (int)(c->sh_exchanges++ & 1u);
-    RFX_CUDA(c, cudaMemcpyAsync(&own->pub[par][first], h + first, (size_t)n * sizeof(unsigned long long), cudaMemcpyHostToDevice, c->stream));
+    RFX_CUDA(c, cudaMemcpyAsync(&own->pub[par][0], h, (size_t)(1 + n) * sizeof(unsigned long long), cudaMemcpyHostToDevice, c->stream));
     for (int i = 0; i < n_dev; i++)
-        RFX_CUDA(c, cudaMemcpyAsync(&own->pub[par][dev_first + i], c->dstat.as<unsigned long long>() + dev_slots[i], sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
+        RFX_CUDA(c, cudaMemcpyAsync(&own->pub[par][1 + n + i], c->dstat.as<unsigned long long>() + dev_slots[i], sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
     RFX_TRY(shard_barrier(c));
-    gather_pub_kernel<<<1, 256, 0, c->stream>>>(peer_bases(c), par, first, n, c->d_pub);
+    gather_pub_kernel<<<1, 256, 0, c->stream>>>(peer_bases(c), par, 1 + n + n_dev, c->d_pub);
     c->launches++;
     RFX_CUDA(c, cudaMemcpyAsync(h + RFX_PUB_SLOTS, c->d_pub, (size_t)c->sh_world * RFX_PUB_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
     cudaEventRecord(c->ev_comm[1], c->stream);
@@ -159,8 +161,15 @@ int shard_exchange(Ctx* c, int first, int n, const unsigned long long* mine, uns
     float ms = 0;
     cudaEventElapsedTime(&ms, c->ev_comm[0], c->ev_comm[1]);
     c->ms_comm += ms;
-    for (int r = 0; r < c->sh_world; r++)
-        for (int i = 0; i < n; i++) all[(size_t)r * RFX_PUB_SLOTS + first + i] = h[(size_t)(r + 1) * RFX_PUB_SLOTS + first + i];
+    all.world = c->sh_world;
+    for (int r = 0; r < c->sh_world; r++) {
+        const unsigned long long* v = h + (size_t)(r + 1) * RFX_PUB_SLOTS;
+        if (v[0]) {  // the lowest failing rank keeps its own message
+            const int code = -(int)v[0];
+            return r == c->sh_rank ? rc : ctx_fail(c, code, "rank %d failed with error %d in this collective call", r, code);
+        }
+        for (int i = 0; i < n + n_dev; i++) all.v[r][i] = v[1 + i];
+    }
     return RFX_OK;
 }
 
@@ -181,25 +190,23 @@ void shard_release(Ctx* c) {
 int stage_count_sharded(Ctx* c) {
     if (c->sh_world < 1 || !c->peer_base[c->sh_rank]) return ctx_fail(c, RFX_E_STATE, "rfx_count_sharded: call rfx_shard_init / rfx_shard_connect first");
     const int world = c->sh_world, me = c->sh_rank;
-    unsigned long long mine[9], all[RFX_MAX_RANKS * RFX_PUB_SLOTS];
+    unsigned long long mine[8];
+    static_assert(sizeof(mine) / sizeof(mine[0]) <= PUB_VALS, "the slab exchange fits the published block");
+    PubVals all;
     c->ms_comm = 0;
-    // Between two exchanges no rank returns without publishing why: a rank that fails alone would leave its peers waiting in
-    // the next barrier until it times out.  Every rank checks every rank's status word and returns the same code.
     // 1. the bin count every rank uses: given by the caller, or agreed on from the global number of k-mer instances
     uint32_t B = c->sh_bins;
     if (!B) {
         mine[0] = c->n_instances;
-        RFX_TRY(shard_exchange(c, PUB_INSTANCES, 1, mine, all));
-        uint64_t tot = 0;
-        for (int r = 0; r < world; r++) tot += all[(size_t)r * RFX_PUB_SLOTS + PUB_INSTANCES];
-        B = choose_bin_count(c, tot, world);
+        RFX_TRY(shard_exchange(c, RFX_OK, 1, mine, all));
+        B = choose_bin_count(c, all.sum(0), world);
     }
-    if (B % (uint32_t)world) return ctx_fail(c, RFX_E_INVALID, "sharded counting: %u bins are not a multiple of %d ranks", B, world);
+    int prc = B % (uint32_t)world ? ctx_fail(c, RFX_E_INVALID, "sharded counting: %u bins are not a multiple of %d ranks", B, world) : RFX_OK;
     const uint32_t bps = B / (uint32_t)world;
     // 2. own reads -> slabs over all B bins (the streamed scan of rfx_push_fastq already did it when it ran with B bins)
     c->sh_bins_run = B;
     c->shard_id = -1; c->n_seg = 0;
-    int prc = stage_partition_slab(c);
+    if (prc == RFX_OK) prc = stage_partition_slab(c);
     if (prc == RFX_OK && !c->have_records) {
         // A few minimiser bins hold most of this rank's records (low-complexity reads: poly-A / poly-G, microsatellites) and the
         // overflow list was too small.  Unlike one GPU there is no compact layout to fall back to, but the scan counted every
@@ -224,47 +231,31 @@ int stage_count_sharded(Ctx* c) {
     mine[5] = c->n_ovf;
     mine[6] = B;
     mine[7] = c->n_instances;
-    mine[8] = (unsigned long long)-prc;  // status word: 0, or the rfx_status (negated) this rank returns
-    RFX_TRY(shard_exchange(c, PUB_SLAB_REC, 9, mine, all));
-    if (prc != RFX_OK) return prc;
-    for (int r = 0; r < world; r++) {
-        const unsigned long long st = all[(size_t)r * RFX_PUB_SLOTS + PUB_SLAB_REC + 8];
-        if (st) return ctx_fail(c, -(int)st, "sharded counting: rank %d could not partition its reads (error %d there)", r, -(int)st);
-    }
+    RFX_TRY(shard_exchange(c, prc, 8, mine, all));
     // 4. count the own bins out of everybody's slabs (and overflow lists)
     ExtSrcs S;
     memset(&S, 0, sizeof(S));
     int n_seg = 0;
-    uint64_t inst_global = 0;
     for (int r = 0; r < world; r++) {
-        const unsigned long long* v = all + (size_t)r * RFX_PUB_SLOTS + PUB_SLAB_REC;
-        if (v[6] != B) return ctx_fail(c, RFX_E_STATE, "sharded counting: rank %d uses %llu bins, this rank %u", r, v[6], B);
-        inst_global += v[7];
+        if (all.at(r, 6) != B) return ctx_fail(c, RFX_E_STATE, "sharded counting: rank %d uses %llu bins, this rank %u", r, all.at(r, 6), B);
         ExtSrc& a = S.s[n_seg++];
-        a.rec = reinterpret_cast<const uint64_t*>(c->peer_base[r] + v[0]);
-        a.slab_cnt = reinterpret_cast<const uint32_t*>(c->peer_base[r] + v[1]);
-        a.slab_cap = (uint32_t)v[2];
+        a.rec = reinterpret_cast<const uint64_t*>(c->peer_base[r] + all.at(r, 0));
+        a.slab_cnt = reinterpret_cast<const uint32_t*>(c->peer_base[r] + all.at(r, 1));
+        a.slab_cap = (uint32_t)all.at(r, 2);
         a.bin_base = (uint32_t)me * bps;
-        if (v[5]) {
+        if (all.at(r, 5)) {
             ExtSrc& o = S.s[n_seg++];
-            o.rec = reinterpret_cast<const uint64_t*>(c->peer_base[r] + v[3]);
-            o.off = reinterpret_cast<const uint64_t*>(c->peer_base[r] + v[4]);
+            o.rec = reinterpret_cast<const uint64_t*>(c->peer_base[r] + all.at(r, 3));
+            o.off = reinterpret_cast<const uint64_t*>(c->peer_base[r] + all.at(r, 4));
             o.bin_base = (uint32_t)me * bps;
         }
     }
-    c->sh_inst_global = inst_global;
+    c->sh_inst_global = all.sum(7);
     const int crc = stage_count_segments(c, S, n_seg, bps, false);
     // 5. nobody may touch its slabs again before every rank has counted; the same exchange tells everybody the global row count
-    mine[0] = crc == RFX_OK ? c->n_rows : 0;
-    mine[1] = (unsigned long long)-crc;
-    RFX_TRY(shard_exchange(c, PUB_INSTANCES, 2, mine, all));
-    if (crc != RFX_OK) return crc;
-    c->sh_rows_global = 0;
-    for (int r = 0; r < world; r++) {
-        const unsigned long long st = all[(size_t)r * RFX_PUB_SLOTS + PUB_INSTANCES + 1];
-        if (st) return ctx_fail(c, -(int)st, "sharded counting: rank %d could not count its bins (error %d there)", r, -(int)st);
-        c->sh_rows_global += all[(size_t)r * RFX_PUB_SLOTS + PUB_INSTANCES];
-    }
+    mine[0] = c->n_rows;
+    RFX_TRY(shard_exchange(c, crc, 1, mine, all));
+    c->sh_rows_global = all.sum(0);
     c->n_bins = B;
     return RFX_OK;
 }
@@ -387,47 +378,43 @@ template <class KT> static int table_pull(Ctx* c, const TablePull& P) {
 int stage_shard_table(Ctx* c) {
     if (c->sh_world < 1 || !c->peer_base[c->sh_rank]) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: call rfx_shard_init / rfx_shard_connect first");
     const int world = c->sh_world, me = c->sh_rank;
-    unsigned long long mine[3 + RFX_MAX_RANKS], all[RFX_MAX_RANKS * RFX_PUB_SLOTS] = {};
-    auto got = [&](int r, int slot) { return all[(size_t)r * RFX_PUB_SLOTS + PUB_TABLE + slot]; };
+    unsigned long long mine[2 + RFX_MAX_RANKS];
+    static_assert(sizeof(mine) / sizeof(mine[0]) <= PUB_VALS, "the routing exchange fits the published block");
+    PubVals all;
     c->st_active = false;
     c->ms_comm = 0;
     stage_begin(c);
     // 1. what every rank holds.  Every rank checks every rank's values in the same order, so that all ranks return the same
-    //    error together instead of leaving their peers in a barrier
-    mine[0] = c->have_counts ? 1 : 0;
-    mine[1] = c->have_counts ? c->n_rows : 0;
-    mine[2] = (unsigned long long)c->k;
-    mine[3] = c->sh_bins;
-    RFX_TRY(shard_exchange(c, PUB_TABLE, 4, mine, all));
+    //    error together
+    const int rc_have = c->have_counts ? RFX_OK : ctx_fail(c, RFX_E_STATE, "rfx_shard_table: no count table on this rank (every rank loads a slice first, an empty one will do)");
+    mine[0] = c->have_counts ? c->n_rows : 0;
+    mine[1] = (unsigned long long)c->k;
+    mine[2] = c->sh_bins;
+    RFX_TRY(shard_exchange(c, rc_have, 3, mine, all));
     uint64_t rows_global = 0;
     for (int r = 0; r < world; r++) {
-        if (!got(r, 0)) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: rank %d holds no count table (every rank loads a slice first, an empty one will do)", r);
-        if (got(r, 2) != got(0, 2)) return ctx_fail(c, RFX_E_INVALID, "rfx_shard_table: rank %d has k = %llu, rank 0 k = %llu", r, got(r, 2), got(0, 2));
-        if (got(r, 3) != got(0, 3)) return ctx_fail(c, RFX_E_INVALID, "rfx_shard_table: rank %d set %llu bins, rank 0 %llu", r, got(r, 3), got(0, 3));
-        rows_global += got(r, 1);
+        if (all.at(r, 1) != all.at(0, 1)) return ctx_fail(c, RFX_E_INVALID, "rfx_shard_table: rank %d has k = %llu, rank 0 k = %llu", r, all.at(r, 1), all.at(0, 1));
+        if (all.at(r, 2) != all.at(0, 2)) return ctx_fail(c, RFX_E_INVALID, "rfx_shard_table: rank %d set %llu bins, rank 0 %llu", r, all.at(r, 2), all.at(0, 2));
+        rows_global += all.at(r, 0);
     }
     // the bin count: the caller's, or the one counting from reads picks for this many rows at typical coverage (~100 rows a bin)
-    uint32_t B = (uint32_t)got(0, 3);
+    uint32_t B = (uint32_t)all.at(0, 2);
     if (!B) B = choose_bin_count(c, 64 * rows_global, world);
     if (B % (uint32_t)world) return ctx_fail(c, RFX_E_INVALID, "rfx_shard_table: %u bins are not a multiple of %d ranks", B, world);
     const uint32_t bps = B / (uint32_t)world;
     set_minimizer(c, B);
-    // 2. own rows -> send buffer grouped by owner.  A rank that fails here still takes part in the next exchange
+    // 2. own rows -> send buffer grouped by owner
     unsigned long long hist[RFX_MAX_RANKS] = {0};
     const int rc_send = c->wide ? table_route_scatter<u128>(c, B, bps, hist) : table_route_scatter<uint64_t>(c, B, bps, hist);
     const size_t ksz = c->wide ? sizeof(u128) : sizeof(uint64_t);
     const unsigned long long send_at = c->sh_send.p ? (unsigned long long)(c->sh_send.as<uint8_t>() - c->arena) : 0ull;
-    mine[0] = rc_send == RFX_OK ? 0 : 1;
-    mine[1] = send_at + send_keys_off();
-    mine[2] = send_at + send_counts_off(c->n_rows, ksz);
-    for (int o = 0; o < world; o++) mine[3 + o] = hist[o];
-    RFX_TRY(shard_exchange(c, PUB_TABLE, 3 + world, mine, all));
-    if (rc_send != RFX_OK) return rc_send;
+    mine[0] = send_at + send_keys_off();
+    mine[1] = send_at + send_counts_off(c->n_rows, ksz);
+    for (int o = 0; o < world; o++) mine[2 + o] = hist[o];
+    RFX_TRY(shard_exchange(c, rc_send, 2 + world, mine, all));
     uint64_t sent = 0;
-    for (int r = 0; r < world; r++) {
-        if (got(r, 0)) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: rank %d could not route its rows", r);
-        for (int o = 0; o < world; o++) sent += got(r, 3 + o);
-    }
+    for (int r = 0; r < world; r++)
+        for (int o = 0; o < world; o++) sent += all.at(r, 2 + o);
     if (sent != rows_global) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: %llu rows routed, %llu loaded", (unsigned long long)sent, (unsigned long long)rows_global);
     // 3. pull the own rows out of every rank's send buffer
     TablePull P;
@@ -435,23 +422,17 @@ int stage_shard_table(Ctx* c) {
     P.n = world;
     for (int q = 0; q < world; q++) {
         uint64_t before = 0;  // rows of sender q that go to lower ranks
-        for (int o = 0; o < me; o++) before += got(q, 3 + o);
-        P.keys[q] = c->peer_base[q] + got(q, 1) + before * ksz;
-        P.counts[q] = reinterpret_cast<const uint32_t*>(c->peer_base[q] + got(q, 2)) + before;
-        P.start[q + 1] = P.start[q] + got(q, 3 + me);
+        for (int o = 0; o < me; o++) before += all.at(q, 2 + o);
+        P.keys[q] = c->peer_base[q] + all.at(q, 0) + before * ksz;
+        P.counts[q] = reinterpret_cast<const uint32_t*>(c->peer_base[q] + all.at(q, 1)) + before;
+        P.start[q + 1] = P.start[q] + all.at(q, 2 + me);
     }
     const uint64_t recv = P.start[world];
     const int rc_recv = c->wide ? table_pull<u128>(c, P) : table_pull<uint64_t>(c, P);
     // 4. nobody may reuse its send buffer before every owner has pulled: one more exchange, which also checks the total
-    mine[0] = rc_recv == RFX_OK ? 0 : 1;
-    mine[1] = recv;
-    RFX_TRY(shard_exchange(c, PUB_TABLE, 2, mine, all));
-    if (rc_recv != RFX_OK) return rc_recv;
-    uint64_t received = 0;
-    for (int r = 0; r < world; r++) {
-        if (got(r, 0)) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: rank %d could not receive its rows", r);
-        received += got(r, 1);
-    }
+    mine[0] = recv;
+    RFX_TRY(shard_exchange(c, rc_recv, 1, mine, all));
+    const uint64_t received = all.sum(0);
     if (received != rows_global) return ctx_fail(c, RFX_E_STATE, "rfx_shard_table: %llu rows received, %llu sent", (unsigned long long)received, (unsigned long long)rows_global);
     c->ms[1] = stage_end(c);
     c->sh_rows_global = rows_global;

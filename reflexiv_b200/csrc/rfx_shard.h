@@ -29,22 +29,29 @@ struct PeerBases {
     int n, me;
 };
 
-// slots of ShardCtl::pub
-enum {
-    PUB_INSTANCES = 0,
-    PUB_SLAB_REC = 1,   // 9 slots: slab records, slab counts, slab cap, overflow records, overflow offsets, n overflow, bins, instances, status
-    PUB_TABLE = 1,      // rfx_shard_table, 3 + RFX_MAX_RANKS slots (never in use together with PUB_SLAB_REC)
-    PUB_GRAPH = 12,     // rfx_shard_graph.cu: GPub
-    PUB_END = RFX_PUB_SLOTS
+// values one exchange can carry: slot 0 of the published block is the caller's status
+constexpr int PUB_VALS = RFX_PUB_SLOTS - 1;
+
+// everybody's values of the last exchange: value i of rank r (the caller's host values, then its device counters)
+struct PubVals {
+    unsigned long long v[RFX_MAX_RANKS][PUB_VALS];
+    int world = 0;
+    unsigned long long at(int r, int i) const { return v[r][i]; }
+    unsigned long long sum(int i) const {
+        unsigned long long s = 0;
+        for (int r = 0; r < world; r++) s += v[r][i];
+        return s;
+    }
 };
 
 PeerBases peer_bases(const Ctx* c);
 int shard_barrier(Ctx* c);                       // enqueue a cross-GPU barrier on the context's stream
 int shard_check(Ctx* c, const char* what);       // synchronise the stream, report a barrier that timed out
-// publish slots [first, first + n) (host values `mine`, then n_dev device counters dstat[dev_slots[i]] copied on the stream into slots dev_first + i),
-// barrier, read everybody's slots back: all[r * RFX_PUB_SLOTS + slot]
-int shard_exchange(Ctx* c, int first, int n, const unsigned long long* mine, unsigned long long* all /* [RFX_MAX_RANKS * RFX_PUB_SLOTS] */, int n_dev = 0,
-                   const int* dev_slots = nullptr, int dev_first = 0);
+// Publish the status `rc` (RFX_OK or the code this rank fails with), n host values `mine` and n_dev device counters
+// dstat[dev_slots[i]] (copied on the stream), barrier, read everybody's values back into `all`.  If any rank published a
+// failure, every rank returns the code of the lowest failing rank: a rank that fails still takes part, and its peers do not
+// wait for it in the next barrier.
+int shard_exchange(Ctx* c, int rc, int n, const unsigned long long* mine, PubVals& all, int n_dev = 0, const int* dev_slots = nullptr);
 void shard_graph_release(Ctx* c);
 void shard_graph_reset(Ctx* c);  // forget the graph stages' arena buffers (rfx_reset)
 void shard_graph_stats(Ctx* c, rfx_shard_stats_t* out);

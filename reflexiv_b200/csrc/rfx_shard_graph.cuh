@@ -85,14 +85,14 @@ struct SGView {
     __device__ __forceinline__ int owner_of_bin(uint32_t bin) const { return bps == 1u ? (int)bin : (int)__umul64hi((uint64_t)bin, inv_bps); }
 };
 
-// slots of the published block (ShardCtl::pub, from PUB_GRAPH on): arena offsets first, then values
+// what sg_publish exchanges: arena offsets first, then values
 enum {
     GP_KEYS, GP_COUNTS, GP_HT, GP_BLOOM, GP_ALIVE, GP_LFLAG, GP_RFLAG, GP_EFFL, GP_EFFR, GP_SUCC, GP_PRED, GP_NXTL1, GP_L1ENT, GP_L1LOC, GP_L2UP0,
     GP_L2UP1, GP_L2NODE, GP_L2FIN, GP_CHAINLEN, GP_TAILRF, GP_CTGIDX, GP_CTGOFF, GP_CTGBASES, GP_INBOX, GP_RESPBOX, GP_REQCNT, GP_NPTR,
     GP_NROWS = GP_NPTR, GP_HTCAP, GP_BLOOMMASK, GP_HOST,  // GP_HOST: 6 host values, then up to 6 device values
     GP_NHOST = 6, GP_DEV = GP_HOST + GP_NHOST, GP_NDEV = 6, GP_END = GP_DEV + GP_NDEV
 };
-static_assert(PUB_GRAPH + GP_END <= RFX_PUB_SLOTS, "published block too small");
+static_assert(GP_END <= PUB_VALS, "published block too small");
 
 struct GShard {
     DevBuf rmin, work, pend_ref, inbox, respbox, req_cnt, nxt_l1, l1_ent, l1_loc, l1_fin, l1_dst, l2_l1, l2_node, l2_up[2], l2_fin, tail_rf, pubsrc, all_keys, all_counts;
@@ -898,10 +898,10 @@ struct SGProf {
     }
 };
 
-// publish the arena offsets of this rank's graph buffers + values; rebuild the view of everybody's buffers
-static int sg_publish(Ctx* c, SGView& V, const unsigned long long host_vals[GP_NHOST], int n_dev, const int* dev_slots, unsigned long long* all) {
+// publish the status `rc`, the arena offsets of this rank's graph buffers + values; rebuild the view of everybody's buffers
+static int sg_publish(Ctx* c, int rc, SGView& V, const unsigned long long host_vals[GP_NHOST], int n_dev, const int* dev_slots, PubVals& all) {
     GShard* gs = c->gshard;
-    unsigned long long mine[GP_END];
+    unsigned long long mine[GP_DEV];
     auto off_of = [&](const void* p) -> unsigned long long { return p ? (unsigned long long)((const uint8_t*)p - c->arena) : ~0ull; };
     const void* ptrs[GP_NPTR] = {c->keys.p, c->counts.p, c->ht.p, c->g_bloom.p, c->alive.p, c->lflag.p, c->rflag.p, c->eff_l.p, c->eff_r.p, c->succ.p, c->pred.p, gs->nxt_l1.p,
                                  gs->l1_ent.p, gs->l1_loc.p, gs->l2_up[0].p, gs->l2_up[1].p, gs->l2_node.p, gs->l2_fin.p, c->chain_len.p, gs->tail_rf.p,
@@ -911,9 +911,8 @@ static int sg_publish(Ctx* c, SGView& V, const unsigned long long host_vals[GP_N
     mine[GP_HTCAP] = c->ht_cap;
     mine[GP_BLOOMMASK] = 0;
     for (int i = 0; i < GP_NHOST; i++) mine[GP_HOST + i] = host_vals ? host_vals[i] : 0ull;
-    // device values: gathered into a staging block right behind the host values by one small copy each
-    for (int i = 0; i < GP_NDEV; i++) mine[GP_DEV + i] = 0ull;
-    RFX_TRY(shard_exchange(c, PUB_GRAPH, GP_END, mine, all, n_dev, dev_slots, PUB_GRAPH + GP_DEV));
+    // device values (at GP_DEV + i): copied right behind the host values by one small copy each
+    RFX_TRY(shard_exchange(c, rc, GP_DEV, mine, all, n_dev, dev_slots));
     V.me = c->sh_rank; V.world = c->sh_world; V.k = c->k; V.m = c->m;
     V.B = c->n_bins; V.bps = c->n_bins / (uint32_t)c->sh_world;
     V.filter = c->g_bloom.as<uint32_t>();
@@ -924,9 +923,8 @@ static int sg_publish(Ctx* c, SGView& V, const unsigned long long host_vals[GP_N
         SGPeer& P = V.p[r];
         memset(&P, 0, sizeof(P));
         if (r >= c->sh_world) continue;
-        const unsigned long long* v = all + (size_t)r * RFX_PUB_SLOTS + PUB_GRAPH;
         uint8_t* base = c->peer_base[r];
-        auto at = [&](int slot) -> uint8_t* { return v[slot] == ~0ull ? nullptr : base + v[slot]; };
+        auto at = [&](int slot) -> uint8_t* { return all.at(r, slot) == ~0ull ? nullptr : base + all.at(r, slot); };
         P.keys = at(GP_KEYS); P.counts = (const uint32_t*)at(GP_COUNTS); P.ht = (const uint32_t*)at(GP_HT); P.filter = (const uint32_t*)at(GP_BLOOM);
         P.alive = at(GP_ALIVE); P.lflag = (int32_t*)at(GP_LFLAG); P.rflag = (int32_t*)at(GP_RFLAG); P.eff_l = (int32_t*)at(GP_EFFL); P.eff_r = (int32_t*)at(GP_EFFR);
         P.succ = (uint32_t*)at(GP_SUCC); P.pred = (uint32_t*)at(GP_PRED); P.nxt_l1 = (uint32_t*)at(GP_NXTL1);
@@ -935,30 +933,24 @@ static int sg_publish(Ctx* c, SGView& V, const unsigned long long host_vals[GP_N
         P.chain_len = (uint32_t*)at(GP_CHAINLEN); P.tail_rf = (int32_t*)at(GP_TAILRF); P.ctg_idx = (uint32_t*)at(GP_CTGIDX); P.ctg_off = (uint64_t*)at(GP_CTGOFF);
         P.ctg_bases = (char*)at(GP_CTGBASES);
         P.inbox = at(GP_INBOX); P.respbox = (uint4*)at(GP_RESPBOX); P.req_cnt = (unsigned long long*)at(GP_REQCNT);
-        P.ht_cap = (uint32_t)v[GP_HTCAP];
+        P.ht_cap = (uint32_t)all.at(r, GP_HTCAP);
     }
     return RFX_OK;
 }
-static inline unsigned long long sg_sum(const unsigned long long* all, int world, int slot) {
-    unsigned long long s = 0;
-    for (int r = 0; r < world; r++) s += all[(size_t)r * RFX_PUB_SLOTS + PUB_GRAPH + slot];
-    return s;
-}
 
 // a closed path somewhere: rank 0 pulls every shard table and runs the single-GPU stages over the whole table
-template <class KT> static int sg_fallback_whole_table(Ctx* c, const SGView& V, const unsigned long long* all) {
+template <class KT> static int sg_fallback_whole_table(Ctx* c, const SGView& V, const PubVals& all) {
     GShard* gs = c->gshard;
     cudaStream_t st = c->stream;
     gs->fell_back = 1;
     int rc = RFX_OK;
     if (c->sh_rank == 0) {
-        uint64_t tot = 0;
-        for (int r = 0; r < c->sh_world; r++) tot += all[(size_t)r * RFX_PUB_SLOTS + PUB_GRAPH + GP_NROWS];
+        const uint64_t tot = all.sum(GP_NROWS);
         RFX_TRY(devbuf_reserve(c, gs->all_keys, (tot + 1) * sizeof(KT)));
         RFX_TRY(devbuf_reserve(c, gs->all_counts, (tot + 1) * sizeof(uint32_t)));
         uint64_t pos = 0;
         for (int r = 0; r < c->sh_world; r++) {
-            const uint64_t nr = all[(size_t)r * RFX_PUB_SLOTS + PUB_GRAPH + GP_NROWS];
+            const uint64_t nr = all.at(r, GP_NROWS);
             if (nr) {
                 RFX_CUDA(c, cudaMemcpyAsync(gs->all_keys.as<KT>() + pos, V.p[r].keys, nr * sizeof(KT), cudaMemcpyDefault, st));
                 RFX_CUDA(c, cudaMemcpyAsync(gs->all_counts.as<uint32_t>() + pos, V.p[r].counts, nr * sizeof(uint32_t), cudaMemcpyDefault, st));
@@ -980,15 +972,12 @@ template <class KT> static int sg_fallback_whole_table(Ctx* c, const SGView& V, 
     return rc;
 }
 
-// The K5 prologue of rfx_assemble_sharded and rfx_sort_kmers_sharded: the per-node arrays of the fork filters, the index over
-// the own rows, the presence bits of all ranks and the request / answer channels, published to the peers.  `chains`: also the
-// buffers of the chain ranking and the contigs (K6, K7) and their presets.  Every rank must call it (a barrier when world > 1).
-template <class KT> static int sg_k5_prologue(Ctx* c, bool chains, SGView& V, unsigned long long* all, SGProf& prof) {
-    cudaStream_t st = c->stream;
+// The buffers of the K5 prologue (sg_k5_prologue), and the sizes every rank computes the same.  A failure comes back as a
+// code: the rank still publishes it.
+template <class KT> static int sg_k5_reserve(Ctx* c, bool chains) {
     GShard* gs = c->gshard;
     const int world = c->sh_world;
     const uint64_t n_rows = c->n_rows, n = 2 * n_rows, nn = n ? n : 1;
-    unsigned long long* dstat = c->dstat.as<unsigned long long>();
     RFX_TRY(devbuf_reserve(c, c->rflag, nn * sizeof(int32_t)));
     RFX_TRY(devbuf_reserve(c, c->lflag, nn * sizeof(int32_t)));
     RFX_TRY(devbuf_reserve(c, c->alive, nn + 8));
@@ -1019,7 +1008,7 @@ template <class KT> static int sg_k5_prologue(Ctx* c, bool chains, SGView& V, un
     }
     // the own index: one region, load factor <= 1/4.  Presence bits: a region per minimiser bin of ALL ranks (SGView), the
     // region size from the global row count rfx_count_sharded left behind, so that every rank computes the same
-    const uint32_t B = c->n_bins, bps = B / (uint32_t)world;
+    const uint32_t B = c->n_bins;
     {
         const uint64_t per_bin = (c->sh_rows_global + B - 1) / B;
         uint64_t rb = (16 * per_bin + 63) / 64 * 64;
@@ -1027,7 +1016,7 @@ template <class KT> static int sg_k5_prologue(Ctx* c, bool chains, SGView& V, un
         if (rb > (1u << 24)) rb = 1u << 24;
         gs->rb = (uint32_t)rb;
     }
-    const uint64_t filter_bytes = (uint64_t)B * gs->rb / 8, slice_bytes = (uint64_t)bps * gs->rb / 8;
+    const uint64_t filter_bytes = (uint64_t)B * gs->rb / 8;
     const uint64_t slots = 4 * n_rows + 2;
     RFX_TRY(devbuf_reserve(c, c->ht, slots * sizeof(uint32_t)));
     RFX_TRY(devbuf_reserve(c, c->g_bloom, filter_bytes + 64));
@@ -1039,10 +1028,25 @@ template <class KT> static int sg_k5_prologue(Ctx* c, bool chains, SGView& V, un
     RFX_TRY(devbuf_reserve(c, gs->respbox, (size_t)world * gs->chan_cap * sizeof(uint4)));
     RFX_TRY(devbuf_reserve(c, gs->req_cnt, 3 * RFX_MAX_RANKS * sizeof(unsigned long long)));
     c->ht_cap = slots; c->g_bins = 1; c->g_m = c->m; c->g_bloom_mask = 0;
+    return RFX_OK;
+}
 
+// The K5 prologue of rfx_assemble_sharded and rfx_sort_kmers_sharded: the per-node arrays of the fork filters, the index over
+// the own rows, the presence bits of all ranks and the request / answer channels, published to the peers.  `chains`: also the
+// buffers of the chain ranking and the contigs (K6, K7) and their presets.  Every rank must call it (a barrier when world > 1),
+// with the status it has so far (`rc`): a rank that already failed reserves nothing and only publishes its code.
+template <class KT> static int sg_k5_prologue(Ctx* c, int rc, bool chains, SGView& V, PubVals& all, SGProf& prof) {
+    cudaStream_t st = c->stream;
+    GShard* gs = c->gshard;
+    const int world = c->sh_world;
+    const uint64_t n_rows = c->n_rows, n = 2 * n_rows, nn = n ? n : 1;
+    unsigned long long* dstat = c->dstat.as<unsigned long long>();
+    if (rc == RFX_OK) rc = sg_k5_reserve<KT>(c, chains);
     // everything is allocated: tell the others where (nothing behind these addresses is valid yet)
-    RFX_TRY(sg_publish(c, V, nullptr, 0, nullptr, all));
-    gs->n_rows_global = sg_sum(all, world, GP_NROWS);
+    RFX_TRY(sg_publish(c, rc, V, nullptr, 0, nullptr, all));
+    gs->n_rows_global = all.sum(GP_NROWS);
+    const uint32_t B = c->n_bins, bps = B / (uint32_t)world;
+    const uint64_t slice_bytes = (uint64_t)bps * gs->rb / 8, slots = c->ht_cap;
     prof.mark("reserve+publish1");
     // own presence bits (+ the per-row minima) first: the peers pull them while this rank builds its index
     RFX_CUDA(c, cudaMemsetAsync(gs->req_cnt.p, 0, 3 * RFX_MAX_RANKS * sizeof(unsigned long long), st));
@@ -1086,16 +1090,15 @@ template <class KT> static int sg_k5_prologue(Ctx* c, bool chains, SGView& V, un
     return RFX_OK;
 }
 
-template <class KT> static int sharded_graph_impl(Ctx* c) {
+// `rc`: the entry checks of this rank, published by the prologue
+template <class KT> static int sharded_graph_impl(Ctx* c, int rc) {
     cudaStream_t st = c->stream;
     if (!c->gshard) c->gshard = new GShard();
     GShard* gs = c->gshard;
     const int world = c->sh_world;
     const uint64_t n_rows = c->n_rows, n = 2 * n_rows, nn = n ? n : 1;
     unsigned long long* dstat = c->dstat.as<unsigned long long>();
-    unsigned long long all[RFX_MAX_RANKS * RFX_PUB_SLOTS];
-    if (n >= GID_MASK) return ctx_fail(c, RFX_E_CAPACITY, "sharded assembly: more than 2^28 rows on one rank");
-    if (!c->n_bins || c->n_bins % (uint32_t)world) return ctx_fail(c, RFX_E_STATE, "sharded assembly needs the table of rfx_count_sharded (rows sharded by minimiser bin)");
+    PubVals all;
     RFX_CUDA(c, cudaMemsetAsync(c->dstat.p, 0, DS_NSLOTS * sizeof(uint64_t), st));
     c->n_oriented = c->n_budget = c->n_budget_adm = c->n_cycles = c->n_contigs = c->n_contig_bases = 0;
     c->have_sorted = false; c->have_contigs = false;
@@ -1109,7 +1112,7 @@ template <class KT> static int sharded_graph_impl(Ctx* c) {
     // ---- K5 ----
     stage_begin(c);
     SGView V;
-    RFX_TRY(sg_k5_prologue<KT>(c, true, V, all, prof));
+    RFX_TRY(sg_k5_prologue<KT>(c, rc, true, V, all, prof));
     // (the peers' indexes are first touched by the answering kernels, behind the barrier that follows the first pass)
     const int E = c->prm.min_error_coverage;
     const uint4* rmin = gs->rmin.as<uint4>();
@@ -1150,11 +1153,11 @@ template <class KT> static int sharded_graph_impl(Ctx* c) {
     c->launches += 9;
     {
         const int slots_dev[3] = {DS_FLAGGED, DS_GRAPH_ERR, DS_REMOTE};
-        RFX_TRY(sg_publish(c, V, nullptr, 3, slots_dev, all));  // [barrier] every pred[] has its remote writes
+        RFX_TRY(sg_publish(c, RFX_OK, V, nullptr, 3, slots_dev, all));  // [barrier] every pred[] has its remote writes
     }
     prof.mark("publish2");
-    const unsigned long long flagged = sg_sum(all, world, GP_DEV + 0), gerr = sg_sum(all, world, GP_DEV + 1);
-    gs->n_remote = all[(size_t)c->sh_rank * RFX_PUB_SLOTS + PUB_GRAPH + GP_DEV + 2];
+    const unsigned long long flagged = all.sum(GP_DEV + 0), gerr = all.sum(GP_DEV + 1);
+    gs->n_remote = all.at(c->sh_rank, GP_DEV + 2);
     if (gerr) return ctx_fail(c, RFX_E_GRAPH, "sharded fork filters: a (k-1)-mer with degree > 1 (codes 1, 2), a row on a rank that does not own its minimiser bin (3) or a request channel that overflowed (4); codes add up to %llu", gerr);
     if (flagged) {
         if (n) {
@@ -1177,12 +1180,12 @@ template <class KT> static int sharded_graph_impl(Ctx* c) {
     c->launches++;
     {
         const int slots_dev[2] = {DS_NSPL, DS_NL2};
-        RFX_TRY(sg_publish(c, V, nullptr, 2, slots_dev, all));  // [barrier] spl_id / l2_of of every rank are final
+        RFX_TRY(sg_publish(c, RFX_OK, V, nullptr, 2, slots_dev, all));  // [barrier] spl_id / l2_of of every rank are final
     }
     prof.mark("select+publish3");
-    const uint64_t m1 = all[(size_t)c->sh_rank * RFX_PUB_SLOTS + PUB_GRAPH + GP_DEV + 0];
-    const uint64_t m2 = all[(size_t)c->sh_rank * RFX_PUB_SLOTS + PUB_GRAPH + GP_DEV + 1];
-    const uint64_t m2_all = sg_sum(all, world, GP_DEV + 1);
+    const uint64_t m1 = all.at(c->sh_rank, GP_DEV + 0);
+    const uint64_t m2 = all.at(c->sh_rank, GP_DEV + 1);
+    const uint64_t m2_all = all.sum(GP_DEV + 1);
     gs->n_l1 = m1; gs->n_l2 = m2;
     int rounds = 1;
     while ((1ull << rounds) < m2_all + 1) rounds++;
@@ -1235,67 +1238,69 @@ template <class KT> static int sharded_graph_impl(Ctx* c) {
     c->launches += 3;
     {
         const int slots_dev[5] = {DS_SG_CYCLE, DS_BUDGET, DS_ABSORBED, DS_CYCLES, DS_XBAR_ERR};
-        RFX_TRY(sg_publish(c, V, nullptr, 5, slots_dev, all));  // [barrier] every head knows its chain's length and right flag
+        RFX_TRY(sg_publish(c, RFX_OK, V, nullptr, 5, slots_dev, all));  // [barrier] every head knows its chain's length and right flag
     }
     prof.mark("l1_fin+node_fin+publish4");
     c->ms[4] += stage_end(c);
-    const unsigned long long any_cycle = sg_sum(all, world, GP_DEV + 0);
-    c->n_budget = all[(size_t)c->sh_rank * RFX_PUB_SLOTS + PUB_GRAPH + GP_DEV + 1];
-    c->n_budget_adm = all[(size_t)c->sh_rank * RFX_PUB_SLOTS + PUB_GRAPH + GP_DEV + 2];
-    c->n_cycles = all[(size_t)c->sh_rank * RFX_PUB_SLOTS + PUB_GRAPH + GP_DEV + 3];
+    const unsigned long long any_cycle = all.sum(GP_DEV + 0);
+    c->n_budget = all.at(c->sh_rank, GP_DEV + 1);
+    c->n_budget_adm = all.at(c->sh_rank, GP_DEV + 2);
+    c->n_cycles = all.at(c->sh_rank, GP_DEV + 3);
     if (any_cycle) {
         stage_begin(c);
         const int frc = sg_fallback_whole_table<KT>(c, V, all);
-        // nobody may touch its table before rank 0 has read it
-        RFX_TRY(shard_barrier(c));
-        RFX_TRY(shard_check(c, "sharded assembly (whole-table fallback)"));
         c->ms[5] += stage_end(c);
-        RFX_TRY(frc);
-        c->have_contigs = true;
+        // The barrier of this publish also keeps every peer from touching its table before rank 0 has read it: rank 0 enqueues
+        // it behind its copies.
         unsigned long long hv[GP_NHOST] = {c->n_contigs, c->n_contig_bases, c->n_oriented, 0, 0, 0};
-        RFX_TRY(sg_publish(c, V, hv, 0, nullptr, all));
-        gs->n_contigs_global = sg_sum(all, world, GP_HOST + 0);
-        gs->n_bases_global = sg_sum(all, world, GP_HOST + 1);
-        gs->n_oriented_global = sg_sum(all, world, GP_HOST + 2);
+        RFX_TRY(sg_publish(c, frc, V, hv, 0, nullptr, all));
+        gs->n_contigs_global = all.sum(GP_HOST + 0);
+        gs->n_bases_global = all.sum(GP_HOST + 1);
+        gs->n_oriented_global = all.sum(GP_HOST + 2);
+        c->have_contigs = true;
         return RFX_OK;
     }
 
     // ---- K7 ----
     stage_begin(c);
-    ScanPlan<U64x3> plan;
-    RFX_TRY(devbuf_reserve(c, c->scan_ws, ScanPlan<U64x3>::workspace_elems(nn) * sizeof(U64x3)));
-    plan.bind(n, c->scan_ws.as<U64x3>());
-    SContigIn in{c->alive.as<uint8_t>(), c->pred.as<uint32_t>(), c->chain_len.as<uint32_t>(), c->eff_l.as<int32_t>(), gs->tail_rf.as<int32_t>(), c->k, c->prm.min_contig};
+    // the own contigs' layout; a rank that cannot reserve it still publishes, with its code
     U64x3 tot{0, 0, 0};
-    if (n) {
-        scan_prepare(plan, in, OpAddU64x3{}, U64x3{0, 0, 0}, st);
-        c->launches += 2 * plan.levels;
-        RFX_CUDA(c, cudaMemcpyAsync(&tot, plan.total, sizeof(tot), cudaMemcpyDeviceToHost, st));
-        cudaError_t e = cudaStreamSynchronize(st);
-        if (e != cudaSuccess) return ctx_fail(c, RFX_E_CUDA, "sharded contig scan failed: %s", cudaGetErrorString(e));
-    }
-    prof.mark("contig_scan");
-    RFX_TRY(devbuf_reserve(c, c->ctg_off, (tot.a + 1) * sizeof(uint64_t)));
-    RFX_TRY(devbuf_reserve(c, c->ctg_left, (tot.a + 1) * sizeof(int32_t)));
-    RFX_TRY(devbuf_reserve(c, c->ctg_right, (tot.a + 1) * sizeof(int32_t)));
-    RFX_TRY(devbuf_reserve(c, c->ctg_bases, tot.b + 16));
-    RFX_CUDA(c, cudaMemsetAsync(c->ctg_bases.p, 0, tot.b + 16, st));  // the bases arrive as OR-ed words (sg_gather_kernel)
-    if (n) {
-        SContigOut out{c->eff_l.as<int32_t>(), gs->tail_rf.as<int32_t>(), c->ctg_idx.as<uint32_t>(), c->ctg_off.as<uint64_t>(), c->ctg_left.as<int32_t>(), c->ctg_right.as<int32_t>()};
-        scan_apply(plan, in, out, OpAddU64x3{}, U64x3{0, 0, 0}, st);
-        set_u64_kernel<<<1, 1, 0, st>>>(c->ctg_off.as<uint64_t>() + tot.a, plan.total);
-        c->launches += 2;
-    } else {
-        RFX_CUDA(c, cudaMemsetAsync(c->ctg_off.p, 0, sizeof(uint64_t), st));
-    }
+    const int lrc = [&]() -> int {
+        ScanPlan<U64x3> plan;
+        RFX_TRY(devbuf_reserve(c, c->scan_ws, ScanPlan<U64x3>::workspace_elems(nn) * sizeof(U64x3)));
+        plan.bind(n, c->scan_ws.as<U64x3>());
+        SContigIn in{c->alive.as<uint8_t>(), c->pred.as<uint32_t>(), c->chain_len.as<uint32_t>(), c->eff_l.as<int32_t>(), gs->tail_rf.as<int32_t>(), c->k, c->prm.min_contig};
+        if (n) {
+            scan_prepare(plan, in, OpAddU64x3{}, U64x3{0, 0, 0}, st);
+            c->launches += 2 * plan.levels;
+            RFX_CUDA(c, cudaMemcpyAsync(&tot, plan.total, sizeof(tot), cudaMemcpyDeviceToHost, st));
+            cudaError_t e = cudaStreamSynchronize(st);
+            if (e != cudaSuccess) return ctx_fail(c, RFX_E_CUDA, "sharded contig scan failed: %s", cudaGetErrorString(e));
+        }
+        prof.mark("contig_scan");
+        RFX_TRY(devbuf_reserve(c, c->ctg_off, (tot.a + 1) * sizeof(uint64_t)));
+        RFX_TRY(devbuf_reserve(c, c->ctg_left, (tot.a + 1) * sizeof(int32_t)));
+        RFX_TRY(devbuf_reserve(c, c->ctg_right, (tot.a + 1) * sizeof(int32_t)));
+        RFX_TRY(devbuf_reserve(c, c->ctg_bases, tot.b + 16));
+        RFX_CUDA(c, cudaMemsetAsync(c->ctg_bases.p, 0, tot.b + 16, st));  // the bases arrive as OR-ed words (sg_gather_kernel)
+        if (n) {
+            SContigOut out{c->eff_l.as<int32_t>(), gs->tail_rf.as<int32_t>(), c->ctg_idx.as<uint32_t>(), c->ctg_off.as<uint64_t>(), c->ctg_left.as<int32_t>(), c->ctg_right.as<int32_t>()};
+            scan_apply(plan, in, out, OpAddU64x3{}, U64x3{0, 0, 0}, st);
+            set_u64_kernel<<<1, 1, 0, st>>>(c->ctg_off.as<uint64_t>() + tot.a, plan.total);
+            c->launches += 2;
+        } else {
+            RFX_CUDA(c, cudaMemsetAsync(c->ctg_off.p, 0, sizeof(uint64_t), st));
+        }
+        return RFX_OK;
+    }();
     c->n_contigs = tot.a; c->n_contig_bases = tot.b; c->n_oriented = tot.c;
     {
         unsigned long long hv[GP_NHOST] = {tot.a, tot.b, tot.c, 0, 0, 0};
-        RFX_TRY(sg_publish(c, V, hv, 0, nullptr, all));  // [barrier] contig tables laid out, buffers published
+        RFX_TRY(sg_publish(c, lrc, V, hv, 0, nullptr, all));  // [barrier] contig tables laid out, buffers published
     }
-    gs->n_contigs_global = sg_sum(all, world, GP_HOST + 0);
-    gs->n_bases_global = sg_sum(all, world, GP_HOST + 1);
-    gs->n_oriented_global = sg_sum(all, world, GP_HOST + 2);
+    gs->n_contigs_global = all.sum(GP_HOST + 0);
+    gs->n_bases_global = all.sum(GP_HOST + 1);
+    gs->n_oriented_global = all.sum(GP_HOST + 2);
     prof.mark("scan_apply+publish5");
     if (m1) sg_l1_dst_kernel<<<grid_n(m1), 256, 0, st>>>(V, m1, gs->l1_fin.as<uint64_t>(), gs->l1_dst.as<unsigned long long>());
     {
@@ -1316,10 +1321,14 @@ template <class KT> static int sharded_graph_impl(Ctx* c) {
 
 int stage_assemble_sharded(Ctx* c) {
     if (c->sh_world < 1 || !c->peer_base[c->sh_rank]) return ctx_fail(c, RFX_E_STATE, "rfx_assemble_sharded: call rfx_shard_init / rfx_shard_connect first");
-    if (!c->have_counts) return ctx_fail(c, RFX_E_STATE, "rfx_assemble_sharded: no count table (call rfx_count_sharded first)");
-    if (!c->prm.bubble) return ctx_fail(c, RFX_E_UNSUPPORTED, "-bubble: undefined in the reference (see rfx_assemble)");
-    if (c->k < 2) return ctx_fail(c, RFX_E_INVALID, "assembly needs k >= 2");
-    return c->wide ? sharded_graph_impl<u128>(c) : sharded_graph_impl<uint64_t>(c);
+    int rc = RFX_OK;
+    if (!c->have_counts) rc = ctx_fail(c, RFX_E_STATE, "rfx_assemble_sharded: no count table (call rfx_count_sharded first)");
+    else if (!c->prm.bubble) rc = ctx_fail(c, RFX_E_UNSUPPORTED, "-bubble: undefined in the reference (see rfx_assemble)");
+    else if (c->k < 2) rc = ctx_fail(c, RFX_E_INVALID, "assembly needs k >= 2");
+    else if (2 * c->n_rows >= GID_MASK) rc = ctx_fail(c, RFX_E_CAPACITY, "sharded assembly: more than 2^28 rows on one rank");
+    else if (!c->n_bins || c->n_bins % (uint32_t)c->sh_world)
+        rc = ctx_fail(c, RFX_E_STATE, "sharded assembly needs the table of rfx_count_sharded (rows sharded by minimiser bin)");
+    return c->wide ? sharded_graph_impl<u128>(c, rc) : sharded_graph_impl<uint64_t>(c, rc);
 }
 
 // ---- Count_<k>_sorted across ranks (rfx_sort_kmers_sharded) -------------------------------------------------------------
@@ -1332,7 +1341,7 @@ template <class KT> static int sharded_sorted_impl(Ctx* c, int E, double fold, i
     const int world = c->sh_world;
     const uint64_t n = 2 * c->n_rows, nn = n ? n : 1;
     unsigned long long* dstat = c->dstat.as<unsigned long long>();
-    unsigned long long all[RFX_MAX_RANKS * RFX_PUB_SLOTS];
+    PubVals all;
     RFX_CUDA(c, cudaMemsetAsync(c->dstat.p, 0, DS_NSLOTS * sizeof(uint64_t), st));
     c->n_sorted = 0;
     c->have_sorted = false; c->have_contigs = false;  // the index, the alive bytes and the flag arrays are taken over
@@ -1343,10 +1352,10 @@ template <class KT> static int sharded_sorted_impl(Ctx* c, int E, double fold, i
     prof.on = getenv("RFX_SHARD_PROF") != nullptr && c->sh_rank == 0;
     prof.st = st;
     prof.mark("start");
-    RFX_TRY(devbuf_reserve(c, c->srt_left, nn * sizeof(int32_t)));
-    RFX_TRY(devbuf_reserve(c, c->srt_right, nn * sizeof(int32_t)));
+    int rc = devbuf_reserve(c, c->srt_left, nn * sizeof(int32_t));
+    if (rc == RFX_OK) rc = devbuf_reserve(c, c->srt_right, nn * sizeof(int32_t));
     SGView V;
-    RFX_TRY(sg_k5_prologue<KT>(c, false, V, all, prof));
+    RFX_TRY(sg_k5_prologue<KT>(c, rc, false, V, all, prof));
     const uint4* rmin = gs->rmin.as<uint4>();
     // pass 1 over the own nodes (requests out), [barrier], the owners answer, [barrier], pass 2 over the nodes that waited
     const unsigned g2 = sm_count() * 8u;
@@ -1378,9 +1387,9 @@ template <class KT> static int sharded_sorted_impl(Ctx* c, int E, double fold, i
     c->launches += world > 1 ? 6 : 2;
     // survivors (alive & 2), as rfx_sort_kmers counts them
     uint64_t total = 0;
-    if (n) {
+    const int rc_scan = n ? devbuf_reserve(c, c->scan_ws, ScanPlan<uint64_t>::workspace_elems(n) * sizeof(uint64_t)) : RFX_OK;
+    if (n && rc_scan == RFX_OK) {
         ScanPlan<uint64_t> plan;
-        RFX_TRY(devbuf_reserve(c, c->scan_ws, ScanPlan<uint64_t>::workspace_elems(n) * sizeof(uint64_t)));
         plan.bind(n, c->scan_ws.as<uint64_t>());
         scan_prepare(plan, AliveBoth{c->alive.as<uint8_t>()}, OpAddU64{}, (uint64_t)0, st);
         c->launches += 2 * plan.levels;
@@ -1391,18 +1400,14 @@ template <class KT> static int sharded_sorted_impl(Ctx* c, int E, double fold, i
     prof.mark("survivors");
     // [barrier] every rank is done with its channels; survivors and error words of all ranks
     {
-        const unsigned long long mine[3] = {total, 0, 0};  // slots 1, 2: filled from the device counters
-        const int slots_dev[2] = {DS_GRAPH_ERR, DS_REMOTE};
-        RFX_TRY(shard_exchange(c, PUB_TABLE, 3, mine, all, 2, slots_dev, PUB_TABLE + 1));
+        const unsigned long long mine[1] = {total};
+        const int slots_dev[2] = {DS_GRAPH_ERR, DS_REMOTE};  // values 1, 2
+        RFX_TRY(shard_exchange(c, rc_scan, 1, mine, all, 2, slots_dev));
     }
     prof.mark("exchange");
-    unsigned long long survivors = 0, gerr = 0;
-    for (int r = 0; r < world; r++) {
-        survivors += all[(size_t)r * RFX_PUB_SLOTS + PUB_TABLE];
-        gerr += all[(size_t)r * RFX_PUB_SLOTS + PUB_TABLE + 1];
-    }
-    gs->n_remote = all[(size_t)c->sh_rank * RFX_PUB_SLOTS + PUB_TABLE + 2];
-    gs->n_oriented_global = survivors;
+    const unsigned long long gerr = all.sum(1);
+    gs->n_remote = all.at(c->sh_rank, 2);
+    gs->n_oriented_global = all.sum(0);
     c->ms[3] = stage_end(c);
     prof.report(c->sh_rank);
     if (gerr) return ctx_fail(c, RFX_E_GRAPH, "sharded sorted filters: a row on a rank that does not own its minimiser bin (code 3) or a request channel that overflowed (4); codes add up to %llu", gerr);
@@ -1414,32 +1419,32 @@ template <class KT> static int sharded_sorted_impl(Ctx* c, int E, double fold, i
 int stage_sorted_sharded(Ctx* c, int E, double fold, int max_kmer_size) {
     if (c->sh_world < 1 || !c->peer_base[c->sh_rank]) return ctx_fail(c, RFX_E_STATE, "rfx_sort_kmers_sharded: call rfx_shard_init / rfx_shard_connect first");
     const int world = c->sh_world;
-    unsigned long long mine[7], all[RFX_MAX_RANKS * RFX_PUB_SLOTS] = {};
-    auto got = [&](int r, int slot) { return all[(size_t)r * RFX_PUB_SLOTS + PUB_TABLE + slot]; };
+    unsigned long long mine[6];
+    static_assert(sizeof(mine) / sizeof(mine[0]) <= PUB_VALS, "the agreement exchange fits the published block");
+    PubVals all;
     c->ms_comm = 0;
     stage_begin(c);
     // What every rank holds and was asked for, before any barrier or buffer.  Every rank checks every rank's values in the same
-    // order, so that all ranks return the same error together instead of leaving their peers in a barrier.
+    // order, so that all ranks return the same error together.
+    const bool sharded = c->have_counts && c->n_bins && c->n_bins % (uint32_t)world == 0;
+    const int rc = sharded ? RFX_OK
+                           : ctx_fail(c, RFX_E_STATE, "rfx_sort_kmers_sharded: this rank holds no table sharded by minimiser bin (rfx_count_sharded, or rfx_load_counts* and rfx_shard_table first)");
     unsigned long long fold_bits = 0;
     memcpy(&fold_bits, &fold, sizeof(fold_bits));
-    mine[0] = c->have_counts && c->n_bins && c->n_bins % (uint32_t)world == 0 ? 1 : 0;
-    mine[1] = (unsigned long long)c->k;
-    mine[2] = c->n_bins;
-    mine[3] = (uint32_t)E;
-    mine[4] = fold_bits;
-    mine[5] = (uint32_t)max_kmer_size;
-    mine[6] = c->have_counts ? c->n_rows : 0;
-    RFX_TRY(shard_exchange(c, PUB_TABLE, 7, mine, all));
-    for (int r = 0; r < world; r++)
-        if (!got(r, 0))
-            return ctx_fail(c, RFX_E_STATE, "rfx_sort_kmers_sharded: rank %d holds no table sharded by minimiser bin (rfx_count_sharded, or rfx_load_counts* and rfx_shard_table first)", r);
-    static const char* what[6] = {"", "k", "bin count", "min_error_coverage", "min_repeat_fold", "max_kmer_size"};
+    mine[0] = (unsigned long long)c->k;
+    mine[1] = c->n_bins;
+    mine[2] = (uint32_t)E;
+    mine[3] = fold_bits;
+    mine[4] = (uint32_t)max_kmer_size;
+    mine[5] = c->have_counts ? c->n_rows : 0;
+    RFX_TRY(shard_exchange(c, rc, 6, mine, all));
+    static const char* what[5] = {"k", "bin count", "min_error_coverage", "min_repeat_fold", "max_kmer_size"};
     for (int r = 1; r < world; r++)
-        for (int s = 1; s < 6; s++)
-            if (got(r, s) != got(0, s)) return ctx_fail(c, RFX_E_INVALID, "rfx_sort_kmers_sharded: rank %d has another %s than rank 0", r, what[s]);
+        for (int s = 0; s < 5; s++)
+            if (all.at(r, s) != all.at(0, s)) return ctx_fail(c, RFX_E_INVALID, "rfx_sort_kmers_sharded: rank %d has another %s than rank 0", r, what[s]);
     RFX_TRY(sorted_domain(c, "rfx_sort_kmers_sharded", E, fold, max_kmer_size));
     for (int r = 0; r < world; r++)
-        if (2 * got(r, 6) >= GID_MASK) return ctx_fail(c, RFX_E_CAPACITY, "rfx_sort_kmers_sharded: rank %d holds more than 2^28 rows", r);
+        if (2 * all.at(r, 5) >= GID_MASK) return ctx_fail(c, RFX_E_CAPACITY, "rfx_sort_kmers_sharded: rank %d holds more than 2^28 rows", r);
     return c->wide ? sharded_sorted_impl<u128>(c, E, fold, max_kmer_size + 3) : sharded_sorted_impl<uint64_t>(c, E, fold, max_kmer_size + 3);
 }
 

@@ -212,6 +212,6 @@ class LocalRanks:
         failed = [(r, e) for r, e in enumerate(err) if e is not None]
         if len(failed) == 1:
             raise failed[0][1]
-        if failed:  # a rank that fails leaves its peers waiting in a barrier until they time out: show every rank's story
+        if failed:  # a collective call fails on every rank at once; other code in `fn` may fail on some: show every rank's story
             raise RuntimeError("; ".join(f"rank {r}: {e}" for r, e in failed)) from failed[0][1]
         return out

@@ -203,18 +203,65 @@ def test_reads_then_table_then_reads_on_the_same_contexts(R, orc):
             c.close()
 
 
-def test_closed_paths(R, orc):
-    """A circular genome has no head: the sharded assembly falls back to rank 0 assembling the whole table."""
+def _tiled_table(orc, glen, seed, circular):
+    """Error-free reads tiling a genome of glen bases every 7 bases, twice: oracle table and its rfx_load_counts layout."""
     from workload import synth
-    g = synth.genome(2000, 9)
-    circ = bytes(g) + bytes(g[:200])
-    reads = [circ[i:i + 120] for i in range(0, 2000, 7)] * 2
+    g = bytes(synth.genome(glen, seed))
+    src = g + g[:200] if circular else g
+    reads = [src[i:i + 120] for i in range(0, glen if circular else glen - 119, 7)] * 2
     txt = "".join(f"@r{i}\n{r.decode()}\n+\n{'I' * len(r)}\n" for i, r in enumerate(reads)).encode()
     t = _oracle_table(orc, txt, 31, 2)
-    keys, cnt = _ref_layout(t, 31), t["counts"].astype(np.uint32)
+    return t, _ref_layout(t, 31), t["counts"].astype(np.uint32)
+
+
+def test_closed_paths(R, orc):
+    """A circular genome has no head: the sharded assembly falls back to rank 0 assembling the whole table."""
+    t, keys, cnt = _tiled_table(orc, 2000, 9, circular=True)
     results = _run_loaded(R, _contiguous(keys, cnt, 2), 31, min_contig=50)
     a, fell_back = _check_against_oracle(orc, t, 31, 8, 50, results)
     assert fell_back and a["n_cycles"] >= 1
+
+
+def test_closed_paths_fallback_failing_on_rank_0_fails_on_every_rank_at_once(R, orc):
+    """The arena holds everything both ranks need up to the whole-table fallback, not rank 0's copy of the whole table and
+    the single-GPU stages on it: every rank returns rank 0's RFX_E_NOMEM within seconds, and the contexts stay usable."""
+    from reflexiv_b200 import _lib, sharded
+    t, keys, cnt = _tiled_table(orc, 2000, 9, circular=True)
+    slices = _contiguous(keys, cnt, 2)
+    # how much of the arena every rank uses, from a run in a large arena (the layout of a bump allocator is deterministic);
+    # only rank 0 reserves anything in the fallback
+    used = [r["sh"]["arena_used"] for r in _run_loaded(R, slices, 31, min_contig=50)]
+    arena = (used[0] - 1) & ~4095  # rfx_shard_init rounds up to 4 KiB: below what rank 0 needs at the end of its fallback
+    assert max(used[1:]) <= arena, (used, arena)  # ... and above what rank 1 needs, and rank 0 before the fallback
+
+    ctxs = _ctxs(R, 2, 31, min_contig=50)
+    try:
+        grp = sharded.LocalRanks(ctxs, arena_bytes=arena)
+
+        def body(rank, ctx):
+            ctx.reset()
+            ctx.load_counts(*slices[rank])
+            ctx.shard_table()
+            try:
+                ctx.assemble_sharded()
+            except _lib.RfxError as err:
+                return err
+            return None
+        t0 = time.perf_counter()
+        errs = grp.run(body)
+        took = time.perf_counter() - t0
+        assert all(e is not None and e.code == _lib.RFX_E_NOMEM for e in errs), errs
+        assert "arena exhausted" in str(errs[0]) and "rank 0" in str(errs[1])
+        assert took < 5.0  # the fallback's exchange carries rank 0's status: rank 1 does not wait for a barrier to time out
+        assert ctxs[0].shard_stats()["fell_back"] and ctxs[1].shard_stats()["fell_back"]
+        # the ranks stay in step: the same contexts then assemble a linear genome correctly
+        t2, keys2, cnt2 = _tiled_table(orc, 1000, 10, circular=False)
+        results = [None] * 2
+        grp.run(_load_body(_contiguous(keys2, cnt2, 2), results))
+        _check_against_oracle(orc, t2, 31, 8, 50, results)
+    finally:
+        for c in ctxs:
+            c.close()
 
 
 def test_errors_come_back_from_every_rank_at_once(R, orc):
@@ -230,24 +277,29 @@ def test_errors_come_back_from_every_rank_at_once(R, orc):
     ctxs = _ctxs(R, world, 31)
     try:
         grp = sharded.LocalRanks(ctxs, arena_bytes=1 << 30)
-
-        def body(rank, ctx):
-            ctx.reset()
-            if rank != 1:  # rank 1 never loads a table
-                ctx.load_counts(*slices[rank])
-            try:
-                ctx.shard_table()
-            except _lib.RfxError as err:
-                return err.code
-            return 0
-        t0 = time.perf_counter()
-        codes = grp.run(body)
-        assert codes == [_lib.RFX_E_STATE] * world
-        assert time.perf_counter() - t0 < 5.0  # the first exchange catches it: nobody waits for a barrier to time out
-        # the ranks stay in step: the same contexts then re-shard and assemble correctly
-        results = [None] * world
-        grp.run(_load_body(slices, results))
-        _check_against_oracle(orc, t, 31, 8, 100, results)
+        # rank 1 holds no table: it never loads one (shard_table), or it drops its shard before the assembly
+        for case in ("shard_table", "assemble_sharded"):
+            def body(rank, ctx):
+                ctx.reset()
+                if rank != 1 or case == "assemble_sharded":
+                    ctx.load_counts(*slices[rank])
+                try:
+                    ctx.shard_table()
+                    if case == "assemble_sharded":
+                        if rank == 1:
+                            ctx.reset()
+                        ctx.assemble_sharded()
+                except _lib.RfxError as err:
+                    return err.code
+                return 0
+            t0 = time.perf_counter()
+            codes = grp.run(body)
+            assert codes == [_lib.RFX_E_STATE] * world, case
+            assert time.perf_counter() - t0 < 5.0  # the first exchange catches it: nobody waits for a barrier to time out
+            # the ranks stay in step: the same contexts then re-shard and assemble correctly
+            results = [None] * world
+            grp.run(_load_body(slices, results))
+            _check_against_oracle(orc, t, 31, 8, 100, results)
     finally:
         for c in ctxs:
             c.close()
