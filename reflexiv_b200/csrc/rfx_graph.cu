@@ -12,7 +12,8 @@
 // Data layout in HBM: the filtered table (keys[], counts[]) is the only copy of the k-mers.  An
 // oriented k-mer is an id  oid = 2*row + strand  (strand 1 = reverse complement of keys[row]); every
 // per-node array (flags, links, ranks) is indexed by oid.  A 32-bit open-addressing index (ht[]) maps a
-// canonical k-mer to its row; neighbours are found by probing the 4 possible extensions.
+// canonical k-mer to its row.  K5 probes it once per node for the 4 possible successors and stores them (N(Y), below);
+// both fork filters and the links read their neighbour sets from there.
 //
 // After the two fork filters every (k-1)-mer has at most one surviving out-edge and one in-edge, so
 // the reference's sort-and-merge iteration converges to the maximal paths of that graph; pointer
@@ -29,9 +30,10 @@ namespace rfx {
 
 // The index is local to minimiser bins: a row lives in the hash region of the bin its canonical minimiser hashes to
 // (regions are back to back in ht[], 4 * rows + 2 slots each).  A neighbour shares k-1 bases with the node that asks
-// for it, so its minimiser -- hence its region -- is almost always the node's own: the probes of the fork filters and
-// of the link pass stay inside a few hundred bytes that the neighbouring threads (rows come out of the counting
-// kernel grouped by bin) have just touched, instead of landing anywhere in a table of hundreds of megabytes.  The
+// for it, so its minimiser -- hence its region -- is almost always the node's own: the probes of the adjacency pass
+// (and of the fork filters' direct fallback) stay inside a few hundred bytes that the neighbouring threads (rows come
+// out of the counting kernel grouped by bin) have just touched, instead of landing anywhere in a table of hundreds of
+// megabytes.  The
 // asking node computes the m-mer hashes of its own k-mer once; a candidate's minimiser is then the minimum over the
 // shared (k-1)-mer plus one new m-mer.  (The same bin -> owner map is what lets a sharded run route a probe.)
 template <class KT> struct Graph {
@@ -129,15 +131,91 @@ template <class KT> __global__ void ht_build_kernel(Graph<KT> G, const uint32_t*
     }
 }
 
+// ---- K5: adjacency, fork filters, links ---------------------------------------------------------------------------
+// The index is probed once per oriented k-mer: the adjacency pass stores N(Y), the oriented ids of the 4 possible
+// successors suffix(Y)·b of every oriented k-mer Y (slot b, NONE32 where absent), 16 B per oriented id.  Every
+// neighbour set the filters and the links need is one of these sets, read at the node or at a neighbour:
+//   successors of Y              N(Y)
+//   predecessors of Y            { rc(z) : z in N(Y^1) }                 (Y^1: the other strand, the same row)
+//   right group  prefix(Y)·b     N(P), P any predecessor of Y           (slot b)
+//   left group   a·suffix(Y)     { rc(z) : z in N(S^1) }, S any successor of Y   (slot 3 - a holds rc(a·suffix(Y)))
+// so a node costs 4 index probes instead of 10.  A node without a predecessor (successor) has no stored set that names
+// its right (left) group; it probes its siblings directly.  On clean data those are the chain ends; on noisy data the
+// error tips.
+// The even ids' sets are in s[0], the odd ids' in s[1], both indexed by row.
+struct Adj {
+    uint4* s[2];
+    __device__ __forceinline__ uint4* set(uint64_t oid) const { return ((oid & 1u) ? s[1] : s[0]) + (oid >> 1); }  // (a select: no local copy of s)
+    __device__ __forceinline__ uint4 out(uint32_t oid) const { return *set(oid); }
+};
+__device__ __forceinline__ uint32_t adj_slot(const uint4& v, uint32_t b) { return b == 0 ? v.x : b == 1 ? v.y : b == 2 ? v.z : v.w; }
+
+template <class KT> __device__ __forceinline__ bool is_palindrome(const Graph<KT>& G, KT Z) { return !(G.k & 1) && revcomp(Z, G.k) == Z; }
+// oriented id of revcomp(Z), given z = find(Z): the other strand of z's row -- except for a palindromic row, which is
+// one node: find returns its even id, and the odd id is not a node (alive = 0)
+template <class KT> __device__ __forceinline__ uint32_t rc_oid(const Graph<KT>& G, uint32_t z, KT Z) { return is_palindrome(G, Z) ? z : z ^ 1u; }
+
+template <class KT>
+__global__ void __launch_bounds__(256) adjacency_kernel(Graph<KT> G, Adj A, uint64_t n) {
+    const KT sufmask = mask_bases<KT>(G.k - 1);
+    for (uint64_t oid = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; oid < n; oid += (uint64_t)gridDim.x * blockDim.x) {
+        const KT X = G.oriented((uint32_t)oid);
+        const KT suffix = X & sufmask;
+        uint32_t pre_min = 0, suf_min = 0;
+        if (G.g_bins > 1) G.minima(X, pre_min, suf_min);
+        uint32_t s[4];
+#pragma unroll
+        for (uint32_t b = 0; b < 4; b++) {
+            uint32_t cz;
+            const uint32_t hl = G.g_bins > 1 ? G.last_mm(suffix, b) : 0u;
+            s[b] = G.find((suffix << 2) | (KT)b, hl < suf_min ? hl : suf_min, &cz);
+        }
+        *A.set(oid) = make_uint4(s[0], s[1], s[2], s[3]);
+    }
+}
+
+// counts of the group prefix(X)·b by probing the 3 siblings of X (own: X's count)
+template <class KT> __device__ __forceinline__ void probe_right_group(const Graph<KT>& G, KT X, uint32_t own, uint32_t cnt[4]) {
+    const KT prefix = X >> 2;
+    const uint32_t myb = (uint32_t)X & 3u;
+    uint32_t pre_min = 0, suf_min = 0;
+    if (G.g_bins > 1) G.minima(X, pre_min, suf_min);
+#pragma unroll
+    for (uint32_t b = 0; b < 4; b++) {
+        if (b == myb) { cnt[b] = own; continue; }
+        const KT Z = (prefix << 2) | (KT)b;
+        const KT zc = revcomp(Z, G.k);
+        const uint32_t hl = G.g_bins > 1 ? G.last_mm(prefix, b) : 0u;
+        const uint32_t r = G.lookup(zc < Z ? zc : Z, hl < pre_min ? hl : pre_min);
+        cnt[b] = r == NONE32 ? 0u : G.counts[r];
+    }
+}
+// counts of the right-filter survivors among a·suffix(X) by probing the 3 siblings of X (own: X's count)
+template <class KT> __device__ __forceinline__ void probe_left_group(const Graph<KT>& G, KT X, const uint8_t* alive, uint32_t own, uint32_t cnt[4]) {
+    const int top = 2 * (G.k - 1);
+    const KT suffix = X & mask_bases<KT>(G.k - 1);
+    const uint32_t mya = (uint32_t)(X >> top) & 3u;
+    uint32_t pre_min = 0, suf_min = 0;
+    if (G.g_bins > 1) G.minima(X, pre_min, suf_min);
+#pragma unroll
+    for (uint32_t a = 0; a < 4; a++) {
+        if (a == mya) { cnt[a] = own; continue; }
+        uint32_t cz = 0;
+        const uint32_t hf = G.g_bins > 1 ? G.first_mm(suffix, a) : 0u;
+        const uint32_t oz = G.find(((KT)a << top) | suffix, hf < suf_min ? hf : suf_min, &cz);
+        cnt[a] = (oz != NONE32 && (alive[oz] & 1)) ? cz : 0u;
+    }
+}
+
 // The alive byte of an oriented k-mer: bit0 survives the right fork filter, bit1 survives both, bit2 right flag < 0,
 // bit3 left flag < 0.  The sign bits are all a neighbour needs to know about a node's flags (junction_joins), so in
 // a sharded run one byte per node is the only per-node state that crosses GPUs.
-// All per-node kernels take an oid range [lo, hi): the whole table on one GPU, the rank's own rows in a sharded run.
 //
 // A7.
 template <class KT>
-__global__ void right_filter_kernel(Graph<KT> G, int E, uint8_t* __restrict__ alive, int32_t* __restrict__ rflag, uint64_t lo, uint64_t hi) {
-    for (uint64_t oid = lo + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; oid < hi; oid += (uint64_t)gridDim.x * blockDim.x) {
+__global__ void __launch_bounds__(256) right_filter_kernel(Graph<KT> G, Adj A, int E, uint8_t* __restrict__ alive, int32_t* __restrict__ rflag, uint64_t n) {
+    const KT sufmask = mask_bases<KT>(G.k - 1);
+    for (uint64_t oid = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; oid < n; oid += (uint64_t)gridDim.x * blockDim.x) {
         const uint32_t row = (uint32_t)(oid >> 1);
         const KT key = G.keys[row];
         const KT rc = revcomp(key, G.k);
@@ -145,22 +223,25 @@ __global__ void right_filter_kernel(Graph<KT> G, int E, uint8_t* __restrict__ al
         const KT X = (oid & 1u) ? rc : key;
         const KT prefix = X >> 2;
         const uint32_t myb = (uint32_t)X & 3u;
-        uint32_t pre_min = 0, suf_min = 0;
-        if (G.g_bins > 1) G.minima(X, pre_min, suf_min);
+        // a predecessor: the reverse complement of a successor of revcomp(X), whose out-set is stored next to X's
+        const KT rpre = ((oid & 1u) ? key : rc) & sufmask;  // revcomp(prefix(X))
+        const uint4 in = A.out((uint32_t)oid ^ 1u);
+        uint32_t z = NONE32, zc = 0;
+#pragma unroll
+        for (int c = 3; c >= 0; c--)
+            if (adj_slot(in, c) != NONE32) { z = adj_slot(in, c); zc = c; }
+        const uint32_t own = G.counts[row];
         uint32_t cnt[4];
+        if (z != NONE32) {
+            const uint4 grp = A.out(rc_oid(G, z, (rpre << 2) | (KT)zc));
+#pragma unroll
+            for (uint32_t b = 0; b < 4; b++) cnt[b] = b == myb ? own : adj_slot(grp, b) == NONE32 ? 0u : G.counts[adj_slot(grp, b) >> 1];
+        } else {
+            probe_right_group(G, X, own, cnt);
+        }
         bool dup[4];
 #pragma unroll
-        for (uint32_t b = 0; b < 4; b++) {
-            if (b == myb) { cnt[b] = G.counts[row]; dup[b] = (rc == key); }
-            else {
-                const KT Z = (prefix << 2) | (KT)b;
-                const KT zc = revcomp(Z, G.k);
-                const uint32_t hl = G.g_bins > 1 ? G.last_mm(prefix, b) : 0u;
-                const uint32_t r = G.lookup(zc < Z ? zc : Z, hl < pre_min ? hl : pre_min);
-                cnt[b] = r == NONE32 ? 0u : G.counts[r];
-                dup[b] = (Z == zc);
-            }
-        }
+        for (uint32_t b = 0; b < 4; b++) dup[b] = is_palindrome(G, (prefix << 2) | (KT)b);
         const ForkResult res = right_fork(cnt, dup, E, G.k - 1);
         alive[oid] = (uint8_t)(((res.winner == (int)myb) ? 1 : 0) | (res.flag < 0 ? 4 : 0));
         rflag[oid] = res.flag;
@@ -169,27 +250,32 @@ __global__ void right_filter_kernel(Graph<KT> G, int E, uint8_t* __restrict__ al
 
 // A8.
 template <class KT>
-__global__ void left_filter_kernel(Graph<KT> G, int E, uint8_t* alive, int32_t* __restrict__ lflag, uint64_t lo, uint64_t hi) {
+__global__ void __launch_bounds__(256) left_filter_kernel(Graph<KT> G, Adj A, int E, uint8_t* alive, int32_t* __restrict__ lflag, uint64_t n) {
     const int top = 2 * (G.k - 1);
     const KT sufmask = mask_bases<KT>(G.k - 1);
-    for (uint64_t oid = lo + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; oid < hi; oid += (uint64_t)gridDim.x * blockDim.x) {
+    for (uint64_t oid = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; oid < n; oid += (uint64_t)gridDim.x * blockDim.x) {
         lflag[oid] = 0;
         if (!(alive[oid] & 1)) continue;
         const KT X = G.oriented((uint32_t)oid);
         const KT suffix = X & sufmask;
         const uint32_t mya = (uint32_t)(X >> top) & 3u;
-        uint32_t pre_min = 0, suf_min = 0;
-        if (G.g_bins > 1) G.minima(X, pre_min, suf_min);
-        uint32_t cnt[4];
+        const uint4 out = A.out((uint32_t)oid);
+        uint32_t s = NONE32, sb = 0;
 #pragma unroll
-        for (uint32_t a = 0; a < 4; a++) {
-            if (a == mya) cnt[a] = G.counts[oid >> 1];
-            else {
-                uint32_t cz = 0;
-                const uint32_t hf = G.g_bins > 1 ? G.first_mm(suffix, a) : 0u;
-                const uint32_t oz = G.find(((KT)a << top) | suffix, hf < suf_min ? hf : suf_min, &cz);
-                cnt[a] = (oz != NONE32 && (alive[oz] & 1)) ? cz : 0u;
+        for (int b = 3; b >= 0; b--)
+            if (adj_slot(out, b) != NONE32) { s = adj_slot(out, b); sb = b; }
+        const uint32_t own = G.counts[oid >> 1];
+        uint32_t cnt[4];
+        if (s != NONE32) {
+            const uint4 grp = A.out(rc_oid(G, s, (suffix << 2) | (KT)sb));
+#pragma unroll
+            for (uint32_t a = 0; a < 4; a++) {
+                const uint32_t z = adj_slot(grp, 3 - a);
+                const uint32_t oz = (a == mya || z == NONE32) ? NONE32 : rc_oid(G, z, ((KT)a << top) | suffix);
+                cnt[a] = a == mya ? own : (oz != NONE32 && (alive[oz] & 1)) ? G.counts[z >> 1] : 0u;
             }
+        } else {
+            probe_left_group(G, X, alive, own, cnt);
         }
         const ForkResult res = left_fork(cnt, E, G.k - 1);
         if (res.winner == (int)mya) { alive[oid] = (uint8_t)((alive[oid] & 4) | 3 | (res.flag < 0 ? 8 : 0)); lflag[oid] = res.flag; }
@@ -197,8 +283,8 @@ __global__ void left_filter_kernel(Graph<KT> G, int E, uint8_t* alive, int32_t* 
 }
 
 // ---- Count_<k>_sorted (SURVEY 8f-2): the fork filters of ReflexivDSKmerLeftAndRightSorting.java ----------------
-// Same probing as A7 / A8; what differs is the rule (sorted_right_fork / sorted_left_fork, rfx_core.h) and that the
-// left filter needs, from every candidate, the coverage and the right flag the right filter left on it.
+// Every node probes its siblings in the index; what differs from A7 / A8 is the rule (sorted_right_fork /
+// sorted_left_fork, rfx_core.h) and that the left filter needs, from every candidate, the coverage and the right flag the right filter left on it.
 template <class KT>
 __global__ void sorted_right_kernel(Graph<KT> G, int E, double fold, int X, uint8_t* __restrict__ alive, int32_t* __restrict__ cov, int32_t* __restrict__ rflag,
                                     uint64_t n) {
@@ -266,23 +352,16 @@ __global__ void sorted_left_kernel(Graph<KT> G, int E, double fold, int X, uint8
 // Neighbour links.  succ/pred are preset to NONE32.  A node writes its successor's pred[] and EVERY junction is linked
 // (raw links): which of them hold is decided afterwards (budget walks + junction_finalize_kernel) and only matters when
 // some flag is non-negative, i.e. a real fork survived (DS_FLAGGED).
-template <class KT>
-__global__ void link_kernel(Graph<KT> G, const uint8_t* __restrict__ alive, const int32_t* __restrict__ lflag, const int32_t* __restrict__ rflag,
-                            uint32_t* __restrict__ succ, uint32_t* pred, unsigned long long* dstat, uint64_t lo, uint64_t hi) {
-    const KT sufmask = mask_bases<KT>(G.k - 1);
-    for (uint64_t oid = lo + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; oid < hi; oid += (uint64_t)gridDim.x * blockDim.x) {
+__global__ void __launch_bounds__(256) link_kernel(Adj A, const uint8_t* __restrict__ alive, const int32_t* __restrict__ lflag, const int32_t* __restrict__ rflag,
+                                                   uint32_t* __restrict__ succ, uint32_t* pred, unsigned long long* dstat, uint64_t n) {
+    for (uint64_t oid = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; oid < n; oid += (uint64_t)gridDim.x * blockDim.x) {
         if (!(alive[oid] & 2)) continue;
-        const KT X = G.oriented((uint32_t)oid);
-        const KT suffix = X & sufmask;
-        uint32_t pre_min = 0, suf_min = 0;
-        if (G.g_bins > 1) G.minima(X, pre_min, suf_min);
+        const uint4 out = A.out((uint32_t)oid);
         uint32_t next = NONE32;
         int n_cand = 0;
 #pragma unroll
         for (uint32_t b = 0; b < 4; b++) {
-            uint32_t cz;
-            const uint32_t hl = G.g_bins > 1 ? G.last_mm(suffix, b) : 0u;
-            const uint32_t oy = G.find((suffix << 2) | (KT)b, hl < suf_min ? hl : suf_min, &cz);
+            const uint32_t oy = adj_slot(out, b);
             if (oy != NONE32 && (alive[oy] & 2)) { next = oy; n_cand++; }
         }
         if (n_cand > 1) { atomicExch(&dstat[DS_GRAPH_ERR], 1ull); continue; }
@@ -698,10 +777,13 @@ template <class KT> static int graph_impl(Ctx* c) {
         int32_t* rflag = c->rflag.as<int32_t>();
         uint32_t* succ = c->succ.as<uint32_t>();
         uint32_t* pred = c->pred.as<uint32_t>();
-        right_filter_kernel<KT><<<grid_n(n), 256, 0, st>>>(G, E, alive, rflag, 0, n);
-        left_filter_kernel<KT><<<grid_n(n), 256, 0, st>>>(G, E, alive, lflag, 0, n);
-        link_kernel<KT><<<grid_n(n), 256, 0, st>>>(G, alive, lflag, rflag, succ, pred, dstat, 0, n);
-        c->launches += 3;
+        // the out-sets live in the splitter buffers, which nothing reads before K6 writes them
+        const Adj A{{c->sp_ad[0].as<uint4>(), c->sp_ad[1].as<uint4>()}};
+        adjacency_kernel<KT><<<grid_n(n), 256, 0, st>>>(G, A, n);
+        right_filter_kernel<KT><<<grid_n(n), 256, 0, st>>>(G, A, E, alive, rflag, n);
+        left_filter_kernel<KT><<<grid_n(n), 256, 0, st>>>(G, A, E, alive, lflag, n);
+        link_kernel<<<grid_n(n), 256, 0, st>>>(A, alive, lflag, rflag, succ, pred, dstat, n);
+        c->launches += 4;
         cudaMemcpyAsync(h, c->dstat.p, sizeof(h), cudaMemcpyDeviceToHost, st);
         cudaError_t e = cudaStreamSynchronize(st);
         if (e != cudaSuccess) { rc = ctx_fail(c, RFX_E_CUDA, "graph kernels failed: %s", cudaGetErrorString(e)); break; }
