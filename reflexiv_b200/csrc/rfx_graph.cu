@@ -22,6 +22,8 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <utility>
+
 #include "rfx_internal.h"
 #include "rfx_graph.cuh"
 #include "rfx_scan.cuh"
@@ -509,30 +511,72 @@ __global__ void __launch_bounds__(256) rank_all_kernel(const unsigned long long*
     if (blockIdx.x == 0 && threadIdx.x == 0) dstat[DS_RANK_CUR] = (unsigned long long)cur;
 }
 
+// Index of a new entry for every thread that wants one, ~0 for the others: ONE global atomic per block and call (a quarter
+// of a million warps bumping the same counter cost more than the kernel around them).  Every thread of the block must call.
+__device__ __forceinline__ unsigned long long block_reserve(bool want, unsigned long long* counter) {
+    __shared__ uint32_t s_count;
+    __shared__ unsigned long long s_base;
+    const uint32_t lane = threadIdx.x & 31u;
+    if (threadIdx.x == 0) s_count = 0;
+    __syncthreads();
+    const uint32_t m = __ballot_sync(0xffffffffu, want);
+    uint32_t wbase = 0;
+    if (lane == 0 && m) wbase = atomicAdd(&s_count, (uint32_t)__popc(m));
+    wbase = __shfl_sync(0xffffffffu, wbase, 0);
+    __syncthreads();
+    if (threadIdx.x == 0 && s_count) s_base = atomicAdd(counter, (unsigned long long)s_count);
+    __syncthreads();
+    return want ? s_base + wbase + __popc(m & ((1u << lane) - 1u)) : ~0ull;
+}
+// Adds every thread's v to *counter with ONE global atomic per block.  Every thread of the block must call.
+__device__ __forceinline__ void block_add(unsigned long long v, unsigned long long* counter) {
+    __shared__ unsigned long long s_sum;
+    if (threadIdx.x == 0) s_sum = 0;
+    __syncthreads();
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
+    if ((threadIdx.x & 31u) == 0 && v) atomicAdd(&s_sum, v);
+    __syncthreads();
+    if (threadIdx.x == 0 && s_sum) atomicAdd(counter, s_sum);
+}
+
 // ---- K6 (work-efficient variant): rank through a sample of splitters ------------------------------------------
 // Heads and one node in 16 (hash of the id) are splitters.  Each splitter walks its successors up to the next
 // splitter, stamping (owner, offset) on the way: every node is touched once.  Only the splitter list (n/16 entries,
-// L2 resident) goes through pointer jumping; a last pass adds the offsets.  ~2 random accesses per node instead of
-// one per node per round.
+// L2 resident) goes through pointer jumping.  Everything a chain needs as a whole (its length, its tail, whether it is
+// a contig and where the contig goes) is then worked out over the splitter list too; one last pass over the nodes
+// writes the bases.
 __device__ __forceinline__ bool is_random_splitter(uint32_t x) { return (fmix32(x ^ 0xa5a5a5a5u) & 15u) == 0u; }
 
-__global__ void splitter_select_kernel(uint64_t n, const uint8_t* __restrict__ alive, const uint32_t* __restrict__ pred, uint32_t* __restrict__ spl_id,
-                                       uint32_t* __restrict__ spl_node, uint64_t* __restrict__ sp_ad, unsigned long long* dstat) {
-    for (uint64_t x = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; x < n; x += (uint64_t)gridDim.x * blockDim.x) {
-        uint32_t id = NONE32;
-        if ((alive[x] & 2) && (pred[x] == NONE32 || is_random_splitter((uint32_t)x))) {
-            id = (uint32_t)atomicAdd(&dstat[DS_NSPL], 1ull);
+// Splitter ids come out in no particular order (one atomic per block).  Also counts the nodes that survived both
+// filters (DS_ORIENTED), which the walks' count (DS_REACHED) is compared with.
+__global__ void __launch_bounds__(256) splitter_select_kernel(uint64_t n, const uint8_t* __restrict__ alive, const uint32_t* __restrict__ pred, uint32_t* __restrict__ spl_id,
+                                                              uint32_t* __restrict__ spl_node, uint64_t* __restrict__ sp_ad, unsigned long long* dstat) {
+    unsigned long long n_alive = 0;
+    for (uint64_t x0 = (uint64_t)blockIdx.x * blockDim.x; x0 < n; x0 += (uint64_t)gridDim.x * blockDim.x) {  // block-uniform trip count
+        const uint64_t x = x0 + threadIdx.x;
+        bool s = false;
+        if (x < n && (alive[x] & 2)) {
+            n_alive++;
+            s = is_random_splitter((uint32_t)x) || pred[x] == NONE32;
+        }
+        const uint32_t id = (uint32_t)block_reserve(s, &dstat[DS_NSPL]);
+        if (s) {
+            spl_id[x] = id;  // read by the walks only at random splitters: nothing else needs a value
             spl_node[id] = (uint32_t)x;
             sp_ad[id] = ad_pack(id, 0u);
         }
-        spl_id[x] = id;
     }
+    block_add(n_alive, &dstat[DS_ORIENTED]);
 }
-__global__ void splitter_walk_kernel(const unsigned long long* m_ptr, const uint32_t* __restrict__ spl_node, const uint32_t* __restrict__ succ,
-                                     const uint32_t* __restrict__ spl_id, uint64_t* __restrict__ loc, uint64_t* sp_ad) {
+// A splitter whose segment is the last of its chain records (tail node, segment length) in spl_tail.
+__global__ void __launch_bounds__(256) splitter_walk_kernel(const unsigned long long* m_ptr, const uint32_t* __restrict__ spl_node, const uint32_t* __restrict__ succ,
+                                                            const uint32_t* __restrict__ spl_id, uint64_t* __restrict__ loc, uint64_t* sp_ad,
+                                                            uint64_t* __restrict__ spl_tail, unsigned long long* dstat) {
     const uint64_t m = *m_ptr;  // number of splitters, still on the device: no host round trip between select and walk
+    unsigned long long stamped = 0;
     for (uint64_t id = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; id < m; id += (uint64_t)gridDim.x * blockDim.x) {
-        const uint32_t x = spl_node[id];
+        uint32_t x = spl_node[id];
         uint32_t off = 0;
         loc[x] = ad_pack((uint32_t)id, 0u);
         uint32_t y = succ[x];
@@ -541,10 +585,35 @@ __global__ void splitter_walk_kernel(const unsigned long long* m_ptr, const uint
             if (is_random_splitter(y)) { sp_ad[spl_id[y]] = ad_pack((uint32_t)id, off + 1u); break; }  // my segment ends in front of it
             off++;
             loc[y] = ad_pack((uint32_t)id, off);
+            x = y;
             y = succ[y];
         }
+        stamped += off + 1u;
+        spl_tail[id] = y == NONE32 ? ad_pack(x, off + 1u) : ~0ull;
     }
+    block_add(stamped, &dstat[DS_REACHED]);
 }
+// Per splitter, after pointer jumping: a root whose node has a predecessor means a closed path (DS_CYCLE_NODES, as
+// rank_finalize_kernel); the splitter that holds a chain's tail segment tells the chain's first splitter the chain
+// length and the tail's right flag.  Without closed paths every root is a head and has exactly one tail segment.
+__global__ void __launch_bounds__(256) splitter_fin_kernel(const unsigned long long* m_ptr, const uint64_t* sp_ad0, const uint64_t* sp_ad1,
+                                                           const uint32_t* __restrict__ spl_node, const uint32_t* __restrict__ pred,
+                                                           const uint64_t* __restrict__ spl_tail, const int32_t* __restrict__ rflag, uint64_t* spl_chain,
+                                                           unsigned long long* dstat) {
+    const uint64_t m = *m_ptr;
+    const uint64_t* sp_ad = dstat[DS_RANK_CUR] ? sp_ad1 : sp_ad0;
+    bool on_cycle = false;
+    for (uint64_t id = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; id < m; id += (uint64_t)gridDim.x * blockDim.x) {
+        const uint64_t v = sp_ad[id];
+        const uint32_t root = (uint32_t)v;
+        on_cycle |= pred[spl_node[root]] != NONE32;
+        if (root != (uint32_t)id) spl_chain[id] = 0;  // no chain starts here
+        const uint64_t t = spl_tail[id];
+        if (t != ~0ull) spl_chain[root] = ((uint64_t)(uint32_t)rflag[(uint32_t)t] << 32) | ((v >> 32) + (t >> 32));
+    }
+    if (__any_sync(0xffffffffu, on_cycle) && (threadIdx.x & 31) == 0) atomicExch(&dstat[DS_CYCLE_NODES], 1ull);
+}
+// ad[] of every node, for the cycle detection (cycle_mark_kernel): loc of a node no walk reached must read ~0
 __global__ void rank_finalize_kernel(uint64_t n, const uint8_t* __restrict__ alive, const uint32_t* __restrict__ pred, const uint64_t* __restrict__ loc,
                                      const uint64_t* sp_ad0, const uint64_t* sp_ad1, const uint32_t* __restrict__ spl_node, uint64_t* __restrict__ ad,
                                      unsigned long long* dstat) {
@@ -596,68 +665,58 @@ __global__ void cycle_cut_kernel(uint64_t n, const uint32_t* __restrict__ lab, u
     }
 }
 
-__global__ void tails_kernel(uint64_t n, const uint8_t* __restrict__ alive, const uint32_t* __restrict__ succ, const uint64_t* __restrict__ ad,
-                             uint32_t* __restrict__ chain_len, uint32_t* __restrict__ tail_of) {
-    for (uint64_t x = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; x < n; x += (uint64_t)gridDim.x * blockDim.x) {
-        if ((alive[x] & 2) && succ[x] == NONE32) {
-            const uint64_t v = ad[x];
-            const uint32_t h = (uint32_t)v;
-            chain_len[h] = (uint32_t)(v >> 32) + 1u;
-            tail_of[h] = (uint32_t)x;
-        }
-    }
-}
-
 // ---- K7: contigs ----------------------------------------------------------------------------------
+// Selection and offsets by a scan over the splitters: a chain is one entry, at its first splitter.
 struct ContigIn {
-    const uint8_t* alive;
-    const uint32_t* pred;
-    const uint32_t* chain_len;
-    const uint32_t* tail_of;
+    const uint64_t* spl_chain;
+    const uint32_t* spl_node;
     const int32_t* lflag;
-    const int32_t* rflag;
     int k, min_contig;
-    __device__ __forceinline__ U64x3 operator()(uint64_t x) const {
-        if (!(alive[x] & 2)) return U64x3{0, 0, 0};
-        if (pred[x] != NONE32) return U64x3{0, 0, 1};
-        const uint64_t len = (uint64_t)chain_len[x] + (uint64_t)k - 1;
+    __device__ __forceinline__ U64x3 operator()(uint64_t id) const {
+        const uint64_t ch = spl_chain[id];
+        if ((uint32_t)ch == 0) return U64x3{0, 0, 0};
+        const uint64_t len = (uint64_t)(uint32_t)ch + (uint64_t)k - 1;
         // DSKmerToContig, ReflexivDSMain.java:749-754
-        const bool keep = !(lflag[x] <= -10000000 && rflag[tail_of[x]] <= -10000000) && len >= (uint64_t)min_contig;
-        return keep ? U64x3{1, len, 1} : U64x3{0, 0, 1};
+        const bool keep = !(lflag[spl_node[id]] <= -10000000 && (int32_t)(ch >> 32) <= -10000000) && len >= (uint64_t)min_contig;
+        return keep ? U64x3{1, len, 0} : U64x3{0, 0, 0};
     }
 };
 struct ContigOut {
-    const uint32_t* tail_of;
+    const uint64_t* spl_chain;
+    const uint32_t* spl_node;
     const int32_t* lflag;
-    const int32_t* rflag;
     uint32_t* ctg_idx;
     uint64_t* ctg_off;
     int32_t* ctg_left;
     int32_t* ctg_right;
-    __device__ __forceinline__ void operator()(uint64_t x, U64x3 excl, U64x3 v) const {
-        ctg_idx[x] = v.a ? (uint32_t)excl.a : NONE32;
+    __device__ __forceinline__ void operator()(uint64_t id, U64x3 excl, U64x3 v) const {
+        ctg_idx[id] = v.a ? (uint32_t)excl.a : NONE32;
         if (v.a) {
             ctg_off[excl.a] = excl.b;
-            ctg_left[excl.a] = lflag[x];
-            ctg_right[excl.a] = rflag[tail_of[x]];
+            ctg_left[excl.a] = lflag[spl_node[id]];
+            ctg_right[excl.a] = (int32_t)(spl_chain[id] >> 32);
         }
     }
 };
 
+// Per node: rank = the splitter's distance from the chain's first splitter + the node's offset in the segment; the node
+// writes its last base at offset + k-1 + rank, a head also its first k-1 bases.
 template <class KT>
-__global__ void gather_contigs_kernel(Graph<KT> G, const uint8_t* __restrict__ alive, const uint64_t* __restrict__ ad,
-                                      const uint32_t* __restrict__ ctg_idx, const uint64_t* __restrict__ ctg_off, char* __restrict__ out) {
+__global__ void __launch_bounds__(256) contig_bases_kernel(Graph<KT> G, const uint8_t* __restrict__ alive, const uint64_t* __restrict__ loc,
+                                                           const uint64_t* __restrict__ sp_ad, const uint32_t* __restrict__ ctg_idx,
+                                                           const uint64_t* __restrict__ ctg_off, char* __restrict__ out) {
     const uint64_t n = 2 * G.n_rows;
     for (uint64_t x = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; x < n; x += (uint64_t)gridDim.x * blockDim.x) {
         if (!(alive[x] & 2)) continue;
-        const uint64_t v = ad[x];
-        const uint32_t h = (uint32_t)v;
-        const uint32_t ci = ctg_idx[h];
+        const uint64_t l = loc[x];
+        const uint64_t v = sp_ad[(uint32_t)l];
+        const uint32_t ci = ctg_idx[(uint32_t)v];
         if (ci == NONE32) continue;
+        const uint32_t rank = (uint32_t)(v >> 32) + (uint32_t)(l >> 32);
         const KT X = G.oriented((uint32_t)x);
         char* dst = out + ctg_off[ci];
-        dst[(uint64_t)(G.k - 1) + (uint32_t)(v >> 32)] = "ACGT"[(uint32_t)X & 3u];
-        if (h == (uint32_t)x)
+        dst[(uint64_t)(G.k - 1) + rank] = "ACGT"[(uint32_t)X & 3u];
+        if (rank == 0)
             for (int j = 0; j < G.k - 1; j++) dst[j] = "ACGT"[(uint32_t)(X >> (2 * (G.k - 1 - j))) & 3u];
     }
 }
@@ -755,22 +814,20 @@ template <class KT> static int graph_impl(Ctx* c) {
     RFX_TRY(devbuf_reserve(c, c->alive, n));
     RFX_TRY(devbuf_reserve(c, c->succ, n * sizeof(uint32_t)));
     RFX_TRY(devbuf_reserve(c, c->pred, n * sizeof(uint32_t)));
-    RFX_TRY(devbuf_reserve(c, c->tail_of, n * sizeof(uint32_t)));  // doubles as open_next until the tails pass
-    RFX_TRY(devbuf_reserve(c, c->ad[0], n * sizeof(uint64_t)));
     for (int i = 0; i < 2; i++) RFX_TRY(devbuf_reserve(c, c->sp_ad[i], n * sizeof(uint64_t)));
     RFX_TRY(devbuf_reserve(c, c->spl_id, n * sizeof(uint32_t)));
     RFX_TRY(devbuf_reserve(c, c->spl_node, n * sizeof(uint32_t)));
     RFX_TRY(devbuf_reserve(c, c->loc, n * sizeof(uint64_t)));
-    RFX_TRY(devbuf_reserve(c, c->chain_len, n * sizeof(uint32_t)));
+    RFX_TRY(devbuf_reserve(c, c->spl_tail, n * sizeof(uint64_t)));
+    RFX_TRY(devbuf_reserve(c, c->spl_chain, n * sizeof(uint64_t)));
     RFX_TRY(devbuf_reserve(c, c->ctg_idx, n * sizeof(uint32_t)));
+    RFX_TRY(devbuf_reserve(c, c->scan_ws, ScanPlan<U64x3>::workspace_elems(n) * sizeof(U64x3)));
     int rc = RFX_OK;
     do {
         if ((rc = build_index<KT>(c)) != RFX_OK) break;
         Graph<KT> G = make_graph<KT>(c);
         cudaMemsetAsync(c->succ.p, 0xff, n * sizeof(uint32_t), st);
         cudaMemsetAsync(c->pred.p, 0xff, n * sizeof(uint32_t), st);
-        cudaMemsetAsync(c->chain_len.p, 0, n * sizeof(uint32_t), st);
-        cudaMemsetAsync(c->tail_of.p, 0xff, n * sizeof(uint32_t), st);
         const int E = c->prm.min_error_coverage;
         uint8_t* alive = c->alive.as<uint8_t>();
         int32_t* lflag = c->lflag.as<int32_t>();
@@ -809,84 +866,99 @@ template <class KT> static int graph_impl(Ctx* c) {
         }
 
         // ---- K6 ----
+        // select -> walk -> jumping rounds -> per-splitter finish -> (K7) contig scan over the splitters, ONE host round
+        // trip at the end: the splitter count stays on the device, and the closed-path check, the reached-node count
+        // and the scan total come back together.
         stage_begin(c);
+        uint32_t* spl_id = c->spl_id.as<uint32_t>();
+        uint32_t* spl_node = c->spl_node.as<uint32_t>();
+        uint64_t* loc = c->loc.as<uint64_t>();
+        uint64_t* spl_tail = c->spl_tail.as<uint64_t>();
+        uint64_t* spl_chain = c->spl_chain.as<uint64_t>();
+        const unsigned long long* m_ptr = dstat + DS_NSPL;
+        ScanPlan<U64x3> plan;
+        plan.bind(n, c->scan_ws.as<U64x3>());  // at most n splitters
+        plan.live = m_ptr;
+        const ContigIn in{spl_chain, spl_node, lflag, c->k, c->prm.min_contig};
+        U64x3 tot{0, 0, 0};
         int limit = 2;
         while ((1ull << limit) < n + 1) limit++;
         limit += 2;
-        int cur = 0;
-        for (int attempt = 0; attempt < 2; attempt++) {
-            cur = 0;
-            {
-                uint32_t* spl_id = c->spl_id.as<uint32_t>();
-                uint32_t* spl_node = c->spl_node.as<uint32_t>();
-                uint64_t* loc = c->loc.as<uint64_t>();
-                cudaMemsetAsync(dstat + DS_NSPL, 0, sizeof(uint64_t), st);
-                cudaMemsetAsync(loc, 0xff, n * sizeof(uint64_t), st);
-                splitter_select_kernel<<<grid_n(n), 256, 0, st>>>(n, alive, pred, spl_id, spl_node, c->sp_ad[0].as<uint64_t>(), dstat);
-                // select -> walk -> jumping rounds -> finalize; the splitter count stays on the device
-                splitter_walk_kernel<<<sm_count() * 16, 256, 0, st>>>(dstat + DS_NSPL, spl_node, succ, spl_id, loc, c->sp_ad[0].as<uint64_t>());
-                cudaMemsetAsync(dstat + DS_RANK_FLAGS, 0, 3 * sizeof(uint64_t), st);
-                cudaMemsetAsync(dstat + DS_RANK_CUR, 0, sizeof(uint64_t), st);
-                if (n <= (16ull << 20) && !c->arena) {  // (a rank of a sharded run may share its device with a peer that waits in a barrier: no co-resident grid)
-                    // up to ~10^6 splitters: every round in one cooperative launch, no host round trip at all
-                    const unsigned long long* m_ptr = dstat + DS_NSPL;
-                    uint64_t* a0 = c->sp_ad[0].as<uint64_t>();
-                    uint64_t* a1 = c->sp_ad[1].as<uint64_t>();
-                    unsigned long long* ds = dstat;
-                    void* args[] = {(void*)&m_ptr, (void*)&a0, (void*)&a1, (void*)&ds};
-                    e = cudaLaunchCooperativeKernel((void*)rank_all_kernel, dim3(sm_count() * 4), dim3(256), args, 0, st);
-                    if (e != cudaSuccess) break;
-                } else {
-                    // long lists: one launch per round over as many threads as entries (the co-resident grid of the
-                    // cooperative kernel has too few loads in flight); the host looks at the "changed" flag every 4 rounds
-                    uint64_t m = 0;
-                    cudaMemcpyAsync(&m, dstat + DS_NSPL, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
-                    e = cudaStreamSynchronize(st);
-                    if (e != cudaSuccess) break;
-                    int scur = 0;
-                    if (m) {
-                        int slimit = 2;
-                        while ((1ull << slimit) < m + 1) slimit++;
-                        slimit += 2;
-                        for (int round = 0; round < slimit;) {
-                            cudaMemsetAsync(dstat + DS_CHANGED, 0, sizeof(uint64_t), st);
-                            for (int q = 0; q < 4 && round < slimit; q++, round++) {
-                                rank_step_kernel<<<grid_n(m), 256, 0, st>>>(m, c->sp_ad[scur].as<uint64_t>(), c->sp_ad[scur ^ 1].as<uint64_t>(), dstat);
-                                c->launches++;
-                                scur ^= 1;
-                            }
-                            uint64_t changed = 0;
-                            cudaMemcpyAsync(&changed, dstat + DS_CHANGED, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
-                            e = cudaStreamSynchronize(st);
-                            if (e != cudaSuccess) break;
-                            if (!changed) break;
-                        }
-                        if (e != cudaSuccess) break;
-                    }
-                    set_value_kernel<<<1, 1, 0, st>>>(dstat + DS_RANK_CUR, (unsigned long long)scur);
-                }
-                cudaMemsetAsync(dstat + DS_CYCLE_NODES, 0, sizeof(uint64_t), st);
-                rank_finalize_kernel<<<grid_n(n), 256, 0, st>>>(n, alive, pred, loc, c->sp_ad[0].as<uint64_t>(), c->sp_ad[1].as<uint64_t>(), spl_node, c->ad[0].as<uint64_t>(), dstat);
+        for (int attempt = 0;; attempt++) {
+            splitter_select_kernel<<<grid_n(n), 256, 0, st>>>(n, alive, pred, spl_id, spl_node, c->sp_ad[0].as<uint64_t>(), dstat);
+            splitter_walk_kernel<<<sm_count() * 16, 256, 0, st>>>(m_ptr, spl_node, succ, spl_id, loc, c->sp_ad[0].as<uint64_t>(), spl_tail, dstat);
+            cudaMemsetAsync(dstat + DS_RANK_FLAGS, 0, 3 * sizeof(uint64_t), st);
+            cudaMemsetAsync(dstat + DS_RANK_CUR, 0, sizeof(uint64_t), st);
+            c->launches += 2;
+            if (n <= (16ull << 20) && !c->arena) {  // (a rank of a sharded run may share its device with a peer that waits in a barrier: no co-resident grid)
+                // up to ~10^6 splitters: every round in one cooperative launch, no host round trip at all
+                uint64_t* a0 = c->sp_ad[0].as<uint64_t>();
+                uint64_t* a1 = c->sp_ad[1].as<uint64_t>();
+                unsigned long long* ds = dstat;
+                void* args[] = {(void*)&m_ptr, (void*)&a0, (void*)&a1, (void*)&ds};
+                e = cudaLaunchCooperativeKernel((void*)rank_all_kernel, dim3(sm_count() * 4), dim3(256), args, 0, st);
+                if (e != cudaSuccess) break;
                 c->launches++;
-                c->launches += 3;
-                uint64_t any_cycle = 0;
-                cudaMemcpyAsync(&any_cycle, dstat + DS_CYCLE_NODES, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+            } else {
+                // long lists: one launch per round over as many threads as entries (the co-resident grid of the
+                // cooperative kernel has too few loads in flight); the host looks at the "changed" flag every 4 rounds
+                uint64_t m = 0;
+                cudaMemcpyAsync(&m, m_ptr, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
                 e = cudaStreamSynchronize(st);
-                if (e != cudaSuccess || !any_cycle) break;
+                if (e != cudaSuccess) break;
+                int scur = 0;
+                if (m) {
+                    int slimit = 2;
+                    while ((1ull << slimit) < m + 1) slimit++;
+                    slimit += 2;
+                    for (int round = 0; round < slimit;) {
+                        cudaMemsetAsync(dstat + DS_CHANGED, 0, sizeof(uint64_t), st);
+                        for (int q = 0; q < 4 && round < slimit; q++, round++) {
+                            rank_step_kernel<<<grid_n(m), 256, 0, st>>>(m, c->sp_ad[scur].as<uint64_t>(), c->sp_ad[scur ^ 1].as<uint64_t>(), dstat);
+                            c->launches++;
+                            scur ^= 1;
+                        }
+                        uint64_t changed = 0;
+                        cudaMemcpyAsync(&changed, dstat + DS_CHANGED, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
+                        e = cudaStreamSynchronize(st);
+                        if (e != cudaSuccess) break;
+                        if (!changed) break;
+                    }
+                    if (e != cudaSuccess) break;
+                }
+                set_value_kernel<<<1, 1, 0, st>>>(dstat + DS_RANK_CUR, (unsigned long long)scur);
+                c->launches++;
             }
-            if (attempt == 1) break;
-            // cycles: every junction of a closed path joins, no node is a head
-            RFX_TRY(devbuf_reserve(c, c->cmin[0], 2 * n * sizeof(uint32_t)));
-            RFX_TRY(devbuf_reserve(c, c->cmin[1], 2 * n * sizeof(uint32_t)));
+            splitter_fin_kernel<<<grid_n(n), 256, 0, st>>>(m_ptr, c->sp_ad[0].as<uint64_t>(), c->sp_ad[1].as<uint64_t>(), spl_node, pred, spl_tail, rflag, spl_chain, dstat);
+            cudaEventRecord(c->ev1, st);  // K6 ends here unless a closed path turns up
+            scan_prepare(plan, in, OpAddU64x3{}, U64x3{0, 0, 0}, st);
+            c->launches += 1 + 2 * plan.levels;
+            cudaMemcpyAsync(&tot, plan.total, sizeof(tot), cudaMemcpyDeviceToHost, st);
+            cudaMemcpyAsync(h, c->dstat.p, sizeof(h), cudaMemcpyDeviceToHost, st);
+            e = cudaStreamSynchronize(st);
+            if (e != cudaSuccess) break;
+            if (!h[DS_CYCLE_NODES] && h[DS_REACHED] == h[DS_ORIENTED]) break;
+            if (attempt == 1) { rc = ctx_fail(c, RFX_E_GRAPH, "a closed path survived its cut"); break; }
+            // cycles: every junction of a closed path joins, no node is a head.  ad[] of every node, with ~0 in loc for the
+            // nodes on closed paths that no walk reached: walk again over a cleared loc (its splitter-list writes go to the
+            // buffer that pointer jumping left unused)
+            const int cur = (int)h[DS_RANK_CUR];
+            if ((rc = devbuf_reserve(c, c->ad[0], n * sizeof(uint64_t))) != RFX_OK) break;
+            if ((rc = devbuf_reserve(c, c->cmin[0], 2 * n * sizeof(uint32_t))) != RFX_OK) break;
+            if ((rc = devbuf_reserve(c, c->cmin[1], 2 * n * sizeof(uint32_t))) != RFX_OK) break;
+            cudaMemsetAsync(loc, 0xff, n * sizeof(uint64_t), st);
+            splitter_walk_kernel<<<sm_count() * 16, 256, 0, st>>>(m_ptr, spl_node, succ, spl_id, loc, c->sp_ad[cur ^ 1].as<uint64_t>(), spl_tail, dstat);
+            rank_finalize_kernel<<<grid_n(n), 256, 0, st>>>(n, alive, pred, loc, c->sp_ad[0].as<uint64_t>(), c->sp_ad[1].as<uint64_t>(), spl_node, c->ad[0].as<uint64_t>(), dstat);
             uint32_t* lab[2] = {c->cmin[0].as<uint32_t>(), c->cmin[1].as<uint32_t>()};
             uint32_t* ptr[2] = {lab[0] + n, lab[1] + n};
             cudaMemsetAsync(dstat + DS_CYCLE_NODES, 0, sizeof(uint64_t), st);
-            cycle_mark_kernel<<<grid_n(n), 256, 0, st>>>(n, alive, pred, c->ad[cur].as<uint64_t>(), lab[0], ptr[0], dstat);
-            c->launches++;
+            cycle_mark_kernel<<<grid_n(n), 256, 0, st>>>(n, alive, pred, c->ad[0].as<uint64_t>(), lab[0], ptr[0], dstat);
+            c->launches += 3;
             uint64_t cyc_nodes = 0;
             cudaMemcpyAsync(&cyc_nodes, dstat + DS_CYCLE_NODES, sizeof(uint64_t), cudaMemcpyDeviceToHost, st);
             e = cudaStreamSynchronize(st);
-            if (e != cudaSuccess || cyc_nodes == 0) break;
+            if (e != cudaSuccess) break;
+            if (cyc_nodes == 0) { rc = ctx_fail(c, RFX_E_GRAPH, "chain ranking saw a closed path that cycle detection did not find"); break; }
             int b = 0;
             for (int round = 0; round < limit; round++) {
                 cycle_min_step_kernel<KT><<<grid_n(n), 256, 0, st>>>(G, lab[b], ptr[b], lab[b ^ 1], ptr[b ^ 1]);
@@ -895,44 +967,35 @@ template <class KT> static int graph_impl(Ctx* c) {
             }
             cycle_cut_kernel<<<grid_n(n), 256, 0, st>>>(n, lab[b], succ, pred, dstat);
             c->launches++;
+            // the second attempt counts afresh
+            const int fresh[] = {DS_NSPL, DS_ORIENTED, DS_REACHED, DS_CYCLE_NODES};
+            for (int slot : fresh) cudaMemsetAsync(dstat + slot, 0, sizeof(uint64_t), st);
         }
+        if (rc != RFX_OK) break;
         if (e != cudaSuccess) { rc = ctx_fail(c, RFX_E_CUDA, "list ranking failed: %s", cudaGetErrorString(e)); break; }
-        const uint64_t* ad = c->ad[cur].as<uint64_t>();
-        tails_kernel<<<grid_n(n), 256, 0, st>>>(n, alive, succ, ad, c->chain_len.as<uint32_t>(), c->tail_of.as<uint32_t>());
-        c->launches += 1;
-        e = cudaStreamSynchronize(st);
-        if (e != cudaSuccess) { rc = ctx_fail(c, RFX_E_CUDA, "chain kernels failed: %s", cudaGetErrorString(e)); break; }
-        c->ms[4] += stage_end(c);
+        // the event at the end of K6 has completed: K7 is timed from there
+        float ms_k6 = 0;
+        cudaEventElapsedTime(&ms_k6, c->ev0, c->ev1);
+        c->ms[4] += ms_k6;
+        std::swap(c->ev0, c->ev1);
 
         // ---- K7 ----
-        stage_begin(c);
-        ScanPlan<U64x3> plan;
-        if ((rc = devbuf_reserve(c, c->scan_ws, ScanPlan<U64x3>::workspace_elems(n) * sizeof(U64x3))) != RFX_OK) break;
-        plan.bind(n, c->scan_ws.as<U64x3>());
-        ContigIn in{alive, pred, c->chain_len.as<uint32_t>(), c->tail_of.as<uint32_t>(), lflag, rflag, c->k, c->prm.min_contig};
-        scan_prepare(plan, in, OpAddU64x3{}, U64x3{0, 0, 0}, st);
-        c->launches += 2 * plan.levels;
-        U64x3 tot;
-        cudaMemcpyAsync(&tot, plan.total, sizeof(tot), cudaMemcpyDeviceToHost, st);
-        cudaMemcpyAsync(h, c->dstat.p, sizeof(h), cudaMemcpyDeviceToHost, st);
-        e = cudaStreamSynchronize(st);
-        if (e != cudaSuccess) { rc = ctx_fail(c, RFX_E_CUDA, "contig scan failed: %s", cudaGetErrorString(e)); break; }
         if ((rc = devbuf_reserve(c, c->ctg_off, (tot.a + 1) * sizeof(uint64_t))) != RFX_OK) break;
         if ((rc = devbuf_reserve(c, c->ctg_left, (tot.a + 1) * sizeof(int32_t))) != RFX_OK) break;
         if ((rc = devbuf_reserve(c, c->ctg_right, (tot.a + 1) * sizeof(int32_t))) != RFX_OK) break;
         if ((rc = devbuf_reserve(c, c->ctg_bases, tot.b + 16)) != RFX_OK) break;
-        ContigOut out{c->tail_of.as<uint32_t>(), lflag, rflag, c->ctg_idx.as<uint32_t>(), c->ctg_off.as<uint64_t>(), c->ctg_left.as<int32_t>(),
-                      c->ctg_right.as<int32_t>()};
+        const ContigOut out{spl_chain, spl_node, lflag, c->ctg_idx.as<uint32_t>(), c->ctg_off.as<uint64_t>(), c->ctg_left.as<int32_t>(), c->ctg_right.as<int32_t>()};
         scan_apply(plan, in, out, OpAddU64x3{}, U64x3{0, 0, 0}, st);
         set_u64_kernel<<<1, 1, 0, st>>>(c->ctg_off.as<uint64_t>() + tot.a, plan.total);
-        gather_contigs_kernel<KT><<<grid_n(n), 256, 0, st>>>(G, alive, ad, c->ctg_idx.as<uint32_t>(), c->ctg_off.as<uint64_t>(), c->ctg_bases.as<char>());
+        contig_bases_kernel<KT><<<grid_n(n), 256, 0, st>>>(G, alive, loc, c->sp_ad[h[DS_RANK_CUR]].as<uint64_t>(), c->ctg_idx.as<uint32_t>(), c->ctg_off.as<uint64_t>(),
+                                                          c->ctg_bases.as<char>());
         c->launches += 3;
         e = cudaStreamSynchronize(st);
         if (e != cudaSuccess) { rc = ctx_fail(c, RFX_E_CUDA, "contig gather failed: %s", cudaGetErrorString(e)); break; }
         c->ms[5] += stage_end(c);
         c->n_contigs = tot.a;
         c->n_contig_bases = tot.b;
-        c->n_oriented = tot.c;
+        c->n_oriented = h[DS_ORIENTED];
         c->n_budget_adm = h[DS_ABSORBED];
         c->n_cycles = h[DS_CYCLES];
         c->have_contigs = true;

@@ -146,14 +146,15 @@ struct Ctx {
     DevBuf alive;         // u8[2*n_rows]  bit0: survives right filter, bit1: survives both
     DevBuf succ, pred;    // u32[2*n_rows]
     DevBuf ad[2];         // u64[2*n_rows] packed (ancestor, distance) for pointer jumping, double buffered
-    DevBuf spl_id;        // u32[2*n_rows] splitter index of a node, NONE if it is not a splitter
+    DevBuf spl_id;        // u32[2*n_rows] splitter index of a node (NONE where it is not one: sharded runs only write that)
     DevBuf spl_node;      // u32[2*n_rows] node of a splitter
     DevBuf loc;           // u64[2*n_rows] (owning splitter, offset from it)
     DevBuf sp_ad[2];      // u64[2*n_rows] packed (ancestor, distance) over the splitter list
     DevBuf cmin[2];
-    DevBuf chain_len;     // u32[2*n_rows] at heads
-    DevBuf tail_of;       // u32[2*n_rows] at heads
-    DevBuf ctg_idx;       // u32[2*n_rows] at heads: contig index or NONE
+    DevBuf spl_tail;      // u64[2*n_rows] per splitter: (last node, nodes) of a segment that ends its chain, ~0 for the others
+    DevBuf spl_chain;     // u64[2*n_rows] per splitter: (right flag of the tail, chain length) at a chain's first splitter, 0 elsewhere
+    DevBuf chain_len;     // u32[2*n_rows] at heads (sharded chain ranking)
+    DevBuf ctg_idx;       // u32[2*n_rows] contig index or NONE: per splitter on one GPU, at heads in a sharded run
     DevBuf ctg_off;       // u64[n_contigs + 1]
     DevBuf ctg_left, ctg_right;  // i32[n_contigs]
     DevBuf ctg_bases;     // char[total]
@@ -243,6 +244,7 @@ enum {
     DS_FQ_IRREGULAR = 40, //   position (mod 4) of the sequence lines, lineMark behind the chunk if the layout is regular
     DS_FQ_SEQPOS = 41,
     DS_FQ_NEXT = 42,
+    DS_REACHED = 43,      // nodes the splitter walks stamped: all alive nodes unless some sit on a closed path without a splitter
     DS_NSLOTS = 48
 };
 

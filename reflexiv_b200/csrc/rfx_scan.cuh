@@ -54,9 +54,15 @@ template <class T, class Op> __device__ __forceinline__ T warp_scan_incl(T v, Op
     return v;
 }
 
-// Phase A: agg[block] = fold of the block's tile
+// Phase A: agg[block] = fold of the block's tile.  live (optional): the element count as the device knows it, n is then
+// an upper bound and the tiles behind it are empty.
 template <class T, class Op, class In>
-__global__ void __launch_bounds__(SCAN_WARPS * 32) scan_agg_kernel(uint64_t n, In in, Op op, T ident, T* __restrict__ agg) {
+__global__ void __launch_bounds__(SCAN_WARPS * 32) scan_agg_kernel(uint64_t n, const unsigned long long* live, In in, Op op, T ident, T* __restrict__ agg) {
+    if (live && *live < n) n = *live;
+    if ((uint64_t)blockIdx.x * SCAN_TILE >= n) {
+        if (threadIdx.x == 0) agg[blockIdx.x] = ident;
+        return;
+    }
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint64_t base = (uint64_t)blockIdx.x * SCAN_TILE + (uint64_t)warp * 32 * SCAN_ITEMS;
     T acc = ident;
@@ -80,7 +86,9 @@ __global__ void __launch_bounds__(SCAN_WARPS * 32) scan_agg_kernel(uint64_t n, I
 // Phase C: out(i, exclusive prefix, value)
 template <class T, class Op, class In, class Out>
 __global__ void __launch_bounds__(SCAN_WARPS * 32)
-    scan_apply_kernel(uint64_t n, In in, Out out, Op op, T ident, const T* __restrict__ tile_prefix) {
+    scan_apply_kernel(uint64_t n, const unsigned long long* live, In in, Out out, Op op, T ident, const T* __restrict__ tile_prefix) {
+    if (live && *live < n) n = *live;
+    if ((uint64_t)blockIdx.x * SCAN_TILE >= n) return;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint64_t base = (uint64_t)blockIdx.x * SCAN_TILE + (uint64_t)warp * 32 * SCAN_ITEMS;
     T v[SCAN_ITEMS], s[SCAN_ITEMS];
@@ -123,6 +131,8 @@ template <class T> struct ScanPlan {
     uint64_t count[6] = {0};
     T* agg[6] = {nullptr};
     T* total = nullptr;  // device, 1 element
+    // element count on the device, when the host does not know it yet: n (from bind) is then an upper bound
+    const unsigned long long* live = nullptr;
     static size_t workspace_elems(uint64_t n) {
         size_t tot = 1;
         uint64_t c = n;
@@ -130,7 +140,7 @@ template <class T> struct ScanPlan {
         return tot + 8;
     }
     void bind(uint64_t n_, T* ws) {
-        n = n_; levels = 0;
+        n = n_; levels = 0; live = nullptr;
         uint64_t c = n;
         T* p = ws;
         total = p; p += 1;
@@ -148,10 +158,10 @@ template <class T> __global__ void scan_copy_total_kernel(const T* src, T* dst) 
 template <class T, class Op, class In>
 void scan_prepare(ScanPlan<T>& plan, In in, Op op, T ident, cudaStream_t st) {
     if (plan.n == 0) { cudaMemsetAsync(plan.total, 0, sizeof(T), st); return; }
-    scan_agg_kernel<T, Op, In><<<(unsigned)plan.count[0], SCAN_WARPS * 32, 0, st>>>(plan.n, in, op, ident, plan.agg[0]);
+    scan_agg_kernel<T, Op, In><<<(unsigned)plan.count[0], SCAN_WARPS * 32, 0, st>>>(plan.n, plan.live, in, op, ident, plan.agg[0]);
     for (int l = 1; l < plan.levels; l++) {
         ScanInArray<T> src{plan.agg[l - 1]};
-        scan_agg_kernel<T, Op, ScanInArray<T>><<<(unsigned)plan.count[l], SCAN_WARPS * 32, 0, st>>>(plan.count[l - 1], src, op, ident, plan.agg[l]);
+        scan_agg_kernel<T, Op, ScanInArray<T>><<<(unsigned)plan.count[l], SCAN_WARPS * 32, 0, st>>>(plan.count[l - 1], nullptr, src, op, ident, plan.agg[l]);
     }
     // top level has exactly one aggregate = the grand total
     scan_copy_total_kernel<T><<<1, 1, 0, st>>>(plan.agg[plan.levels - 1], plan.total);
@@ -161,7 +171,7 @@ void scan_prepare(ScanPlan<T>& plan, In in, Op op, T ident, cudaStream_t st) {
         ScanOutArray<T> dst{plan.agg[l - 1]};
         const T* pre = (l == plan.levels - 1) ? nullptr : plan.agg[l];
         scan_apply_kernel<T, Op, ScanInArray<T>, ScanOutArray<T>>
-            <<<(unsigned)plan.count[l], SCAN_WARPS * 32, 0, st>>>(plan.count[l - 1], src, dst, op, ident, pre);
+            <<<(unsigned)plan.count[l], SCAN_WARPS * 32, 0, st>>>(plan.count[l - 1], nullptr, src, dst, op, ident, pre);
     }
 }
 
@@ -172,7 +182,7 @@ void scan_apply(ScanPlan<T>& plan, In in, Out out, Op op, T ident, cudaStream_t 
     const T* pre = plan.levels == 1 ? nullptr : plan.agg[0];
     // with a single level there is one tile and its prefix is the identity
     if (plan.levels >= 1 && plan.count[0] > 1) pre = plan.agg[0];
-    scan_apply_kernel<T, Op, In, Out><<<(unsigned)plan.count[0], SCAN_WARPS * 32, 0, st>>>(plan.n, in, out, op, ident, pre);
+    scan_apply_kernel<T, Op, In, Out><<<(unsigned)plan.count[0], SCAN_WARPS * 32, 0, st>>>(plan.n, plan.live, in, out, op, ident, pre);
 }
 
 }  // namespace rfx

@@ -210,23 +210,6 @@ struct SGWork {
     unsigned long long* counter;  // entries in the list (device)
 };
 template <int PASS> __device__ __forceinline__ uint64_t sg_work_count(uint64_t n, const SGWork& W) { return PASS == 1 ? n : (uint64_t)*W.counter; }
-// Index of a new entry for every thread that wants one, ~0 for the others: ONE global atomic per block and call (a quarter
-// of a million warps bumping the same counter cost more than the kernel around them).  Every thread of the block must call.
-__device__ __forceinline__ unsigned long long sg_block_reserve(bool want, unsigned long long* counter) {
-    __shared__ uint32_t s_count;
-    __shared__ unsigned long long s_base;
-    const uint32_t lane = threadIdx.x & 31u;
-    if (threadIdx.x == 0) s_count = 0;
-    __syncthreads();
-    const uint32_t m = __ballot_sync(0xffffffffu, want);
-    uint32_t wbase = 0;
-    if (lane == 0 && m) wbase = atomicAdd(&s_count, (uint32_t)__popc(m));
-    wbase = __shfl_sync(0xffffffffu, wbase, 0);
-    __syncthreads();
-    if (threadIdx.x == 0 && s_count) s_base = atomicAdd(counter, (unsigned long long)s_count);
-    __syncthreads();
-    return want ? s_base + wbase + __popc(m & ((1u << lane) - 1u)) : ~0ull;
-}
 // End of a pass-1 iteration, called by every thread of the block: the marked candidates become requests (positions in the
 // channels reserved per block: one global atomic per owner and block, the lanes rank themselves in shared memory) and the
 // nodes that wait go onto the work list with the places of their answers.  zfun(b) rebuilds candidate b of this thread's node.
@@ -622,9 +605,9 @@ __global__ void sg_select_kernel(const __grid_constant__ SGView V, uint64_t n, u
             p = Me.pred[x];
             s1 = p == NONE32 || gid_rank(p) != V.me || sg_l1_sample((uint32_t)x);
         }
-        const uint32_t id = (uint32_t)sg_block_reserve(s1, &dstat[DS_NSPL]);
+        const uint32_t id = (uint32_t)block_reserve(s1, &dstat[DS_NSPL]);
         const bool s2 = s1 && (p == NONE32 || sg_l2_sample(gid_make(V.me, id)));
-        const uint32_t j = (uint32_t)sg_block_reserve(s2, &dstat[DS_NL2]);
+        const uint32_t j = (uint32_t)block_reserve(s2, &dstat[DS_NL2]);
         if (s1) {
             spl_node[id] = (uint32_t)x;
             if (s2) {
