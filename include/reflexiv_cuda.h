@@ -186,7 +186,9 @@ int rfx_sorted_csv(rfx_ctx* ctx, char* out, uint64_t cap, uint64_t* n_bytes);
  * rfx_stitch_finish keeps one fragment per contig end, joins contig + fragment + contig chains and REPLACES the contigs
  * that rfx_contigs_size / rfx_contigs_copy return.  rfx_reset, rfx_count, rfx_load_counts*, rfx_assemble and rfx_sort_kmers
  * abandon an open stage (its fragments refer to the contigs it was opened on).  The order-dependent choices of the reference (probe collisions, which
- * fragment of a run stays, rings) are fixed as DESIGN.md section 2 lists them. */
+ * fragment of a run stays, rings) are fixed as DESIGN.md section 2 lists them.  On a sharded context (rfx_shard_init)
+ * rfx_stitch_begin returns RFX_E_UNSUPPORTED: there the stage is rfx_stitch_begin_sharded / rfx_stitch_finish_sharded
+ * (multi-GPU block below). */
 typedef struct {
     uint64_t n_probes;      /* keys in the probe table */
     uint64_t n_reads;       /* sequence lines scanned */
@@ -246,7 +248,8 @@ int rfx_load_counts_device(rfx_ctx* ctx, const void* d_keys, const uint32_t* d_c
  * then read and write peer HBM directly: no collective library on the data path.
  *   every rank:  rfx_shard_init -> rfx_shard_export -> [caller gathers the world * RFX_SHARD_HANDLE_BYTES bytes] ->
  *                rfx_shard_connect -> { rfx_reset, rfx_push_fastq*, rfx_count_sharded, rfx_assemble_sharded, results }*
- * rfx_count_sharded, rfx_shard_table, rfx_assemble_sharded and rfx_sort_kmers_sharded are collective: every rank must call
+ * rfx_count_sharded, rfx_shard_table, rfx_assemble_sharded, rfx_sort_kmers_sharded, rfx_stitch_begin_sharded and
+ * rfx_stitch_finish_sharded are collective: every rank must call
  * them (from its own host thread or process); they meet in cross-GPU barriers and fail with RFX_E_STATE if a peer never
  * arrives.  A collective call either succeeds on every rank or fails on every rank at once, with the code of the
  * lowest-numbered rank that failed (that rank keeps its own message, the others name it), and the contexts stay usable for
@@ -316,6 +319,32 @@ int rfx_assemble_sharded(rfx_ctx* ctx);
  * RFX_E_CAPACITY.  rfx_stats: ms_graph is the call's time;
  * rfx_shard_stats: ms_comm and n_remote_probes cover the call. */
 int rfx_sort_kmers_sharded(rfx_ctx* ctx, int32_t min_error_coverage, double min_repeat_fold, int32_t max_kmer_size);
+/* Collective -stitch on a table sharded by minimiser bin: rfx_stitch_begin / rfx_stitch_finish across ranks.
+ *   every rank:  ... rfx_shard_connect -> { rfx_reset, rfx_load_counts* (any slice) -> rfx_shard_table | rfx_push_fastq* ->
+ *                rfx_count_sharded, rfx_stitch_begin_sharded, rfx_push_fastq* / rfx_push_fastq_device* / rfx_push_reads* (this
+ *                rank's reads, any split on record boundaries, possibly none), rfx_stitch_finish_sharded, results }*
+ * The begin and the finish are collective; the pushes between them are not: every rank scans what it was given.  Begin runs
+ * the sharded assembly (every record kept, as rfx_stitch_begin) and builds on every rank the same probe table over global
+ * contig ids (the ranks' contigs in rank order) from a small per-contig summary every rank pulls from every other; finish
+ * pulls every rank's fragments, joins the chains over all contigs and leaves on every rank the stitched records whose head
+ * contig it owns (the rank that held that contig after the assembly; rfx_contigs_* work on them).  The union over the ranks
+ * equals, as a multiset of (sequence, left, right), what rfx_stitch_begin / rfx_stitch_finish give on one context with the
+ * whole table and all the reads, for every split of rows and reads.  k > 31: no probe (as on one context), the result is
+ * the sharded assembly with the -mincontig rule applied.
+ * rfx_stitch_stats per rank: n_reads and n_fragments of this rank's own reads; n_stitched and n_rings over the heads it owns
+ * (heads the -mincontig rule drops included: summed over the ranks they are the one-context values); n_probes,
+ * n_after_pass1 and n_joined global, the same on every rank.  rfx_shard_stats after finish: n_contigs_global and
+ * n_contig_bases_global describe the stitched set; ms_comm covers the call.
+ * Failures follow the rule of the other collective calls.  RFX_E_STATE: a context without an arena, a rank without a table
+ * sharded by minimiser bin, finish with no sharded stage open on some rank, rfx_stitch_finish on a sharded stage (the stage
+ * stays open) and rfx_stitch_finish_sharded on a one-context stage.  RFX_E_INVALID: k or min_contig differing between ranks
+ * (checked before the assembly).  RFX_E_CAPACITY: more than 2^31 - 1 contigs over all ranks, or 2^32 - 1 fragments or more.
+ * RFX_E_NOMEM: an arena too small.  rfx_reset, rfx_count_sharded, rfx_load_counts*, rfx_shard_table, rfx_assemble_sharded
+ * and rfx_sort_kmers_sharded abandon an open stage.
+ * Arena need, besides the sharded assembly: about 160 bytes per contig of ALL ranks (the replicated summary, probe table
+ * and chain links), plus 24 bytes and one byte per base for every fragment of ALL ranks, plus this rank's stitched records. */
+int rfx_stitch_begin_sharded(rfx_ctx* ctx);
+int rfx_stitch_finish_sharded(rfx_ctx* ctx);
 int rfx_shard_stats(rfx_ctx* ctx, rfx_shard_stats_t* out);
 
 /* number of CUDA devices the library can use (a launcher maps ranks to devices with it) */

@@ -106,6 +106,8 @@ SYMBOLS = {
     "rfx_shard_table": (C.c_int, [_P]),
     "rfx_assemble_sharded": (C.c_int, [_P]),
     "rfx_sort_kmers_sharded": (C.c_int, [_P, C.c_int32, C.c_double, C.c_int32]),
+    "rfx_stitch_begin_sharded": (C.c_int, [_P]),
+    "rfx_stitch_finish_sharded": (C.c_int, [_P]),
     "rfx_shard_stats": (C.c_int, [_P, C.POINTER(RfxShardStats)]),
     "rfx_device_count": (C.c_int, [C.POINTER(C.c_int32)]),
 }

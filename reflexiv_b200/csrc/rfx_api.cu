@@ -85,7 +85,8 @@ void free_all_buffers(Ctx* c) {
                      &c->ad[1], &c->rd_src, &c->spl_id, &c->spl_node, &c->loc, &c->sp_ad[0], &c->sp_ad[1], &c->cmin[0], &c->cmin[1], &c->spl_tail, &c->spl_chain, &c->chain_len, &c->ctg_idx, &c->ctg_off,
                      &c->ctg_left, &c->ctg_right, &c->ctg_bases, &c->rx_records, &c->run_desc, &c->rd_runs, &c->seg_off, &c->seg_base, &c->ovf_rec, &c->ovf_bin, &c->g_rowbin, &c->g_binrows, &c->g_hoff, &c->g_bloom, &c->srt_left, &c->srt_right, &c->eff_l, &c->eff_r, &c->seg_ext,
                      &c->st_keys, &c->st_vals, &c->st_bloom, &c->st_firstk, &c->st_ctr, &c->st_len, &c->st_woff, &c->st_hits, &c->st_frags, &c->st_codes, &c->st_nxt, &c->st_prv,
-                     &c->st_role, &c->st_outlen, &c->st_outright, &c->st_slot, &c->sh_send};
+                     &c->st_role, &c->st_outlen, &c->st_outright, &c->st_slot, &c->st_lfirstk, &c->st_lends, &c->st_goff, &c->st_gends, &c->st_gleft,
+                     &c->st_gright, &c->st_gfrags, &c->st_gcodes, &c->sh_send};
     for (DevBuf* b : all) devbuf_free(*b);
 }
 

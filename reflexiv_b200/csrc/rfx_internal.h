@@ -179,6 +179,17 @@ struct Ctx {
     uint64_t st_cap = 0, st_nfrag = 0, st_ncodes = 0, st_reads = 0;
     uint64_t st_stat[6] = {0, 0, 0, 0, 0, 0};  // probes, fragments, after pass 1, joined on both sides, stitched records, rings
     float ms_stitch = 0;
+    // ... across ranks (rfx_stitch_begin_sharded): contig ids are global (the ranks' contigs in rank order); st_firstk and the
+    // arrays below describe ALL contigs, pulled from every rank's summary
+    bool st_sharded = false;     // the open stage is the sharded one
+    DevBuf st_lfirstk, st_lends; // u64[own contigs], u64[2 * own contigs]: this rank's summary (first k-mer, first / last (k-1)-mer)
+    DevBuf st_goff;              // u64[N + 1] global contig offsets (the ranks' contig bases laid end to end)
+    DevBuf st_gends;             // u64[2N]
+    DevBuf st_gleft, st_gright;  // i32[N]
+    DevBuf st_gfrags, st_gcodes; // every rank's fragments and codes, in rank order (rfx_stitch_finish_sharded)
+    uint64_t st_ctg_lo[RFX_MAX_RANKS + 1] = {0};   // global ids of rank r: [st_ctg_lo[r], st_ctg_lo[r + 1])
+    uint64_t st_base_lo[RFX_MAX_RANKS + 1] = {0};  // ... their bases in the global offsets
+    uint64_t st_bases_at[RFX_MAX_RANKS] = {0};     // arena offset of every rank's contig bases
 
     // ---- sharded runs over peer memory (rfx_shard.cu): one context per GPU, every device buffer of the context lives in
     // ONE cudaMalloc'ed arena that the other ranks map (CUDA IPC between processes, plain pointers inside a process) ----
@@ -280,6 +291,8 @@ int stage_sorted(Ctx* c, int min_error_coverage, double min_repeat_fold, int max
 int stage_stitch_begin(Ctx* c);
 int stitch_scan_reads(Ctx* c, const uint8_t* d_text, const uint64_t* rd_src, const uint32_t* rd_len, uint64_t n_reads);
 int stage_stitch_finish(Ctx* c);
+int stage_stitch_begin_sharded(Ctx* c);
+int stage_stitch_finish_sharded(Ctx* c);
 uint32_t choose_bin_count(const Ctx* c, uint64_t instances, int n_shards);
 void set_minimizer(Ctx* c, uint32_t n_bins_total);  // c->m from the TOTAL bin count (rfx_partition.cu)
 int stage_count_sharded(Ctx* c);

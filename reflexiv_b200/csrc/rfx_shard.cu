@@ -558,6 +558,7 @@ int rfx_shard_set_bins(rfx_ctx* c, uint32_t n_bins_total) {
 int rfx_count_sharded(rfx_ctx* c) {
     if (!c) return RFX_E_INVALID;
     cudaSetDevice(c->prm.device);
+    c->st_active = false;  // an open stitch stage is abandoned: its fragments refer to the contigs it was opened on
     return stage_count_sharded(c);
 }
 
@@ -570,7 +571,20 @@ int rfx_shard_table(rfx_ctx* c) {
 int rfx_assemble_sharded(rfx_ctx* c) {
     if (!c) return RFX_E_INVALID;
     cudaSetDevice(c->prm.device);
+    c->st_active = false;  // an open stitch stage is abandoned: its fragments refer to the contigs it was opened on
     return stage_assemble_sharded(c);
+}
+
+int rfx_stitch_begin_sharded(rfx_ctx* c) {
+    if (!c) return RFX_E_INVALID;
+    cudaSetDevice(c->prm.device);
+    return stage_stitch_begin_sharded(c);
+}
+
+int rfx_stitch_finish_sharded(rfx_ctx* c) {
+    if (!c) return RFX_E_INVALID;
+    cudaSetDevice(c->prm.device);
+    return stage_stitch_finish_sharded(c);
 }
 
 int rfx_sort_kmers_sharded(rfx_ctx* c, int32_t min_error_coverage, double min_repeat_fold, int32_t max_kmer_size) {

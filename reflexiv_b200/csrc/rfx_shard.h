@@ -55,6 +55,7 @@ int shard_exchange(Ctx* c, int rc, int n, const unsigned long long* mine, PubVal
 void shard_graph_release(Ctx* c);
 void shard_graph_reset(Ctx* c);  // forget the graph stages' arena buffers (rfx_reset)
 void shard_graph_stats(Ctx* c, rfx_shard_stats_t* out);
+void shard_graph_set_contigs_global(Ctx* c, uint64_t n_contigs, uint64_t n_bases);  // rfx_shard_stats after a stage that replaced the contigs
 void free_all_buffers(Ctx* c);
 
 }  // namespace rfx

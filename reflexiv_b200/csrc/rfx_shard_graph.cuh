@@ -1440,6 +1440,12 @@ void shard_graph_release(Ctx* c) {
     c->gshard = nullptr;
 }
 
+void shard_graph_set_contigs_global(Ctx* c, uint64_t n_contigs, uint64_t n_bases) {
+    if (!c->gshard) c->gshard = new GShard();
+    c->gshard->n_contigs_global = n_contigs;
+    c->gshard->n_bases_global = n_bases;
+}
+
 void shard_graph_stats(Ctx* c, rfx_shard_stats_t* out) {
     if (!c->gshard) return;
     const GShard* gs = c->gshard;

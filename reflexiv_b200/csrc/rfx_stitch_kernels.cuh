@@ -6,6 +6,8 @@
 #ifndef RFX_STITCH_HOSTEMU
 #include "rfx_internal.h"
 #include "rfx_scan.cuh"
+#elif !defined(__grid_constant__)
+#define __grid_constant__
 #endif
 
 namespace rfx {
@@ -85,6 +87,15 @@ __device__ void probe_insert(uint64_t key, uint32_t val, uint64_t* keys, uint32_
         cur = seen;
     }
 }
+// the probes of contig c (its first (k-1)-mer a, its last b) for the ends that are clean and covered <= 4 times (the caller
+// has checked the length)
+__device__ __forceinline__ void probe_contig(uint64_t c, int32_t cl, int32_t cr, uint64_t a, uint64_t b, uint64_t* keys, uint32_t* vals, uint64_t mask,
+                                             const uint64_t* firstk, uint32_t* bloom, unsigned long long* n_probes) {
+    const bool l = cl >= -5 && cl < 0, r = cr >= -5 && cr < 0;
+    if (l) probe_insert(a, (uint32_t)(c << 1) | 1u, keys, vals, mask, firstk, bloom);
+    if (r) probe_insert(b, (uint32_t)(c << 1), keys, vals, mask, firstk, bloom);
+    if (l || r) atomicAdd(n_probes, (unsigned long long)l + (unsigned long long)r);
+}
 __global__ void probe_insert_kernel(const uint64_t* __restrict__ off, const char* __restrict__ bases, const int32_t* __restrict__ cl,
                                     const int32_t* __restrict__ cr, uint64_t n, int k, const uint64_t* __restrict__ firstk, uint64_t* keys,
                                     uint32_t* vals, uint64_t mask, uint32_t* bloom, unsigned long long* n_probes) {
@@ -92,16 +103,44 @@ __global__ void probe_insert_kernel(const uint64_t* __restrict__ off, const char
     for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n; c += (uint64_t)gridDim.x * blockDim.x) {
         const uint64_t len = off[c + 1] - off[c];
         if (len < 61) continue;  // :1229
-        const bool l = cl[c] >= -5 && cl[c] < 0, r = cr[c] >= -5 && cr[c] < 0;
-        if (!l && !r) continue;
+        if (!(cl[c] >= -5 && cl[c] < 0) && !(cr[c] >= -5 && cr[c] < 0)) continue;
         uint64_t a = 0, b = 0;
         for (int j = 0; j < sk; j++) {
             a = (a << 2) | nv((uint8_t)bases[off[c] + j]);
             b = (b << 2) | nv((uint8_t)bases[off[c + 1] - sk + j]);
         }
-        if (l) probe_insert(a, (uint32_t)(c << 1) | 1u, keys, vals, mask, firstk, bloom);
-        if (r) probe_insert(b, (uint32_t)(c << 1), keys, vals, mask, firstk, bloom);
-        atomicAdd(n_probes, (unsigned long long)l + (unsigned long long)r);
+        probe_contig(c, cl[c], cr[c], a, b, keys, vals, mask, firstk, bloom, n_probes);
+    }
+}
+
+// ---- S1 across ranks (rfx_stitch_begin_sharded): every rank summarises its own contigs, pulls everybody's summary and builds
+// the same probe table over global contig ids (a rank's prefix + its local index)
+// ends[2c], ends[2c + 1]: the first and the last (k-1)-mer of contig c (0 for a contig too short to probe)
+__global__ void contig_ends_kernel(const uint64_t* __restrict__ off, const char* __restrict__ bases, uint64_t n, int k, uint64_t* __restrict__ ends) {
+    const int sk = k - 1;
+    for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n; c += (uint64_t)gridDim.x * blockDim.x) {
+        uint64_t a = 0, b = 0;
+        if (off[c + 1] - off[c] >= 61)
+            for (int j = 0; j < sk; j++) {
+                a = (a << 2) | nv((uint8_t)bases[off[c] + j]);
+                b = (b << 2) | nv((uint8_t)bases[off[c + 1] - sk + j]);
+            }
+        ends[2 * c] = a;
+        ends[2 * c + 1] = b;
+    }
+}
+// a rank's contig offsets (possibly in a peer's memory) -> its slice of the global offsets, moved by `add` bases
+__global__ void rebase_off_kernel(const uint64_t* __restrict__ src, uint64_t n, uint64_t add, uint64_t* __restrict__ dst) {
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) dst[i] = src[i] + add;
+}
+// probe_insert_kernel over the pulled summaries: global offsets, ends, flags
+__global__ void probe_insert_ends_kernel(const uint64_t* __restrict__ off, const uint64_t* __restrict__ ends, const int32_t* __restrict__ cl,
+                                         const int32_t* __restrict__ cr, uint64_t n, const uint64_t* __restrict__ firstk, uint64_t* keys, uint32_t* vals,
+                                         uint64_t mask, uint32_t* bloom, unsigned long long* n_probes) {
+    for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n; c += (uint64_t)gridDim.x * blockDim.x) {
+        const uint64_t len = off[c + 1] - off[c];
+        if (len < 61) continue;  // :1229
+        probe_contig(c, cl[c], cr[c], ends[2 * c], ends[2 * c + 1], keys, vals, mask, firstk, bloom, n_probes);
     }
 }
 __global__ void count_keys_kernel(const uint64_t* __restrict__ keys, uint64_t cap, unsigned long long* n) {
@@ -298,46 +337,52 @@ __global__ void chain_heads_kernel(uint64_t n, const uint32_t* __restrict__ nxt,
     }
 }
 // what no head reached lies on a ring: its member with the smallest first k-mer becomes the head (a record never meets itself)
+__device__ __forceinline__ void ring_head_at(uint64_t c, uint64_t n, const uint32_t* __restrict__ nxt, const uint32_t* __restrict__ prv, const Frag* __restrict__ f,
+                                             const uint64_t* __restrict__ firstk, uint8_t* role, unsigned long long* n_rings) {
+    if (prv[c] == NONE32 || role[c] == 2) return;
+    bool smallest = true;
+    uint64_t steps = 0;
+    for (uint32_t cur = next_ctg((uint32_t)c, nxt, prv, f); cur != (uint32_t)c && cur != NONE32 && steps < n; cur = next_ctg(cur, nxt, prv, f), steps++)
+        if (firstk[cur] < firstk[c] || (firstk[cur] == firstk[c] && cur < (uint32_t)c)) { smallest = false; break; }
+    if (smallest) { role[c] = 3; atomicAdd(n_rings, 1ull); }
+}
 __global__ void ring_heads_kernel(uint64_t n, const uint32_t* __restrict__ nxt, const uint32_t* __restrict__ prv, const Frag* __restrict__ f,
                                   const uint64_t* __restrict__ firstk, uint8_t* role, unsigned long long* n_rings) {
-    for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n; c += (uint64_t)gridDim.x * blockDim.x) {
-        if (prv[c] == NONE32 || role[c] == 2) continue;
-        bool smallest = true;
-        uint64_t steps = 0;
-        for (uint32_t cur = next_ctg((uint32_t)c, nxt, prv, f); cur != (uint32_t)c && cur != NONE32 && steps < n; cur = next_ctg(cur, nxt, prv, f), steps++)
-            if (firstk[cur] < firstk[c] || (firstk[cur] == firstk[c] && cur < (uint32_t)c)) { smallest = false; break; }
-        if (smallest) { role[c] = 3; atomicAdd(n_rings, 1ull); }
-    }
+    for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n; c += (uint64_t)gridDim.x * blockDim.x) ring_head_at(c, n, nxt, prv, f, firstk, role, n_rings);
 }
 // length, right flag and keep decision (DSKmerToContig :749-754) of the record every head stands for
+__device__ __forceinline__ void chain_size_at(uint64_t c, uint64_t n, int k, int min_contig, const uint64_t* __restrict__ off, const int32_t* __restrict__ cl,
+                                              const int32_t* __restrict__ cr, const uint32_t* __restrict__ nxt, const uint32_t* __restrict__ prv, const Frag* __restrict__ f,
+                                              const uint8_t* __restrict__ role, uint64_t* out_len, int32_t* out_right, unsigned long long* n_stitched) {
+    const uint64_t sk = (uint64_t)k - 1;
+    uint64_t len = 0;
+    int32_t right = 0;
+    const uint8_t ro = role[c];
+    if (ro != 2 && !(ro == 0 && prv[c] != NONE32)) {  // (role 0 with an arriving fragment: a ring member that is not its head)
+        len = off[c + 1] - off[c];
+        right = cr[c];
+        uint32_t cur = (uint32_t)c;
+        for (uint64_t steps = 0; nxt[cur] != NONE32 && steps < n; steps++) {
+            const Frag F = f[nxt[cur]];
+            len += F.len - sk;
+            right = -10000000;
+            if (prv[F.right_ctg] != nxt[cur]) break;  // another fragment joined the contig this one ends on
+            cur = F.right_ctg;
+            if (cur == (uint32_t)c) break;            // ring closed: the closing fragment ends the record
+            len += off[cur + 1] - off[cur] - sk;
+            right = cr[cur];
+        }
+        if (nxt[c] != NONE32) atomicAdd(n_stitched, 1ull);
+        if ((cl[c] <= -10000000 && right <= -10000000) || len < (uint64_t)min_contig) len = 0;
+    }
+    *out_len = len;
+    *out_right = right;
+}
 __global__ void chain_sizes_kernel(uint64_t n, int k, int min_contig, const uint64_t* __restrict__ off, const int32_t* __restrict__ cl,
                                    const int32_t* __restrict__ cr, const uint32_t* __restrict__ nxt, const uint32_t* __restrict__ prv, const Frag* __restrict__ f,
                                    const uint8_t* __restrict__ role, uint64_t* out_len, int32_t* out_right, unsigned long long* n_stitched) {
-    const uint64_t sk = (uint64_t)k - 1;
-    for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n; c += (uint64_t)gridDim.x * blockDim.x) {
-        uint64_t len = 0;
-        int32_t right = 0;
-        const uint8_t ro = role[c];
-        if (ro != 2 && !(ro == 0 && prv[c] != NONE32)) {  // (role 0 with an arriving fragment: a ring member that is not its head)
-            len = off[c + 1] - off[c];
-            right = cr[c];
-            uint32_t cur = (uint32_t)c;
-            for (uint64_t steps = 0; nxt[cur] != NONE32 && steps < n; steps++) {
-                const Frag F = f[nxt[cur]];
-                len += F.len - sk;
-                right = -10000000;
-                if (prv[F.right_ctg] != nxt[cur]) break;  // another fragment joined the contig this one ends on
-                cur = F.right_ctg;
-                if (cur == (uint32_t)c) break;            // ring closed: the closing fragment ends the record
-                len += off[cur + 1] - off[cur] - sk;
-                right = cr[cur];
-            }
-            if (nxt[c] != NONE32) atomicAdd(n_stitched, 1ull);
-            if ((cl[c] <= -10000000 && right <= -10000000) || len < (uint64_t)min_contig) len = 0;
-        }
-        out_len[c] = len;
-        out_right[c] = right;
-    }
+    for (uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < n; c += (uint64_t)gridDim.x * blockDim.x)
+        chain_size_at(c, n, k, min_contig, off, cl, cr, nxt, prv, f, role, &out_len[c], &out_right[c], n_stitched);
 }
 struct KeepIn {
     const uint64_t* out_len;
@@ -354,30 +399,88 @@ struct KeepOut {
     }
 };
 __global__ void set_end_kernel(uint64_t* p, const U64x3* tot) { *p = tot->b; }
-// one block per record: contig, fragment extension, contig minus its first k-1 bases, ...
+// the record of head c, written by the threads of one block: contig, fragment extension, contig minus its first k-1 bases, ...
+// bases_of(g): the first base of contig g
+template <class BasesOf>
+__device__ __forceinline__ void gather_record(uint64_t c, uint64_t n, int k, const uint64_t* __restrict__ off, BasesOf bases_of, const uint32_t* __restrict__ nxt,
+                                              const uint32_t* __restrict__ prv, const Frag* __restrict__ f, const uint8_t* __restrict__ codes, char* __restrict__ dst) {
+    const uint64_t sk = (uint64_t)k - 1;
+    uint64_t l0 = off[c + 1] - off[c];
+    const char* src = bases_of((uint32_t)c);
+    for (uint64_t j = threadIdx.x; j < l0; j += blockDim.x) dst[j] = src[j];
+    dst += l0;
+    uint32_t cur = (uint32_t)c;
+    for (uint64_t steps = 0; nxt[cur] != NONE32 && steps < n; steps++) {
+        const Frag F = f[nxt[cur]];
+        for (uint64_t j = threadIdx.x; j + sk < F.len; j += blockDim.x) dst[j] = "ACGT"[codes[F.off + sk + j]];
+        dst += F.len - sk;
+        if (prv[F.right_ctg] != nxt[cur]) break;
+        cur = F.right_ctg;
+        if (cur == (uint32_t)c) break;
+        l0 = off[cur + 1] - off[cur] - sk;
+        src = bases_of(cur) + sk;
+        for (uint64_t j = threadIdx.x; j < l0; j += blockDim.x) dst[j] = src[j];
+        dst += l0;
+    }
+}
+struct LocalBases {
+    const uint64_t* off;
+    const char* bases;
+    __device__ __forceinline__ const char* operator()(uint32_t g) const { return bases + off[g]; }
+};
+// one block per record
 __global__ void __launch_bounds__(256) chain_gather_kernel(uint64_t n, int k, const uint64_t* __restrict__ off, const char* __restrict__ bases,
                                                            const uint32_t* __restrict__ nxt, const uint32_t* __restrict__ prv, const Frag* __restrict__ f,
                                                            const uint8_t* __restrict__ codes, const uint64_t* __restrict__ slot_of,
                                                            const uint64_t* __restrict__ new_off, char* __restrict__ out) {
-    const uint64_t sk = (uint64_t)k - 1;
     for (uint64_t c = blockIdx.x; c < n; c += gridDim.x) {
         if (slot_of[c] == ~0ull) continue;
-        char* dst = out + new_off[slot_of[c]];
-        uint64_t l0 = off[c + 1] - off[c];
-        for (uint64_t j = threadIdx.x; j < l0; j += blockDim.x) dst[j] = bases[off[c] + j];
-        dst += l0;
-        uint32_t cur = (uint32_t)c;
-        for (uint64_t steps = 0; nxt[cur] != NONE32 && steps < n; steps++) {
-            const Frag F = f[nxt[cur]];
-            for (uint64_t j = threadIdx.x; j + sk < F.len; j += blockDim.x) dst[j] = "ACGT"[codes[F.off + sk + j]];
-            dst += F.len - sk;
-            if (prv[F.right_ctg] != nxt[cur]) break;
-            cur = F.right_ctg;
-            if (cur == (uint32_t)c) break;
-            l0 = off[cur + 1] - off[cur] - sk;
-            for (uint64_t j = threadIdx.x; j < l0; j += blockDim.x) dst[j] = bases[off[cur] + sk + j];
-            dst += l0;
-        }
+        gather_record(c, n, k, off, LocalBases{off, bases}, nxt, prv, f, codes, out + new_off[slot_of[c]]);
+    }
+}
+
+// ---- S3 / S4 across ranks (rfx_stitch_finish_sharded): every rank holds all fragments and the replicated per-contig arrays
+// over global ids, runs the picks and chain_heads_kernel over all of them, and the kernels below over the heads [lo, hi) it owns.
+// Per-head outputs (out_len, out_right, slot_of) are indexed by c - lo.
+__global__ void ring_heads_range_kernel(uint64_t lo, uint64_t hi, uint64_t n, const uint32_t* __restrict__ nxt, const uint32_t* __restrict__ prv,
+                                        const Frag* __restrict__ f, const uint64_t* __restrict__ firstk, uint8_t* role, unsigned long long* n_rings) {
+    for (uint64_t c = lo + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < hi; c += (uint64_t)gridDim.x * blockDim.x) ring_head_at(c, n, nxt, prv, f, firstk, role, n_rings);
+}
+__global__ void chain_sizes_range_kernel(uint64_t lo, uint64_t hi, uint64_t n, int k, int min_contig, const uint64_t* __restrict__ off, const int32_t* __restrict__ cl,
+                                         const int32_t* __restrict__ cr, const uint32_t* __restrict__ nxt, const uint32_t* __restrict__ prv, const Frag* __restrict__ f,
+                                         const uint8_t* __restrict__ role, uint64_t* out_len, int32_t* out_right, unsigned long long* n_stitched) {
+    for (uint64_t c = lo + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; c < hi; c += (uint64_t)gridDim.x * blockDim.x)
+        chain_size_at(c, n, k, min_contig, off, cl, cr, nxt, prv, f, role, &out_len[c - lo], &out_right[c - lo], n_stitched);
+}
+// where every rank's contigs are: global ids [ctg_lo[r], ctg_lo[r + 1]) hold bases [base_lo[r], base_lo[r + 1]) of the global
+// offsets, stored from bases[r] on (the rank's own contig bases, as seen from this device: possibly a peer's memory)
+struct CtgSources {
+    const char* bases[8];
+    unsigned long long ctg_lo[9], base_lo[9];
+    int n;
+    const uint64_t* off;  // global offsets
+    __device__ __forceinline__ const char* operator()(uint32_t g) const {
+        int r = 0;
+        while (r + 1 < n && (unsigned long long)g >= ctg_lo[r + 1]) r++;
+        return bases[r] + (off[g] - base_lo[r]);
+    }
+};
+// one block per own head: the pieces of its record are read where they lie, contig bases from their owner over peer memory
+__global__ void __launch_bounds__(256) chain_gather_peer_kernel(uint64_t lo, uint64_t hi, uint64_t n, int k, const __grid_constant__ CtgSources P,
+                                                                const uint32_t* __restrict__ nxt, const uint32_t* __restrict__ prv, const Frag* __restrict__ f,
+                                                                const uint8_t* __restrict__ codes, const uint64_t* __restrict__ slot_of,
+                                                                const uint64_t* __restrict__ new_off, char* __restrict__ out) {
+    for (uint64_t c = lo + blockIdx.x; c < hi; c += gridDim.x) {
+        if (slot_of[c - lo] == ~0ull) continue;
+        gather_record(c, n, k, P.off, P, nxt, prv, f, codes, out + new_off[slot_of[c - lo]]);
+    }
+}
+// a rank's fragments (possibly in a peer's memory) -> their place in the global list, code offsets moved by `add`
+__global__ void frag_pull_kernel(const Frag* __restrict__ src, uint64_t n, uint64_t add, Frag* __restrict__ dst) {
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
+        Frag F = src[i];
+        F.off += add;
+        dst[i] = F;
     }
 }
 __global__ void fill_u32_kernel(uint32_t* p, uint64_t n, uint32_t v) {

@@ -314,6 +314,19 @@ class ReflexivContext:
         self._check(self.L.rfx_sorted_size(self._ctx, C.byref(n)), self._ctx)
         return n.value
 
+    def stitch_begin_sharded(self):
+        """Collective stitch_begin() on a table sharded by minimiser bin (after count_sharded() or shard_table()).  Until
+        stitch_finish_sharded() the push_* calls of this rank scan its own reads for fragments (not collective: any split of
+        the reads, a rank may push none)."""
+        self._check(self.L.rfx_stitch_begin_sharded(self._ctx), self._ctx)
+        return self.stitch_stats()
+
+    def stitch_finish_sharded(self):
+        """Collective stitch_finish(): contigs() then returns the stitched records whose head contig this rank owns; their
+        union over the ranks is the one-context result."""
+        self._check(self.L.rfx_stitch_finish_sharded(self._ctx), self._ctx)
+        return self.stitch_stats()
+
     def shard_stats(self) -> dict:
         s = _lib.RfxShardStats()
         self._check(self.L.rfx_shard_stats(self._ctx, C.byref(s)), self._ctx)
