@@ -105,12 +105,8 @@ def _palindromes(rng, half: int, n: int) -> list:
     return out
 
 
-@pytest.mark.parametrize("glen,seed", [(3000, 1), (20000, 2)])
-def test_palindromic_rows_at_k12(R, orc, monkeypatch, glen, seed):
-    """Even k: a palindromic row is one node (find returns its even id, the odd id is dead).  Its predecessors and its
-    left group are reached through the other strand of a neighbour; that strand must be mapped back to the even id, or a
-    palindromic candidate's count is dropped from a left group.  Palindromes sit inside real forks here (repeated
-    11-mers at this genome size)."""
+def palindromic_table_k12(glen: int, seed: int):
+    """k = 12 table: a genome with 40 palindromic 12-mers spliced in, each palindrome again with other flanks."""
     from workload import synth
     k = 12
     rng = np.random.default_rng(seed)
@@ -122,34 +118,47 @@ def test_palindromic_rows_at_k12(R, orc, monkeypatch, glen, seed):
         parts.append(g[pos:pos + 40] + p)
         pos += 40
     seqs = ["".join(parts) + g[pos:], "".join(p + g[i * 7:i * 7 + 5] for i, p in enumerate(pals))]
-    keys, counts = _table(seqs, k, lambda key, si: 10 + (hash((key, seed)) % 3) if si == 0 else 2 + (key % 15))
-    n_pal = sum(int(x) == _rc(int(x), k) for x in keys)
+    return _table(seqs, k, lambda key, si: 10 + (hash((key, seed)) % 3) if si == 0 else 2 + (key % 15))
+
+
+@pytest.mark.parametrize("glen,seed", [(3000, 1), (20000, 2)])
+def test_palindromic_rows_at_k12(R, orc, monkeypatch, glen, seed):
+    """Even k: a palindromic row is one node (find returns its even id, the odd id is dead).  Its predecessors and its
+    left group are reached through the other strand of a neighbour; that strand must be mapped back to the even id, or a
+    palindromic candidate's count is dropped from a left group.  Palindromes sit inside real forks here (repeated
+    11-mers at this genome size)."""
+    keys, counts = palindromic_table_k12(glen, seed)
+    n_pal = sum(int(x) == _rc(int(x), 12) for x in keys)
     assert n_pal >= 20
-    _check_table(R, orc, monkeypatch, keys, counts, k)
+    _check_table(R, orc, monkeypatch, keys, counts, 12)
+
+
+def palindromic_reads_k32(at_stretch: bool = True) -> bytes:
+    """Reads (0.5 % errors) of a genome with a palindromic AT stretch (a closed path) and 12 palindromic 32-mers, one of
+    them twice."""
+    from workload import synth
+    rng = np.random.default_rng(7)
+    g = synth.genome(30_000, 732)
+    if at_stretch:
+        g[20000:20060] = np.frombuffer(b"AT" * 30, np.uint8)
+    for i, p in enumerate(_palindromes(rng, 16, 12)):
+        g[2000 + 1500 * i:2000 + 1500 * i + 32] = np.frombuffer(p.encode(), np.uint8)
+    g[25000:25032] = g[2000:2032]  # one palindrome twice: forks around it
+    return bytes(synth.fastq(g, 6000, read_len=150, frag_len=400, error_rate=0.005, seed_reads=11, seed_errors=12))
 
 
 def test_palindromic_rows_at_k32(R, orc, monkeypatch):
     """k = 32 (two-word keys): palindromic stretches and embedded palindromes in a read set, with repeats."""
-    from workload import synth
-    rng = np.random.default_rng(7)
-    g = synth.genome(30_000, 732)
-    g[20000:20060] = np.frombuffer(b"AT" * 30, np.uint8)
-    for i, p in enumerate(_palindromes(rng, 16, 12)):
-        g[2000 + 1500 * i:2000 + 1500 * i + 32] = np.frombuffer(p.encode(), np.uint8)
-    g[25000:25032] = g[2000:2032]  # one palindrome twice: forks around it
-    txt = synth.fastq(g, 6000, read_len=150, frag_len=400, error_rate=0.005, seed_reads=11, seed_errors=12)
-    _check_reads(R, orc, monkeypatch, txt, 32, 2, min_contig=100)
+    _check_reads(R, orc, monkeypatch, palindromic_reads_k32(), 32, 2, min_contig=100)
 
 
-@pytest.mark.parametrize("k", [31, 12])
-@pytest.mark.parametrize("tip_count", [2, 11])
-def test_fork_groups_at_chain_ends(R, orc, monkeypatch, k, tip_count):
-    """Siblings without a predecessor (forks at the first k-mer of a sequence) and without a successor (forks at the
-    last one): no stored out-set names their groups, so each node probes its siblings directly.  Tips as errors (count 2
-    against 10..12) and as real forks (count 11)."""
+def chain_end_table(k: int, tip_count: int, seed: int = 0):
+    """A 3000-base genome (counts 10..12) with forks at both chain ends and three dead ends inside, the tips at tip_count.
+    Returns the sequences (the genome first, then the branches of the head group, the tail group and the dead ends), keys
+    and counts."""
     from workload import synth
-    rng = np.random.default_rng(100 + k + tip_count)
-    g = synth.genome(3000, 900 + k).tobytes().decode()
+    rng = np.random.default_rng(100 + k + tip_count + 1000 * seed)
+    g = synth.genome(3000, 900 + k + 1000 * seed).tobytes().decode()
 
     def other(b):
         return "ACGT"[("ACGT".index(b) + 1 + int(rng.integers(0, 3))) % 4]
@@ -165,6 +174,16 @@ def test_fork_groups_at_chain_ends(R, orc, monkeypatch, k, tip_count):
         seqs.append(y)
         seqs.append(other(y[0]) + y[1:])
     keys, counts = _table(seqs, k, lambda key, si: 10 + (key % 3) if si == 0 else tip_count)
+    return seqs, keys, counts
+
+
+@pytest.mark.parametrize("k", [31, 12])
+@pytest.mark.parametrize("tip_count", [2, 11])
+def test_fork_groups_at_chain_ends(R, orc, monkeypatch, k, tip_count):
+    """Siblings without a predecessor (forks at the first k-mer of a sequence) and without a successor (forks at the
+    last one): no stored out-set names their groups, so each node probes its siblings directly.  Tips as errors (count 2
+    against 10..12) and as real forks (count 11)."""
+    _, keys, counts = chain_end_table(k, tip_count)
     ff, _ = _check_table(R, orc, monkeypatch, keys, counts, k)
     assert (ff["left"] >= 0).any() or (ff["right"] >= 0).any() or tip_count == 2
 
@@ -178,6 +197,41 @@ def test_one_cycle_and_circular_genome(R, orc, monkeypatch):
     _check_reads(R, orc, monkeypatch, _fq(["A" * 100] * 3), 31, 2)
     _check_reads(R, orc, monkeypatch, _fq(["A" * 60 + circ[:80]] * 3 + ["C" * 50 + "A" * 60] * 3), 31, 2)
     _check_reads(R, orc, monkeypatch, _fq(["ACGT" * 30] * 3), 16, 2)
+
+
+def hairpin_reads(k: int, seed: int = 0):
+    """Odd k: error-free reads (every 5 bases, twice) of a 3000-base genome with six palindromic (k-1)-mers P spliced in.
+    The node X = aP (a the base in front of P) has rc(X) = P·comp(a) among its successors: where the genome goes on with
+    comp(a) that is its only successor (a straight hairpin), elsewhere a fork against X's own row.  Returns the genome, the
+    sites (start of P, straight or not) and the FASTQ text."""
+    from workload import synth
+    assert k % 2 == 1
+    comp = dict(zip("ACGT", "TGCA"))
+    rng = np.random.default_rng(60 + k + 1000 * seed)
+    g = list(synth.genome(3000, 960 + k + 1000 * seed).tobytes().decode())
+    sites = []
+    for i, p in enumerate(_palindromes(rng, (k - 1) // 2, 6)):
+        at, straight = 200 + 450 * i, i % 2 == 0
+        g[at:at + k - 1] = p
+        c = comp[g[at - 1]]
+        g[at + k - 1] = c if straight else "ACGT"[("ACGT".index(c) + 1 + int(rng.integers(0, 3))) % 4]
+        sites.append((at, straight))
+    g = "".join(g)
+    return g, sites, _fq([g[i:i + 120] for i in range(0, len(g) - 119, 5)] * 2)
+
+
+@pytest.mark.parametrize("k", [31, 33, 61])
+def test_hairpins_at_odd_k(R, orc, monkeypatch, k):
+    """A palindromic (k-1)-mer inside a genome: a node whose successor group holds the other strand of its own row, alone
+    (straight hairpin) or next to the genome's successor (a fork against the own row).  k = 33 and 61: two-word keys."""
+    g, sites, txt = hairpin_reads(k)
+    comp = dict(zip("ACGT", "TGCA"))
+    for at, straight in sites:
+        p = g[at:at + k - 1]
+        assert p == p[::-1].translate(str.maketrans("ACGT", "TGCA"))
+        assert (g[at + k - 1] == comp[g[at - 1]]) == straight
+    assert {s for _, s in sites} == {True, False}
+    _check_reads(R, orc, monkeypatch, txt, k, 2, min_contig=k)
 
 
 @pytest.mark.parametrize("skewed", [False, True])
