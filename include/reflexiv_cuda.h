@@ -137,6 +137,21 @@ int rfx_counts_csv(rfx_ctx* ctx, char* out, uint64_t cap, uint64_t* n_bytes);
 /* load an existing filtered table instead of counting (the -kmerc seam, ReflexivDSMain.java:362-713);
  * keys in the layout rfx_counts_copy produces */
 int rfx_load_counts(rfx_ctx* ctx, const uint64_t* keys, const uint32_t* counts, uint64_t n_rows);
+/* Count_<k> text (KmerBinarizer rows) parsed on the device into the context's table, in the internal key layout.
+ * Rows kept iff min_count <= count <= max_count.  append == 0 replaces the table (len == 0: an empty table),
+ * append != 0 extends it.  Every call ends on a line boundary; a last line without '\n' is a row.
+ * Row rule (the `reflexiv` binary's, ReflexivDSMain.java:3872-3948): a trailing '\r' is dropped, empty lines are skipped, one
+ * leading '(' and one trailing ')' are stripped; the k-mer is the first k characters (A=0 C=1 G=2, anything else 3); the count is
+ * everything behind the first ',': 10 or more characters give 10^9, fewer are read as decimal digits up to the first non-digit.
+ * A row with no ',' or fewer than k characters in front of it: RFX_E_INVALID, the message names its line (counted from 1 within
+ * the call), and the context holds no table.  Surviving rows keep their text order and appended calls follow each other: the
+ * table is, row for row, what rfx_load_counts makes of the same rows.  Same effects as rfx_load_counts otherwise (an open stitch
+ * stage is abandoned, contigs and sorted rows are dropped; on a sharded context the table is a loaded slice until
+ * rfx_shard_table).  The text is uploaded in chunks of whole lines (16 MB) into two staging slots while the previous chunk is
+ * parsed; besides the table the call needs 2 chunks of staging plus about 30 bytes per line of one chunk (about 1.8 chunks for
+ * 40-byte rows), in the arena of a sharded context too, where the table grows by doubling (an outgrown block is not reused).
+ * rfx_stats: the call's GPU time is added to ms_parse. */
+int rfx_load_counts_csv(rfx_ctx* ctx, const uint8_t* text, size_t len, int64_t min_count, int64_t max_count, int32_t append);
 
 /* ---- assembly ------------------------------------------------------------------------------
  * replaces DSKmerReverseComplementLong .. DSExtendReflexivKmerToArrayLoop .. DSKmerToContig

@@ -61,6 +61,7 @@ public final class ReflexivCuda implements AutoCloseable {
     private static final MethodHandle COUNTS_COPY = h("rfx_counts_copy", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS));
     private static final MethodHandle COUNTS_CSV = h("rfx_counts_csv", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));
     private static final MethodHandle LOAD_COUNTS = h("rfx_load_counts", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG));
+    private static final MethodHandle LOAD_COUNTS_CSV = h("rfx_load_counts_csv", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, JAVA_LONG, JAVA_LONG, JAVA_INT));
     private static final MethodHandle ASSEMBLE = h("rfx_assemble", FunctionDescriptor.of(JAVA_INT, ADDRESS));
     private static final MethodHandle CONTIGS_SIZE = h("rfx_contigs_size", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS));
     private static final MethodHandle CONTIGS_COPY = h("rfx_contigs_copy", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS));
@@ -199,6 +200,14 @@ public final class ReflexivCuda implements AutoCloseable {
         } catch (Throwable t) {
             throw new RuntimeException(t);
         }
+    }
+
+    /**
+     * -kmerc: Count_<k> text (a mapped part file or a direct buffer, whole lines) parsed on the device; rows with
+     * minCount <= count <= maxCount are kept in text order, behind the current table if append (include/reflexiv_cuda.h).
+     */
+    public void loadCountsCsv(MemorySegment text, long minCount, long maxCount, boolean append) {
+        call(() -> (int) LOAD_COUNTS_CSV.invoke(ctx, text, text.byteSize(), minCount, maxCount, append ? 1 : 0));
     }
 
     /** Both strands of every contig, order unspecified (as the reference's part files). */

@@ -74,6 +74,7 @@ SYMBOLS = {
     "rfx_counts_copy": (C.c_int, [_P, _P, _P]),
     "rfx_counts_csv": (C.c_int, [_P, _P, C.c_uint64, C.POINTER(C.c_uint64)]),
     "rfx_load_counts": (C.c_int, [_P, _P, _P, C.c_uint64]),
+    "rfx_load_counts_csv": (C.c_int, [_P, _P, C.c_size_t, C.c_int64, C.c_int64, C.c_int32]),
     "rfx_assemble": (C.c_int, [_P]),
     "rfx_contigs_size": (C.c_int, [_P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "rfx_contigs_copy": (C.c_int, [_P, _P, _P, _P, _P]),

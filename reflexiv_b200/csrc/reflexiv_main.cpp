@@ -291,7 +291,8 @@ static bool parse_count_rows(const char* data, size_t from, size_t to, int k, in
 
 // KmerBinarizer input: `KMER,count` or legacy `(KMER,count)`, ReflexivDSMain.java:3872-3948.  Large tables are cut at line
 // starts into one piece per host thread (Spark parses every partition of the CSV on its own core); row order is kept.
-static bool parse_counts(const char* data, size_t n, int k, int minc, int maxc, std::vector<uint64_t>& keys, std::vector<uint32_t>& counts) {
+// The -kmerc paths parse on the device (rfx_load_counts_csv); this host parser is the reference the tests compare that against.
+[[maybe_unused]] static bool parse_counts(const char* data, size_t n, int k, int minc, int maxc, std::vector<uint64_t>& keys, std::vector<uint32_t>& counts) {
     unsigned T = std::thread::hardware_concurrency();
     if (const char* e = getenv("REFLEXIV_READERS")) T = (unsigned)std::max(1, atoi(e));
     if (T > 32) T = 32;
@@ -506,34 +507,42 @@ struct SortStage {
     int32_t max_kmer_size;
     bool k_listed;  // k is in -klist: otherwise no row takes part (ReflexivDSKmerLeftAndRightSorting.java:1695)
 };
-// Reads a Count_<k> table the way the one-GPU `run -kmerc` / `sort` does: run keeps cover <= count <= maxcov
-// (ReflexivDSMain.java:405-412), sort count <= maxcov only (ReflexivDSKmerLeftAndRightSorting.java:186-193) and only k-mers whose
-// length is in the list.  False (reported) on a file that cannot be read.
-static bool read_count_table(const std::string& pattern, const rfx_params& p, const SortStage* sort, std::vector<uint64_t>& keys, std::vector<uint32_t>& counts) {
-    bool well_formed = true;
-    const bool read_ok = stream_inputs(pattern, [&](const char* data, size_t n) {
-        well_formed = parse_counts(data, n, p.kmer_size, sort ? INT32_MIN : p.min_kmer_coverage, p.max_kmer_coverage, keys, counts);
-        return well_formed;
-    });
-    if (sort && !sort->k_listed) { keys.clear(); counts.clear(); }
-    if (!well_formed) fprintf(stderr, "reflexiv: malformed k-mer count row\n");
-    return read_ok;
-}
-// `run -kmerc <glob> --gpus N` / `sort -kmerc <glob> --gpus N`: the table is parsed on the host (read_count_table), rank r loads
-// the r-th contiguous slice of its rows, rfx_shard_table sends every row to the owner of its minimiser bin, then the sharded
-// assembly or (sort != nullptr) the sharded Count_<k>_sorted stage
-static int run_kmerc_sharded(int n_gpus, rfx_params p, const SortStage* sort, const std::string& pattern, const std::string& outdir, const std::string& target, bool gz) {
-    std::vector<uint64_t> keys;
-    std::vector<uint32_t> counts;
-    if (!read_count_table(pattern, p, sort, keys, counts)) return 1;
+// `run -kmerc <glob> --gpus N` / `sort -kmerc <glob> --gpus N`: every file is cut into N runs of whole lines and rank r parses its run
+// on its own device (rfx_load_counts_csv, appended to an empty table), rfx_shard_table sends every row to the owner of its minimiser
+// bin, then the sharded assembly or (sort != nullptr) the sharded Count_<k>_sorted stage.  Rows kept: min_count..max_count.
+static int run_kmerc_sharded(int n_gpus, rfx_params p, const SortStage* sort, int64_t min_count, int64_t max_count, const std::string& pattern,
+                             const std::string& outdir, const std::string& target, bool gz) {
     std::vector<Rank> R;
     if (!open_ranks(n_gpus, p, R)) return 1;
-    const uint64_t rows = counts.size();
-    const size_t words = p.kmer_size <= 31 ? 1 : (size_t)(p.kmer_size / 32 + 1);
-    const bool ok = run_ranks(R, [&](Rank& k, int r) {
-        const uint64_t lo = rows * (uint64_t)r / (uint64_t)n_gpus, hi = rows * (uint64_t)(r + 1) / (uint64_t)n_gpus;
-        k.what = "rfx_load_counts";
-        if ((k.rc = rfx_load_counts(k.c, keys.data() + lo * words, counts.data() + lo, hi - lo)) != RFX_OK) return;
+    for (Rank& k : R) {
+        k.what = "rfx_load_counts_csv";
+        k.rc = rfx_load_counts_csv(k.c, nullptr, 0, min_count, max_count, 0);
+    }
+    bool load_ok = true;
+    for (Rank& k : R) load_ok = load_ok && k.rc == RFX_OK;
+    const bool read_ok = load_ok && stream_inputs(pattern, [&](const char* data, size_t n) {
+        std::vector<size_t> cut(n_gpus + 1, n);
+        cut[0] = 0;
+        for (int r = 1; r < n_gpus; r++) {
+            const size_t want = std::max(cut[r - 1], n / n_gpus * r);
+            const char* nl = want < n ? static_cast<const char*>(memchr(data + want, '\n', n - want)) : nullptr;
+            cut[r] = nl ? (size_t)(nl - data) + 1 : n;
+        }
+        std::vector<std::thread> th;
+        for (int r = 0; r < n_gpus; r++)
+            th.emplace_back([&, r] {
+                if (cut[r + 1] > cut[r] && R[r].rc == RFX_OK) R[r].rc = rfx_load_counts_csv(R[r].c, reinterpret_cast<const uint8_t*>(data + cut[r]), cut[r + 1] - cut[r], min_count, max_count, 1);
+            });
+        for (auto& t : th) t.join();
+        for (auto& k : R) load_ok = load_ok && k.rc == RFX_OK;
+        return load_ok;
+    });
+    if (!read_ok || !load_ok) {
+        for (int r = 0; r < n_gpus; r++) if (R[r].rc != RFX_OK) fprintf(stderr, "reflexiv: %s (rank %d): %s\n", R[r].what, r, rfx_last_error(R[r].c));
+        destroy_ranks(R);
+        return 1;
+    }
+    const bool ok = run_ranks(R, [&](Rank& k, int) {
         k.what = "rfx_shard_table";
         if ((k.rc = rfx_shard_table(k.c)) != RFX_OK) return;
         if (sort) {
@@ -652,19 +661,30 @@ int main(int argc, char** argv) {
 
     if (n_gpus > 1 && stitch) { fprintf(stderr, "reflexiv: --gpus applies to runs from reads (-fastq), to -kmerc runs without -stitch and to sort; this one runs on one GPU\n"); n_gpus = 1; }
     if (n_gpus > RFX_SHARD_MAX_RANKS) { fprintf(stderr, "reflexiv: --gpus %d: at most %d\n", n_gpus, RFX_SHARD_MAX_RANKS); return 1; }
+    // the rows a -kmerc table keeps: run cover <= count <= maxcov (ReflexivDSMain.java:405-412), sort count <= maxcov only
+    // (ReflexivDSKmerLeftAndRightSorting.java:186-193) and only k-mers whose length is in the list (:1695): with k outside -klist every
+    // row is still checked and none is kept
+    const int64_t min_count = !sorter ? (int64_t)p.min_kmer_coverage : sort_stage.k_listed ? (int64_t)INT32_MIN : INT64_MAX;
+    const int64_t max_count = p.max_kmer_coverage;
     if (n_gpus > 1) {
         info("Initiating CUDA contexts ...");
-        if (from_kmer) return run_kmerc_sharded(n_gpus, p, sorter ? &sort_stage : nullptr, v["kmerc"], outdir, target, gz);
+        if (from_kmer) return run_kmerc_sharded(n_gpus, p, sorter ? &sort_stage : nullptr, min_count, max_count, v["kmerc"], outdir, target, gz);
         return run_sharded(n_gpus, p, counter, v["fastq"], outdir, target, gz);
     }
     info("Initiating CUDA context ...");
     rfx_ctx* c = nullptr;
     if (rfx_create(&c, &p) != RFX_OK) return fail(nullptr, "rfx_create");
     if (from_kmer) {
-        std::vector<uint64_t> keys;
-        std::vector<uint32_t> counts;
-        if (!read_count_table(v["kmerc"], p, sorter ? &sort_stage : nullptr, keys, counts)) { rfx_destroy(c); return 1; }
-        if (rfx_load_counts(c, keys.data(), counts.data(), counts.size()) != RFX_OK) return fail(c, "rfx_load_counts");
+        // every file parsed on the device as it arrives: the first call replaces the table, the others append
+        bool load_ok = true, loaded = false;
+        const bool read_ok = stream_inputs(v["kmerc"], [&](const char* data, size_t n) {
+            load_ok = rfx_load_counts_csv(c, reinterpret_cast<const uint8_t*>(data), n, min_count, max_count, loaded ? 1 : 0) == RFX_OK;
+            loaded = true;
+            return load_ok;
+        });
+        if (!load_ok) return fail(c, "rfx_load_counts_csv");
+        if (!read_ok) { rfx_destroy(c); return 1; }
+        if (!loaded && rfx_load_counts_csv(c, nullptr, 0, min_count, max_count, 0) != RFX_OK) return fail(c, "rfx_load_counts_csv");  // only empty files
     } else {
         bool push_ok = true, pushed = false;
         const bool read_ok = stream_inputs(v["fastq"], [&](const char* data, size_t n) {

@@ -81,7 +81,7 @@ void devbuf_free(DevBuf& b) {
 
 void free_all_buffers(Ctx* c) {
     DevBuf* all[] = {&c->text, &c->line_start, &c->line_at, &c->nl_masks, &c->seq_flag, &c->scan_ws, &c->rd_len, &c->rd_woff, &c->packed, &c->bin_off, &c->bin_cursor,
-                     &c->records, &c->keys, &c->counts, &c->dstat, &c->ht, &c->rflag, &c->lflag, &c->alive, &c->succ, &c->pred, &c->ad[0],
+                     &c->records, &c->keys, &c->counts, &c->csv_rows, &c->dstat, &c->ht, &c->rflag, &c->lflag, &c->alive, &c->succ, &c->pred, &c->ad[0],
                      &c->ad[1], &c->rd_src, &c->spl_id, &c->spl_node, &c->loc, &c->sp_ad[0], &c->sp_ad[1], &c->cmin[0], &c->cmin[1], &c->spl_tail, &c->spl_chain, &c->chain_len, &c->ctg_idx, &c->ctg_off,
                      &c->ctg_left, &c->ctg_right, &c->ctg_bases, &c->rx_records, &c->run_desc, &c->rd_runs, &c->seg_off, &c->seg_base, &c->ovf_rec, &c->ovf_bin, &c->g_rowbin, &c->g_binrows, &c->g_hoff, &c->g_bloom, &c->srt_left, &c->srt_right, &c->eff_l, &c->eff_r, &c->seg_ext,
                      &c->st_keys, &c->st_vals, &c->st_bloom, &c->st_firstk, &c->st_ctr, &c->st_len, &c->st_woff, &c->st_hits, &c->st_frags, &c->st_codes, &c->st_nxt, &c->st_prv,

@@ -127,6 +127,7 @@ struct Ctx {
     DevBuf keys;        // KT[table_cap]  right-aligned canonical k-mers
     DevBuf counts;      // u32[table_cap]
     DevBuf dstat;       // u64[16] device-side counters
+    DevBuf csv_rows;    // rfx_load_counts_csv: key, count and keep flag of every line of the chunk being parsed (scratch)
     uint64_t table_cap = 0, n_rows = 0, n_distinct = 0, n_bin_splits = 0, n_shard_instances = 0;
     int count_geometry = 0;           // 0: unknown (run the pilot), 1: small table, 2: large table -- survives rfx_reset
     uint32_t count_geometry_bins = 0; // bin count of the run the pilot looked at
@@ -256,6 +257,7 @@ enum {
     DS_FQ_SEQPOS = 41,
     DS_FQ_NEXT = 42,
     DS_REACHED = 43,      // nodes the splitter walks stamped: all alive nodes unless some sit on a closed path without a splitter
+    DS_CSV_BAD = 44,      // rfx_load_counts_csv: first malformed line of the chunk being parsed (~0: none)
     DS_NSLOTS = 48
 };
 
@@ -278,6 +280,7 @@ inline unsigned sm_count() {
 // stage entry points (each in its own .cu)
 int stage_parse_fastq(Ctx* c, const uint8_t* d_text, size_t len, bool first_chunk = true, bool more_follows = false);
 int stage_push_reads(Ctx* c, const uint8_t* h_bases, const uint64_t* h_offsets, uint64_t n_reads);
+int stage_load_counts_csv(Ctx* c, const uint8_t* text, size_t len, int64_t min_count, int64_t max_count, bool append);
 int stage_partition(Ctx* c, int n_shards);
 int stage_partition_slab(Ctx* c, uint64_t ovf_need = 0);
 int stage_stream_partition_begin(Ctx* c, uint64_t est_instances, uint64_t est_reads);

@@ -134,6 +134,13 @@ class ReflexivContext:
         counts = np.ascontiguousarray(counts, dtype=np.uint32)
         self._check(self.L.rfx_load_counts(self._ctx, keys.ctypes.data, counts.ctypes.data, len(counts)), self._ctx)
 
+    def load_counts_csv(self, text, min_count: int, max_count: int, append: bool = False):
+        """Count_<k> text (`KMER,count` / `(KMER,count)` rows) parsed on the device into the table: rows with
+        min_count <= count <= max_count, in text order, behind the current table if append.  The row rule is the `reflexiv`
+        binary's (include/reflexiv_cuda.h); a malformed row raises RfxError (RFX_E_INVALID) naming its line."""
+        a = _as_u8(text)
+        self._check(self.L.rfx_load_counts_csv(self._ctx, a.ctypes.data, a.size, min_count, max_count, 1 if append else 0), self._ctx)
+
     # ---- assembly ----
     def assemble(self):
         self._check(self.L.rfx_assemble(self._ctx), self._ctx)
